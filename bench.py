@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """bench.py — env-turns/sec of the batched Everglades turn step on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
+
+It runs what __graft_entry__.build() compiled and writes nothing into the tree (the tree may be read-only).
 
 One "step" = one game turn for every match of the batch: the random_actions agent kernel for both
 players + the turn-step kernel (--agents fused: one launch of evg_step_agents does both).  Workload (config.workload): BASELINE.json configs[4] at
@@ -50,6 +52,11 @@ UNIT = "env-turns/s"
 # (EvgEpisodeStats.fought_unit_slots), not assumed: a full random-vs-random episode averages 21.6.
 B_ALG_FIXED = 1331
 B_ALG_PER_FOUGHT_SLOT = 16
+# --dump-outputs: at most this many matches, drawn with a fixed seed, so that two builds run with the same arguments
+# dump the same matches.  A match's outputs take at most 892 B as float32 (obs 840, reward 8, done and status 4 each,
+# scores 8, action rows 28 where the step returns them), so the dump stays under 64 MB.
+DUMP_MATCHES = 65536
+DUMP_SEED = 1234
 
 
 def parse_args():
@@ -73,7 +80,16 @@ def parse_args():
                     help="observation transport of the headline e2e number (all lossless; f32 is always reported as e2e_f32 too)")
     ap.add_argument("--agents", default="kernel", choices=["kernel", "fused"],
                     help="random_actions rows from the agent kernel (2 launches/step) or generated inside the step kernel (1 launch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (observations, rewards, done flags and "
+                         "the info arrays) for a fixed sample of rank 0's matches as DIR/<name>.npy, float32, plus the "
+                         "sampled match ids as DIR/match_id.npy, float64")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; --impl reference has none")
+    return args
 
 
 def workload_config(args, world):
@@ -263,6 +279,33 @@ def ncu_traffic(envs_per_gpu, phase):
     return None
 
 
+def capture_outputs(step_out, first):
+    """Host copies of what one step returned, (obs, reward, done, info), for --dump-outputs: the rows of min(N,
+    DUMP_MATCHES) matches drawn with DUMP_SEED (sorted), every array as float32 (the integer ones hold values far below
+    2**24, so the conversion is exact), and the global ids of those matches as float64."""
+    import numpy as np
+    import torch
+
+    obs, rew, done, info = step_out
+    n = obs.shape[0]
+    idx = np.arange(n)
+    if n > DUMP_MATCHES:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MATCHES, replace=False))
+    sel = torch.as_tensor(idx, device=obs.device)
+    out = {"match_id": (first + idx).astype(np.float64)}
+    for name, t in [("obs", obs), ("reward", rew), ("done", done)] + sorted(info.items()):
+        out[name] = t.index_select(0, sel).cpu().numpy().astype(np.float32)
+    return out
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def _emit(line: dict) -> None:
     """The ONE JSON line goes to the real stdout; everything else any library prints (NCCL's version banner,
@@ -297,10 +340,7 @@ def main():
 
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as g
 
-    if rank == 0:
-        g.build()
     if world > 1:
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
@@ -358,14 +398,16 @@ def main():
         a = None if fused else env.random_actions()
         ev[k][0].record(stream)
         if fused:
-            env.step_agents()
+            out = env.step_agents()
         else:
-            env.step(a)
+            out = env.step(a)
         ev[k][1].record(stream)
     t_end.record(stream)
     torch.cuda.synchronize(dev)
     torch.cuda.profiler.stop()
     wall1 = time.perf_counter()
+    # the step's tensors are overwritten by the steps below: copy the last timed step's outputs now
+    dumped = capture_outputs(out, first) if args.dump_outputs and rank == 0 else None
     if world > 1:
         dist.barrier()
     clk = clocks.report(wall0, wall1)
@@ -488,6 +530,8 @@ def main():
         }
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"], line["cpu_baseline_port"] = cpu_baselines(args.cpu_seconds, args.seed)
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         _emit(line)
     if world > 1:
         dist.barrier()

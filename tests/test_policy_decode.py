@@ -49,7 +49,8 @@ def test_device_decode_matches_reference():
 
 def test_reward_shaping_restatement_matches_reference_functions():
     import importlib.util
-    path = "/root/reference/utils/reward_shaping.py"
+    from oracle import ref_harness as rh
+    path = os.path.join(rh.REFERENCE_ROOT, "utils", "reward_shaping.py")
     if not os.path.isfile(path):
         pytest.skip("reference checkout not present")
     spec = importlib.util.spec_from_file_location("ref_reward_shaping", path)
