@@ -25,10 +25,11 @@
 // bf16 operands, fp32 accumulation.  Q is written either row-major [rows][out] (torch's layout) or transposed
 // [out][rows] — what the thread-per-row decode (evg_decode_dqn, pinned to the reference's DQNAgent.filter_actions)
 // reads coalesced.  tests/test_gpu_policy.py checks Q against torch fp32 within the bf16 tolerance stated there.
-// Weight images are built on the host by evgsim.policy.pack_mlp (same swizzle function as below).
+// Weight images are built on the host by evgsim.policy.pack_mlp (same swizzle function as evg_tcgen05.cuh).
 #include <cuda_bf16.h>
 
 #include "evg_internal.h"
+#include "evg_tcgen05.cuh"
 
 namespace evg {
 
@@ -39,7 +40,6 @@ constexpr int kTileM = 128;   // observation rows per tile
 constexpr int kInPad = 128;   // input features, padded (obs_len <= 128)
 constexpr int kChunk = 192;   // hidden units per chunk: 3 swizzle atoms of 64
 constexpr int kOutPad = 144;  // outputs, padded to a multiple of 16 (12 groups x 11 nodes = 132)
-constexpr int kAtomK = 64;    // bf16 elements in one 128-byte swizzle row
 
 // shared-memory carve-up (bytes; every operand block starts on a 1024-byte boundary, as the 128-byte swizzle needs)
 constexpr int kSmA = 0;                                            // 2 atoms x [128 rows x 128 B]
@@ -54,83 +54,6 @@ static_assert(kSmH % 1024 == 0 && kSmW1 % 1024 == 0 && kSmW2 % 1024 == 0 && (kOu
 
 constexpr int kTmemCols = 512;  // power of two >= D1 (192) + D2 (144) columns
 constexpr int kTmemD1 = 0, kTmemD2 = 256;
-
-// K-major operand tile with 128-byte swizzle: element (row r, column k) of a [rows x K] bf16 matrix lives in atom k / 64
-// (a block of rows x 128 bytes), at row r, 16-byte chunk ((k % 64) / 8) ^ (r % 8)
-__host__ __device__ inline int swz_offset(int rows, int r, int k)
-{
-    return (k / kAtomK) * rows * 128 + r * 128 + ((((k % kAtomK) >> 3) ^ (r & 7)) << 4) + (k & 7) * 2;
-}
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start address >> 4 [0:14), leading byte offset >> 4
-// [16:30) (unused for a swizzled K-major operand), stride byte offset >> 4 [32:46) = 1024 B between 8-row groups,
-// version 1 [46:48), layout SWIZZLE_128B = 2 [61:64)
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr)
-{
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (uint64_t)1 << 16 | (uint64_t)(1024 >> 4) << 32 | (uint64_t)1 << 46 | (uint64_t)2 << 61;
-}
-
-// instruction descriptor (cute::UMMA::InstrDescriptor): D fp32 [4:6) = 1, A bf16 [7:10) = 1, B bf16 [10:13) = 1, both
-// K-major, N >> 3 at [17:23), M >> 4 at [24:29)
-__device__ __forceinline__ uint32_t make_idesc(int m, int n)
-{
-    return 1u << 4 | 1u << 7 | 1u << 10 | (uint32_t)(n >> 3) << 17 | (uint32_t)(m >> 4) << 24;
-}
-
-__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
-__device__ __forceinline__ void umma_commit(uint64_t* bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// wait for phase `parity` of an mbarrier; a bounded spin that traps instead of hanging the GPU if the MMAs never arrive
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity)
-{
-    const uint32_t a = smem_u32(bar);
-    for (uint32_t spin = 0;; ++spin) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-            : "=r"(done)
-            : "r"(a), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (spin > (1u << 26)) __trap();
-    }
-}
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
-          "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr));
-}
-
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
-{
-    const __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<const uint32_t*>(&p);
-}
-
-// one bulk copy global -> shared memory, completion counted in bytes on `bar`
-__device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
-                 "r"(smem_u32(bar))
-                 : "memory");
-}
 
 // q_col_stride == 1: Q[row * q_row_stride + col] (row-major); q_row_stride == 1: Q[col * q_col_stride + row] (transposed)
 __global__ void __launch_bounds__(kMlpThreads, 1)

@@ -1,10 +1,14 @@
-"""Policy-in-the-loop glue: the reference's DQN network (agents/DQN/QNetwork.py:37,42 — Linear(105, 528) - ReLU -
-Linear(528, 132)) evaluated by libevgsim's fused tensor-core kernel (evg_policy_mlp: tcgen05 + TMEM, bf16 operands, fp32
-accumulation) on the observation tensor the step kernel writes, and decoded by evg_decode_dqn.
+"""Policy-in-the-loop glue: the reference's two networks evaluated by libevgsim's fused tensor-core kernels (tcgen05 +
+TMEM, bf16 operands, fp32 accumulation) on the observation tensor the step kernel writes.
 
-``pack_mlp`` turns the two weight matrices into the images the kernel copies straight into shared memory (bf16, K-major,
-128-byte swizzle; layout in include/evgsim.h).  ``FusedDQN`` wraps a torch ``Sequential(Linear, ReLU, Linear)`` (or raw
-arrays) for a BatchedEvergladesEnv.  Plumbing only; the network itself is the caller's.
+- DQN (agents/DQN/QNetwork.py:37,42 — Linear(105, 528) - ReLU - Linear(528, 132)): evg_policy_mlp, decoded by
+  evg_decode_dqn.  ``pack_mlp`` builds its weight images, ``FusedDQN`` wraps a torch ``Sequential(Linear, ReLU, Linear)``.
+- PPO's actor (agents/PPO/ActorCritic.py:33-50 without the GRU — Linear(105, L) - Tanh - Linear(L, L) - Tanh -
+  Linear(L, 132) - Tanh - Softmax): evg_policy_ppo, which also draws PPOAgent.get_action's 7 indices on the tape and
+  writes the action rows.  ``pack_ppo`` builds its images, ``FusedPPO`` wraps the torch ``Sequential``.
+
+The images are what the kernels copy straight into shared memory (bf16, K-major, 128-byte swizzle; layout in
+include/evgsim.h).  Plumbing only; the networks themselves are the caller's.
 """
 from __future__ import annotations
 
@@ -15,6 +19,7 @@ import numpy as np
 from . import _capi
 
 IN_PAD, CHUNK, OUT_PAD, ATOM = _capi.MLP_IN_PAD, _capi.MLP_CHUNK, _capi.MLP_OUT_PAD, 64
+PPO_IN_PAD, PPO_MAX_LATENT, PPO_OUT_PAD = _capi.PPO_IN_PAD, _capi.PPO_MAX_LATENT, _capi.PPO_OUT_PAD
 
 
 def to_bf16_bits(x):
@@ -114,4 +119,70 @@ class FusedDQN:
         assert self.out_dim % _capi.NUM_GROUPS == 0
         _capi.check(env._lib.evg_decode_dqn_layout(env._h, C.c_void_p(qt.data_ptr()), self.out_dim // _capi.NUM_GROUPS, -1, 1,
                                                    C.c_void_p(env._actions.data_ptr()), env._stream()))
+        return env._actions
+
+
+def pack_ppo(w1, b1, w2, b2, w3, b3):
+    """w1 [L, in], b1 [L], w2 [L, L], b2 [L], w3 [out, L], b3 [out] (float32, torch.nn.Linear's layout) ->
+    (w1_img, w2_img, w3_img uint8, bias float32, latent, out) as evg_policy_ppo expects them: W1 as an [Lp x 128] block,
+    W2 as [Lp x Ka], W3 as [144 x Ka] (Lp = L rounded up to 16, Ka = L rounded up to 64), zero padded; the biases stay
+    float32, b1 | b2 | b3 at 0, 256 and 512 of one zero-padded vector (the kernel adds them in fp32)."""
+    w1, b1, w2, b2, w3, b3 = (np.asarray(a, dtype=np.float32) for a in (w1, b1, w2, b2, w3, b3))
+    latent, in_dim = w1.shape
+    out = w3.shape[0]
+    assert in_dim < PPO_IN_PAD and 1 <= latent <= PPO_MAX_LATENT and 7 <= out <= PPO_OUT_PAD
+    assert w2.shape == (latent, latent) and w3.shape[1] == latent and b1.shape == b2.shape == (latent,) and b3.shape == (out,)
+    lp, ka = -(-latent // 16) * 16, -(-latent // ATOM) * ATOM
+    bias = np.zeros(2 * PPO_MAX_LATENT + PPO_OUT_PAD, dtype=np.float32)
+    bias[:latent] = b1
+    bias[PPO_MAX_LATENT:PPO_MAX_LATENT + latent] = b2
+    bias[2 * PPO_MAX_LATENT:2 * PPO_MAX_LATENT + out] = b3
+    return _image(w1, lp, PPO_IN_PAD), _image(w2, lp, ka), _image(w3, PPO_OUT_PAD, ka), bias, latent, out
+
+
+def reference_forward_ppo(obs, w1, b1, w2, b2, w3, b3):
+    """What evg_policy_ppo computes, in numpy: bf16-rounded operands (observations, weights, both hidden activations),
+    float32 accumulation, biases added in float32 (not rounded), y = tanh(z), probabilities exp(y) / sum(exp(y)) in
+    float32.  Returns float32 [rows, out]."""
+    f32 = np.float32
+    x = bf16_round(np.asarray(obs, dtype=f32))
+    h = np.tanh((x @ bf16_round(w1).T).astype(f32) + np.asarray(b1, f32)).astype(f32)
+    h = np.tanh((bf16_round(h) @ bf16_round(w2).T).astype(f32) + np.asarray(b2, f32)).astype(f32)
+    y = np.tanh((bf16_round(h) @ bf16_round(w3).T).astype(f32) + np.asarray(b3, f32)).astype(f32)
+    e = np.exp(y).astype(f32)
+    return (e / e.sum(axis=-1, dtype=f32, keepdims=True)).astype(f32)
+
+
+class FusedPPO:
+    """PPO actor forward + PPOAgent.get_action's sampling for a BatchedEvergladesEnv, in one kernel:
+    ``actions = FusedPPO(env, net)()`` reads env.obs in place (so the env must be stepped in the f32 format) and writes
+    env._actions.  The draws come from the tape (seed, global match id, turn, episode, player), not from torch's
+    generator: the rows do not depend on batch size, sharding or call order.  `player` -1 plays both sides, 0 or 1 only
+    that side's rows (the other side's rows are left as they are, e.g. for a scripted opponent)."""
+
+    def __init__(self, env, net=None, weights=None, player=-1, latent=None, div=12, mod=11):
+        import torch
+        if weights is None:
+            lin = [m for m in net if isinstance(m, torch.nn.Linear)]
+            assert len(lin) == 3, "expected Sequential(Linear, Tanh, Linear, Tanh, Linear, Tanh, Softmax)"
+            weights = [t.detach().float().cpu().numpy() for m in lin for t in (m.weight, m.bias)]
+        img1, img2, img3, bias, self.latent, self.out_dim = pack_ppo(*weights)
+        assert latent is None or latent == self.latent, "latent %s != the weights' %d" % (latent, self.latent)
+        assert player in (-1, 0, 1)
+        self.env, self.player, self.div, self.mod = env, int(player), int(div), int(mod)
+        dev = env.device
+        self._w = [torch.from_numpy(a).to(dev) for a in (img1, img2, img3, bias)]
+        shape = (env.num_envs, 2) if self.player < 0 else (env.num_envs,)
+        self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
+        self.probs = torch.empty(shape + (self.out_dim,), dtype=torch.float32, device=dev)
+
+    def __call__(self, want_probs=False):
+        """Action rows int8 [N, 2, 7, 2] (env._actions); fills .idx (int64 [N, 2, 7] or [N, 7]) and, with want_probs,
+        .probs (float32 [N, 2, out] or [N, out])."""
+        env = self.env
+        w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_policy_ppo(env._h, C.c_void_p(env.obs.data_ptr()), self.player, w1, w2, w3, bias, self.latent,
+                                            self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
+                                            C.c_void_p(self.idx.data_ptr()), C.c_void_p(self.probs.data_ptr()) if want_probs else None,
+                                            env._stream()))
         return env._actions

@@ -316,6 +316,33 @@ int evg_decode_indices(EvgSim* sim, const int64_t* d_idx, int32_t div, int32_t m
 int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_w1_img, const void* d_w2_img, int32_t hidden, int32_t out_dim,
                    float* d_q, int32_t q_transposed, void* stream);
 
+/* PPO's feed-forward actor with the action sampling fused behind it, on the tensor cores (csrc/evg_policy_ppo.cu):
+ *     probs = Softmax(Tanh(Linear(latent, out_dim)(Tanh(Linear(latent, latent)(Tanh(Linear(obs_len, latent)(obs)))))))
+ * — agents/PPO/ActorCritic.py:33-50 without the GRU — for the rows of `player` (0, 1, or -1 = both) of the observation
+ * tensor d_obs float32 [n_envs][2][obs_len], then PPOAgent.get_action (agents/PPO/PPOAgent.py:122-127): 7 distinct flat
+ * indices drawn without replacement, written as action rows (idx / div, idx % mod) into d_actions int8 [n_envs][2][7][2]
+ * (only `player`'s rows; PPO's unravel is div 12, mod 11).  bf16 operands, fp32 accumulation, biases added in fp32.
+ * The draws are keyed on the tape (DESIGN.md section 7, domain 3): (seed, global match id, turn and episode of the match's
+ * current state, player) — independent of batch size, sharding and call order.
+ *   d_idx (optional):   int64 [n_envs][2][7] (player -1) or [n_envs][7], the drawn indices in draw order.
+ *   d_probs (optional): float32 [n_envs][2][out_dim] or [n_envs][out_dim], the probabilities the draws were made from.
+ * Weights are IMAGES in the kernel's shared-memory operand layout (bf16, K-major, 128-byte swizzle, zero padded, 16-byte
+ * aligned).  With Lp = latent rounded up to 16 and Ka = latent rounded up to 64:
+ *     d_w1_img: W1[n][k] as an [Lp x EVG_PPO_IN_PAD] block,  (EVG_PPO_IN_PAD / 64) * Lp * 128 bytes
+ *     d_w2_img: W2[n][k] as an [Lp x Ka] block,              (Ka / 64) * Lp * 128 bytes
+ *     d_w3_img: W3[o][k] as an [EVG_PPO_OUT_PAD x Ka] block, (Ka / 64) * EVG_PPO_OUT_PAD * 128 bytes
+ * element (row r, column k) of an [R x K] block at byte (k/64)*R*128 + r*128 + ((((k%64)/8) ^ (r%8)) * 16) + (k%8)*2.
+ *     d_bias: float32 [2 * EVG_PPO_MAX_LATENT + EVG_PPO_OUT_PAD] = b1 at 0, b2 at EVG_PPO_MAX_LATENT, b3 at
+ *             2 * EVG_PPO_MAX_LATENT, zero padded.
+ * evgsim.policy.pack_ppo builds them from a torch module.  1 <= latent <= EVG_PPO_MAX_LATENT, 7 <= out_dim <= EVG_PPO_OUT_PAD,
+ * obs_len < EVG_PPO_IN_PAD. */
+#define EVG_PPO_IN_PAD 128
+#define EVG_PPO_MAX_LATENT 256
+#define EVG_PPO_OUT_PAD 144
+int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_w3_img,
+                   const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions, int64_t* d_idx,
+                   float* d_probs, void* stream);
+
 /* Reward shaping of the reference's training scripts (utils/reward_shaping.py:17-56) on the step's outputs:
  * d_out float32 [n_envs][2].  turnNum (steps played before this one) is read from the observation's turn
  * field, so use it with EVG_AUTORESET_OFF or _TERMINAL (the observation of a finished match is the terminal one). */

@@ -13,7 +13,9 @@ GRU(128, 128) (hidden state carried over the 7 steps and from turn to turn, zero
 sampled per step (ActorCritic.act with use_recurrent, agents/PPO/ActorCritic.py:79-105).  --graph captures the whole
 turn (forward, sampling, decode, step) in a CUDA graph.  The observation tensor the step kernel writes is consumed in place
 (a [N*2, 105] view, no copy, no dtype conversion kernel for fp32); the decoded int8 rows go straight back into the
-step.  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
+step.  --fused runs the network in libevgsim's tcgen05 kernels instead of torch: DQN's forward in evg_policy_mlp (then
+evg_decode_dqn), PPO's forward, sampling and unravel in evg_policy_ppo (its draws come from the simulator's tape, not from
+torch's generator).  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
 """
 import argparse
 import json
@@ -77,7 +79,7 @@ def main():
     ap.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"])
     ap.add_argument("--graph", action="store_true", help="replay the turn (forward, decode, step) from a CUDA graph")
     ap.add_argument("--fused", action="store_true",
-                    help="dqn only: the forward runs in libevgsim's fused tcgen05 kernel (evg_policy_mlp, bf16 operands) instead of torch")
+                    help="dqn / ppo: the policy runs in libevgsim's fused tcgen05 kernels (evg_policy_mlp / evg_policy_ppo, bf16 operands) instead of torch")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -95,9 +97,9 @@ def main():
 
     fused = None
     if args.fused:
-        assert args.policy == "dqn", "--fused is the DQN network's kernel"
+        assert args.policy in ("dqn", "ppo"), "--fused has kernels for the DQN network and the feed-forward PPO actor"
         from evgsim import policy as evp
-        fused = evp.FusedDQN(env, net.float())
+        fused = evp.FusedDQN(env, net.float()) if args.policy == "dqn" else evp.FusedPPO(env, net.float())
 
     def turn():
         env.step(fused() if fused is not None else policy_actions(env, net, args.policy, dtype, hidden))
@@ -133,7 +135,7 @@ def main():
     stats = evgsim.gather_episode_stats(env.episode_stats(), device=env.device) if world > 1 else env.episode_stats()
     if rank == 0:
         sec = float(ms.item()) / 1e3
-        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (evg_policy_mlp)" if args.fused else args.dtype, "fused_forward": bool(args.fused),
+        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % ("evg_policy_mlp" if args.policy == "dqn" else "evg_policy_ppo") if args.fused else args.dtype, "fused_forward": bool(args.fused),
                           "cuda_graph": bool(args.graph),
                           "n_gpus": world, "envs_per_gpu": E, "turns": args.turns, "env_turns_per_s": E * world * args.turns / sec,
                           "ms_per_turn": sec * 1e3 / args.turns, "episodes": stats["episodes"], "wins": stats["wins"], "ties": stats["ties"]}))
