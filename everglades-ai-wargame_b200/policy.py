@@ -79,6 +79,13 @@ def reference_forward(obs, w1, b1, w2, b2):
     return bf16_round(h) @ bf16_round(w2).T + bf16_round(b2)
 
 
+def _check_input_width(w1, env):
+    """The kernels read env.obs_len features per row (and DQN's bias input sits right behind them): a first layer of
+    another width would silently multiply the wrong columns."""
+    if np.shape(w1)[1] != env.obs_len:
+        raise ValueError("the network takes %d inputs, the environment's observations have %d values" % (np.shape(w1)[1], env.obs_len))
+
+
 class FusedDQN:
     """Q-network forward + decode for a BatchedEvergladesEnv: ``actions = FusedDQN(env, net)()`` reads env.obs in place."""
 
@@ -88,6 +95,7 @@ class FusedDQN:
             lin = [m for m in net if isinstance(m, torch.nn.Linear)]
             assert len(lin) == 2, "expected Sequential(Linear, ReLU, Linear)"
             weights = [t.detach().float().cpu().numpy() for t in (lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias)]
+        _check_input_width(weights[0], env)
         img1, img2, self.hidden, self.out_dim = pack_mlp(*weights)
         self.env = env
         dev = env.device
@@ -98,7 +106,15 @@ class FusedDQN:
 
     def _run(self, obs, out, transposed):
         env = self.env
-        obs = env.obs if obs is None else obs
+        if obs is None:
+            obs = env.obs
+        else:  # the kernel reads num_envs * 2 rows of obs_len float32 values from obs.data_ptr(), whatever obs is
+            import torch
+            if obs.dtype != torch.float32 or not obs.is_contiguous() or obs.device != env.device \
+                    or obs.numel() != env.num_envs * 2 * env.obs_len:
+                raise ValueError("obs must be a contiguous float32 tensor of %d x 2 x %d values on %s, got %s %s%s on %s"
+                                 % (env.num_envs, env.obs_len, env.device, obs.dtype, tuple(obs.shape),
+                                    "" if obs.is_contiguous() else " (not contiguous)", obs.device))
         _capi.check(env._lib.evg_policy_mlp(env._h, C.c_void_p(obs.data_ptr()), env.num_envs * 2, C.c_void_p(self._w1.data_ptr()),
                                             C.c_void_p(self._w2.data_ptr()), self.hidden, self.out_dim, C.c_void_p(out.data_ptr()),
                                             int(transposed), env._stream()))
@@ -166,6 +182,7 @@ class FusedPPO:
             lin = [m for m in net if isinstance(m, torch.nn.Linear)]
             assert len(lin) == 3, "expected Sequential(Linear, Tanh, Linear, Tanh, Linear, Tanh, Softmax)"
             weights = [t.detach().float().cpu().numpy() for m in lin for t in (m.weight, m.bias)]
+        _check_input_width(weights[0], env)
         img1, img2, img3, bias, self.latent, self.out_dim = pack_ppo(*weights)
         assert latent is None or latent == self.latent, "latent %s != the weights' %d" % (latent, self.latent)
         assert player in (-1, 0, 1)

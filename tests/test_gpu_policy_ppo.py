@@ -45,17 +45,13 @@ def expected_idx(env, probs, player=-1):
     import ppo_sampling as ps
     st = env.get_state()
     players = (0, 1) if player < 0 else (player,)
-    probs = probs.reshape(env.num_envs, len(players), -1)
-    out = np.zeros((env.num_envs, len(players), 7), dtype=np.int64)
-    for m in range(env.num_envs):
-        t, e = int(st[m]["turn"]), int(st[m]["episode"])
-        for k, p in enumerate(players):
-            out[m, k] = ps.ppo_sample(probs[m, k], ps.policy_uniforms(env.seed, env.env_id_offset + m, t, p, e))
-    return out
+    u = np.stack([[ps.policy_uniforms(env.seed, env.env_id_offset + m, int(st[m]["turn"]), p, int(st[m]["episode"])) for p in players]
+                  for m in range(env.num_envs)])
+    return ps.ppo_sample_rows(probs.reshape(-1, probs.shape[-1]), u.reshape(-1, 7)).reshape(env.num_envs, len(players), 7)
 
 
 @pytest.mark.parametrize("n", [64, 1037, 4096])
-@pytest.mark.parametrize("latent", [128, 248, 100])
+@pytest.mark.parametrize("latent", [128, 248, 100, 1, 15, 16, 17, 63, 64, 65, 129, 160, 192, 193, 255, 256])
 def test_probabilities_and_exact_sampling(evg, cfg, n, latent):
     import torch
     from evgsim import policy

@@ -14,7 +14,7 @@ def _weights(rng, latent, out=132, in_dim=105, scale=1.0):
             for s in ((latent, in_dim), (latent,), (latent, latent), (latent,), (out, latent), (out,))]
 
 
-@pytest.mark.parametrize("latent", [128, 248, 100, 1])
+@pytest.mark.parametrize("latent", [128, 248, 100, 1, 15, 16, 17, 63, 64, 65, 129, 160, 192, 193, 255, 256])
 def test_pack_ppo_places_every_weight_where_the_header_says(latent):
     w1, b1, w2, b2, w3, b3 = _weights(np.random.default_rng(latent), latent)
     img1, img2, img3, bias, L, out = policy.pack_ppo(w1, b1, w2, b2, w3, b3)
@@ -93,6 +93,23 @@ def test_ppo_sample_draws_distinct_indices_and_falls_back_to_the_largest_open_in
     q = np.full(8, np.float32(1 / 8))
     assert ps.ppo_sample(q, np.zeros(7, dtype=np.float32)).tolist() == [0, 1, 2, 3, 4, 5, 6]
     assert ps.ppo_sample(q, np.full(7, 1 - 2 ** -24, dtype=np.float32)).tolist() == [7, 6, 5, 4, 3, 2, 1]
+
+
+def test_ppo_sample_rows_equals_ppo_sample_row_by_row():
+    """The vectorised sampler the GPU tests check whole batches with makes the same draws as the scalar statement,
+    including rows whose mass runs out (the fallback to the largest open index) and uniforms at both ends."""
+    rng = np.random.default_rng(5)
+    for n in (7, 17, 132, 144):
+        p = rng.random((300, n)).astype(np.float32) ** 4  # a few large entries, many tiny ones
+        p[:20] = 0
+        p[np.arange(20), rng.integers(0, n, 20)] = 1  # one index with all the mass
+        p[20:40, : n // 2] = 0
+        p /= p.sum(-1, dtype=np.float32, keepdims=True)
+        u = rng.random((300, 7)).astype(np.float32)
+        u[40:60] = 0
+        u[60:80] = 1 - 2 ** -24
+        want = np.stack([ps.ppo_sample(p[i], u[i]) for i in range(300)])
+        assert np.array_equal(ps.ppo_sample_rows(p, u), want), n
 
 
 def test_ppo_sample_matches_sequential_sampling_without_replacement():
