@@ -908,6 +908,30 @@ int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* 
     return EVG_OK;
 }
 
+int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_wi_img,
+                    const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
+                    float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
+{
+    int rc = check_sim(sim, true);  // the draws and the turn-0 reset of the state read the bound records
+    if (rc) return rc;
+    if (!d_obs || !d_w1_img || !d_w2_img || !d_wi_img || !d_wh_img || !d_w3_img || !d_bias || !d_actions)
+        return fail(EVG_E_ARG, "evg_policy_rppo: null argument");
+    if (!d_hidden) return fail(EVG_E_ARG, "evg_policy_rppo: d_hidden (the GRU state, in and out) is null");
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_rppo: player %d outside -1..1", player);
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "evg_policy_rppo: latent %d outside 1..%d", latent, EVG_PPO_MAX_LATENT);
+    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "evg_policy_rppo: out_dim %d outside %d..%d", out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
+    if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_rppo: div %d / mod %d must be positive", div, mod);
+    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img | (uintptr_t)d_wi_img | (uintptr_t)d_wh_img | (uintptr_t)d_w3_img) % 16)
+        return fail(EVG_E_ARG, "evg_policy_rppo: weight images must be 16-byte aligned");
+    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "evg_policy_rppo: observations of %d values exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    cudaError_t e = evg::launch_policy_rppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
+                                            d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_hidden, d_actions, d_idx, d_probs,
+                                            sim->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_rppo_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
 int evg_shape_reward(EvgSim* sim, int32_t mode, const float* d_reward, const uint8_t* d_done, const float* d_obs, float* d_out,
                      void* stream)
 {

@@ -169,6 +169,10 @@ cudaError_t launch_policy_mlp(const float* obs, int64_t rows, int in_dim, const 
 cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
                               int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream);
+cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+                               const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
+                               int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
+                               cudaStream_t stream);
 cudaError_t launch_obs_to_i16(const float* obs, int16_t* out, int64_t n_values, cudaStream_t stream);
 cudaError_t launch_export(const Tables& t, const uint32_t* records, const double* health, int64_t first, int64_t count,
                           EvgEnvState* out, cudaStream_t stream);

@@ -6,6 +6,10 @@ TMEM, bf16 operands, fp32 accumulation) on the observation tensor the step kerne
 - PPO's actor (agents/PPO/ActorCritic.py:33-50 without the GRU — Linear(105, L) - Tanh - Linear(L, L) - Tanh -
   Linear(L, 132) - Tanh - Softmax): evg_policy_ppo, which also draws PPOAgent.get_action's 7 indices on the tape and
   writes the action rows.  ``pack_ppo`` builds its images, ``FusedPPO`` wraps the torch ``Sequential``.
+- PPO's recurrent actor (agents/PPO/ActorCritic.py:33-60 with use_recurrent — the same head, then GRU(L, L) stepped 7
+  times on the head's output, Linear(L, 132) - Tanh - Softmax after every step, one draw per step): evg_policy_rppo, which
+  carries the GRU state across turns and zeroes it when a match starts over.  ``pack_rppo`` builds its images,
+  ``FusedRPPO`` wraps a module with the reference ActorCritic's ``action_head``, ``action_gru`` and ``action_layer``.
 
 The images are what the kernels copy straight into shared memory (bf16, K-major, 128-byte swizzle; layout in
 include/evgsim.h).  Plumbing only; the networks themselves are the caller's.
@@ -202,4 +206,117 @@ class FusedPPO:
                                             self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
                                             C.c_void_p(self.idx.data_ptr()), C.c_void_p(self.probs.data_ptr()) if want_probs else None,
                                             env._stream()))
+        return env._actions
+
+
+def rppo_weights(actor):
+    """(w1, b1, w2, b2, w_ih, b_ih, w_hh, b_hh, w3, b3) float32 numpy arrays of a module with the reference ActorCritic's
+    action_head (Linear, Tanh, Linear, Tanh), action_gru and action_layer (Linear, Tanh, Softmax).  ValueError for a GRU
+    the kernel does not run: more than one layer, bidirectional, an input width other than the hidden width, no biases."""
+    import torch
+    gru = actor.action_gru
+    if gru.num_layers != 1 or gru.bidirectional or gru.input_size != gru.hidden_size or not gru.bias:
+        raise ValueError("the fused recurrent actor runs one unidirectional GRU layer with biases and input width = hidden "
+                         "width; got num_layers=%d bidirectional=%s input_size=%d hidden_size=%d bias=%s"
+                         % (gru.num_layers, gru.bidirectional, gru.input_size, gru.hidden_size, gru.bias))
+    head = [m for m in actor.action_head if isinstance(m, torch.nn.Linear)]
+    out = [m for m in actor.action_layer if isinstance(m, torch.nn.Linear)]
+    if len(head) != 2 or len(out) != 1:
+        raise ValueError("expected action_head = (Linear, Tanh, Linear, Tanh) and action_layer = (Linear, Tanh, Softmax)")
+    latent = gru.hidden_size
+    if not 1 <= latent <= PPO_MAX_LATENT:
+        raise ValueError("the GRU's width %d is outside 1..%d" % (latent, PPO_MAX_LATENT))
+    if head[1].weight.shape[0] != latent:
+        raise ValueError("the head's output width %d is not the GRU's %d" % (head[1].weight.shape[0], latent))
+    ts = (head[0].weight, head[0].bias, head[1].weight, head[1].bias, gru.weight_ih_l0, gru.bias_ih_l0, gru.weight_hh_l0,
+          gru.bias_hh_l0, out[0].weight, out[0].bias)
+    return [t.detach().float().cpu().numpy() for t in ts]
+
+
+def pack_rppo(w1, b1, w2, b2, w_ih, b_ih, w_hh, b_hh, w3, b3):
+    """The recurrent actor's weights (float32, torch's layouts: w_ih / w_hh [3L, L] and b_ih / b_hh [3L] with gates r, z, n
+    as torch.nn.GRU's weight_ih_l0 ...) -> (w1_img, w2_img, wi_img, wh_img, w3_img uint8, bias float32, latent, out) as
+    evg_policy_rppo expects them.  W1, W2, W3 and b1 | b2 | b3 are pack_ppo's; each GRU matrix is three [Lp x Ka] blocks,
+    one per gate; b_ih gate g follows b3 at 656 + 256 g, b_hh gate g at 1424 + 256 g (include/evgsim.h)."""
+    img1, img2, img3, bias, latent, out = pack_ppo(w1, b1, w2, b2, w3, b3)
+    w_ih, b_ih, w_hh, b_hh = (np.asarray(a, dtype=np.float32) for a in (w_ih, b_ih, w_hh, b_hh))
+    assert w_ih.shape == w_hh.shape == (3 * latent, latent) and b_ih.shape == b_hh.shape == (3 * latent,)
+    lp, ka = -(-latent // 16) * 16, -(-latent // ATOM) * ATOM
+    gates = [np.concatenate([_image(w[g * latent:(g + 1) * latent], lp, ka) for g in range(3)]) for w in (w_ih, w_hh)]
+    gb = np.zeros(6 * PPO_MAX_LATENT, dtype=np.float32)
+    for g in range(3):
+        gb[g * PPO_MAX_LATENT:g * PPO_MAX_LATENT + latent] = b_ih[g * latent:(g + 1) * latent]
+        gb[(3 + g) * PPO_MAX_LATENT:(3 + g) * PPO_MAX_LATENT + latent] = b_hh[g * latent:(g + 1) * latent]
+    return img1, img2, gates[0], gates[1], img3, np.concatenate([bias, gb]), latent, out
+
+
+def reference_forward_rppo(obs, h0, weights, bf16=True):
+    """What evg_policy_rppo computes, in numpy: obs float32 [rows, in], h0 float32 [rows, L], weights as rppo_weights
+    returns them -> (probs float32 [rows, 7, out], h float32 [rows, L]).  With bf16 the operands of every product are
+    rounded to bf16 as the kernel's are (observations, weights, both head activations, h at each step), products
+    accumulate in float32, and the biases, gate arithmetic and h stay float32; r and z add X W_i^T + H W_h^T first and
+    then b_i + b_h, as the kernel's shared accumulator does.  Without bf16 it is plain float32 in torch.nn.GRU's order."""
+    f32 = np.float32
+    w1, b1, w2, b2, w_ih, b_ih, w_hh, b_hh, w3, b3 = (np.asarray(a, dtype=f32) for a in weights)
+    rnd = bf16_round if bf16 else (lambda v: np.asarray(v, dtype=f32))
+    latent = w1.shape[0]
+
+    def sig(v):
+        return (f32(1) / (f32(1) + np.exp(-v))).astype(f32)
+
+    a1 = np.tanh((rnd(obs) @ rnd(w1).T).astype(f32) + b1).astype(f32)
+    x = rnd(np.tanh((rnd(a1) @ rnd(w2).T).astype(f32) + b2).astype(f32))
+    gi = (x @ rnd(w_ih).T).astype(f32)  # the same every step
+    h = np.array(h0, dtype=f32)
+    probs = []
+    for _ in range(7):
+        gh = (rnd(h) @ rnd(w_hh).T).astype(f32)
+        s = slice(0, latent), slice(latent, 2 * latent), slice(2 * latent, 3 * latent)
+        if bf16:
+            r = sig((gi[:, s[0]] + gh[:, s[0]]) + (b_ih[s[0]] + b_hh[s[0]]))
+            z = sig((gi[:, s[1]] + gh[:, s[1]]) + (b_ih[s[1]] + b_hh[s[1]]))
+        else:
+            r = sig(gi[:, s[0]] + b_ih[s[0]] + gh[:, s[0]] + b_hh[s[0]])
+            z = sig(gi[:, s[1]] + b_ih[s[1]] + gh[:, s[1]] + b_hh[s[1]])
+        n = np.tanh((gi[:, s[2]] + b_ih[s[2]]) + r * (gh[:, s[2]] + b_hh[s[2]])).astype(f32)
+        h = ((f32(1) - z) * n + z * h).astype(f32)
+        e = np.exp(np.tanh((rnd(h) @ rnd(w3).T).astype(f32) + b3)).astype(f32)
+        probs.append((e / e.sum(axis=-1, dtype=f32, keepdims=True)).astype(f32))
+    return np.stack(probs, axis=1), h
+
+
+class FusedRPPO:
+    """PPO's recurrent actor + its 7 draws for a BatchedEvergladesEnv, in one kernel: ``actions = FusedRPPO(env, actor)()``
+    reads env.obs in place (the env must be stepped in the f32 format), steps the GRU state ``.hidden`` and writes
+    env._actions.  ``.hidden`` (float32 [N, 2, L], or [N, L] for one player; zero at construction) is read and written
+    back by every call, and a row restarts from zero when its match's record is at turn 0 (after reset() and after an
+    automatic reset): under AUTORESET_TERMINAL / _NEXT that is the ``hidden *= 1 - done`` mask of a torch rollout.  Under
+    AUTORESET_OFF a finished match keeps its state until it is reset.  Step k draws one index from its distribution with
+    replacement (ActorCritic.act: one torch.multinomial(probs, 1) per step), keyed on the tape as FusedPPO's draws.
+    `player` -1 plays both sides, 0 or 1 only that side's rows."""
+
+    def __init__(self, env, actor, player=-1, div=12, mod=11):
+        import torch
+        weights = rppo_weights(actor)
+        _check_input_width(weights[0], env)
+        if player not in (-1, 0, 1):
+            raise ValueError("player must be -1, 0 or 1, got %r" % (player,))
+        img1, img2, imgi, imgh, img3, bias, self.latent, self.out_dim = pack_rppo(*weights)
+        self.env, self.player, self.div, self.mod = env, int(player), int(div), int(mod)
+        dev = env.device
+        self._w = [torch.from_numpy(a).to(dev) for a in (img1, img2, imgi, imgh, img3, bias)]
+        shape = (env.num_envs, 2) if self.player < 0 else (env.num_envs,)
+        self.hidden = torch.zeros(shape + (self.latent,), dtype=torch.float32, device=dev)
+        self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
+        self.probs = torch.empty(shape + (_capi.MAX_ACTIONS, self.out_dim), dtype=torch.float32, device=dev)
+
+    def __call__(self, want_probs=False):
+        """Action rows int8 [N, 2, 7, 2] (env._actions); steps .hidden, fills .idx (int64 [N, 2, 7] or [N, 7]) and, with
+        want_probs, .probs (float32 [N, 2, 7, out] or [N, 7, out]: step k's distribution)."""
+        env = self.env
+        w1, w2, wi, wh, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_policy_rppo(env._h, C.c_void_p(env.obs.data_ptr()), self.player, w1, w2, wi, wh, w3, bias, self.latent,
+                                             self.out_dim, self.div, self.mod, C.c_void_p(self.hidden.data_ptr()),
+                                             C.c_void_p(env._actions.data_ptr()), C.c_void_p(self.idx.data_ptr()),
+                                             C.c_void_p(self.probs.data_ptr()) if want_probs else None, env._stream()))
         return env._actions

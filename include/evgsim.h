@@ -343,6 +343,34 @@ int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* 
                    const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions, int64_t* d_idx,
                    float* d_probs, void* stream);
 
+/* PPO's recurrent actor with its draws fused behind it, on the tensor cores (csrc/evg_policy_rppo.cu): the actor of
+ * agents/PPO/ActorCritic.py:33-60 with use_recurrent (act, :79-105), for the rows of `player` (0, 1, or -1 = both) of
+ * d_obs float32 [n_envs][2][obs_len], with its GRU state carried in d_hidden float32 [rows][latent] (rows = n_envs * 2
+ * for player -1, row 2 m + p; n_envs for one player), read and written back:
+ *     h = 0 if the match's resident record is at turn 0 (a reset, or an automatic reset under EVG_AUTORESET_TERMINAL /
+ *         _NEXT; under EVG_AUTORESET_OFF a finished match keeps its state until it is reset)
+ *     x = tanh(W2 tanh(W1 obs + b1) + b2)
+ *     for k = 0..6: one step of torch.nn.GRU(latent, latent) with input x (gates r, z, n in weight_ih_l0 / weight_hh_l0's
+ *         order: r = sigmoid(W_ir x + b_ir + W_hr h + b_hr), z likewise, n = tanh(W_in x + b_in + r * (W_hn h + b_hn)),
+ *         h = (1 - z) * n + z * h), probs_k = softmax(tanh(W3 h + b3)), idx_k = one draw from probs_k, action row k =
+ *         (idx_k / div, idx_k % mod) into d_actions int8 [n_envs][2][7][2] (only `player`'s rows).
+ * bf16 operands (observations, weights, x, and h as an MMA operand), fp32 accumulation; biases, gate arithmetic and the
+ * state h stay fp32.  Draw k uses uniform u_k of evg_policy_ppo's tape block pair (domain 3), one draw with replacement:
+ * the first j whose ascending fp32 prefix sum of probs_k exceeds u_k times their ascending sum (none: the last j).
+ *   d_idx (optional):   int64 [rows][7], the drawn indices.
+ *   d_probs (optional): float32 [rows][7][out_dim], the distributions the draws were made from.
+ * Images as for evg_policy_ppo (Lp = latent rounded up to 16, Ka = latent rounded up to 64): d_w1_img, d_w2_img,
+ * d_w3_img exactly as there, and
+ *     d_wi_img: weight_ih_l0 as three [Lp x Ka] blocks, gate g (r, z, n) at g * (Ka / 64) * Lp * 128 bytes
+ *     d_wh_img: weight_hh_l0 likewise
+ *     d_bias: float32 [2 * EVG_PPO_MAX_LATENT + EVG_PPO_OUT_PAD + 6 * EVG_PPO_MAX_LATENT] = b1, b2, b3 as for
+ *             evg_policy_ppo, then bias_ih_l0 gate g at 2 * EVG_PPO_MAX_LATENT + EVG_PPO_OUT_PAD + g * EVG_PPO_MAX_LATENT
+ *             and bias_hh_l0 gate g 3 * EVG_PPO_MAX_LATENT further, zero padded.
+ * evgsim.policy.pack_rppo builds them.  1 <= latent <= EVG_PPO_MAX_LATENT, 7 <= out_dim <= EVG_PPO_OUT_PAD. */
+int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_wi_img,
+                    const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
+                    float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream);
+
 /* Reward shaping of the reference's training scripts (utils/reward_shaping.py:17-56) on the step's outputs:
  * d_out float32 [n_envs][2].  turnNum (steps played before this one) is read from the observation's turn
  * field, so use it with EVG_AUTORESET_OFF or _TERMINAL (the observation of a finished match is the terminal one). */

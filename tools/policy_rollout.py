@@ -14,8 +14,9 @@ sampled per step (ActorCritic.act with use_recurrent, agents/PPO/ActorCritic.py:
 turn (forward, sampling, decode, step) in a CUDA graph.  The observation tensor the step kernel writes is consumed in place
 (a [N*2, 105] view, no copy, no dtype conversion kernel for fp32); the decoded int8 rows go straight back into the
 step.  --fused runs the network in libevgsim's tcgen05 kernels instead of torch: DQN's forward in evg_policy_mlp (then
-evg_decode_dqn), PPO's forward, sampling and unravel in evg_policy_ppo (its draws come from the simulator's tape, not from
-torch's generator).  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
+evg_decode_dqn), PPO's forward, sampling and unravel in evg_policy_ppo, the recurrent actor's head, GRU steps, draws
+and unravel in evg_policy_rppo, which also carries the hidden state and zeroes it when a match starts over (their draws
+come from the simulator's tape, not from torch's generator).  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
 """
 import argparse
 import json
@@ -79,7 +80,7 @@ def main():
     ap.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"])
     ap.add_argument("--graph", action="store_true", help="replay the turn (forward, decode, step) from a CUDA graph")
     ap.add_argument("--fused", action="store_true",
-                    help="dqn / ppo: the policy runs in libevgsim's fused tcgen05 kernels (evg_policy_mlp / evg_policy_ppo, bf16 operands) instead of torch")
+                    help="the policy runs in libevgsim's fused tcgen05 kernels (evg_policy_mlp / evg_policy_ppo / evg_policy_rppo, bf16 operands) instead of torch")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -93,13 +94,12 @@ def main():
     env = evgsim.BatchedEvergladesEnv(E, device=local, seed=0, auto_reset=evgsim._capi.AUTORESET_TERMINAL, env_id_offset=first)
     net = build_policy(args.policy, dtype, env.device)
     env.reset()
-    hidden = torch.zeros((1, 2 * E, 128), dtype=dtype, device=env.device) if args.policy == "rppo" else None
+    hidden = torch.zeros((1, 2 * E, 128), dtype=dtype, device=env.device) if args.policy == "rppo" and not args.fused else None
 
     fused = None
-    if args.fused:
-        assert args.policy in ("dqn", "ppo"), "--fused has kernels for the DQN network and the feed-forward PPO actor"
+    if args.fused:  # the recurrent actor's kernel keeps its own state (fused.hidden) and resets it at turn 0
         from evgsim import policy as evp
-        fused = evp.FusedDQN(env, net.float()) if args.policy == "dqn" else evp.FusedPPO(env, net.float())
+        fused = {"dqn": evp.FusedDQN, "ppo": evp.FusedPPO, "rppo": evp.FusedRPPO}[args.policy](env, net.float())
 
     def turn():
         env.step(fused() if fused is not None else policy_actions(env, net, args.policy, dtype, hidden))
@@ -135,7 +135,7 @@ def main():
     stats = evgsim.gather_episode_stats(env.episode_stats(), device=env.device) if world > 1 else env.episode_stats()
     if rank == 0:
         sec = float(ms.item()) / 1e3
-        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % ("evg_policy_mlp" if args.policy == "dqn" else "evg_policy_ppo") if args.fused else args.dtype, "fused_forward": bool(args.fused),
+        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % {"dqn": "evg_policy_mlp", "ppo": "evg_policy_ppo", "rppo": "evg_policy_rppo"}[args.policy] if args.fused else args.dtype, "fused_forward": bool(args.fused),
                           "cuda_graph": bool(args.graph),
                           "n_gpus": world, "envs_per_gpu": E, "turns": args.turns, "env_turns_per_s": E * world * args.turns / sec,
                           "ms_per_turn": sec * 1e3 / args.turns, "episodes": stats["episodes"], "wins": stats["wins"], "ties": stats["ties"]}))
