@@ -170,7 +170,10 @@ SYMBOLS = [
     ("evg_policy_mlp", C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
     ("evg_policy_ppo", C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     ("evg_policy_rppo", C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
-    ("evg_decode_dqn_layout", C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    ("evg_pack_mlp", C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
+    ("evg_pack_ppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    ("evg_pack_rppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_decode_dqn_layout",C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     ("evg_shape_reward", C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_step_kernel_kind", C.c_int, [_P]),
     ("evg_launch_count", C.c_int64, [_P]),

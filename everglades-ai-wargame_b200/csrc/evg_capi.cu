@@ -932,6 +932,66 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
     return EVG_OK;
 }
 
+int evg_pack_mlp(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, int32_t hidden, int32_t out_dim,
+                 void* d_w1_img, void* d_w2_img, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w1_img || !d_w2_img) return fail(EVG_E_ARG, "evg_pack_mlp: null argument");
+    if (sim->layout.obs_len >= EVG_MLP_IN_PAD) return fail(EVG_E_ARG, "evg_pack_mlp: observations of %d values + the bias input exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_MLP_IN_PAD);
+    if (hidden < 1 || hidden > 64 * EVG_MLP_CHUNK || out_dim < 1 || out_dim > EVG_MLP_OUT_PAD) return fail(EVG_E_ARG, "evg_pack_mlp: hidden %d / out_dim %d outside the kernel's tiling (hidden <= %d, out <= %d)", hidden, out_dim, 64 * EVG_MLP_CHUNK, EVG_MLP_OUT_PAD);
+    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img) % 16) return fail(EVG_E_ARG, "evg_pack_mlp: weight images must be 16-byte aligned");
+    cudaError_t e = evg::launch_pack_mlp(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, hidden, out_dim, d_w1_img, d_w2_img, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// evg_pack_ppo and evg_pack_rppo (w_ih != null): the checks of evg_policy_ppo / _rppo that concern the weights
+int pack_ppo_family(const char* fn, EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                    const float* d_b3, const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent,
+                    int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w3 || !d_b3 || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias)
+        return fail(EVG_E_ARG, "%s: null argument", fn);
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
+    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "%s: out_dim %d outside %d..%d", fn, out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
+    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img | (uintptr_t)d_wi_img | (uintptr_t)d_wh_img | (uintptr_t)d_w3_img | (uintptr_t)d_bias) % 16)
+        return fail(EVG_E_ARG, "%s: weight images and the bias vector must be 16-byte aligned", fn);
+    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "%s: observations of %d values exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    cudaError_t e = evg::launch_pack_ppo(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim,
+                                         d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int evg_pack_ppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
+                 int32_t latent, int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_w3_img, float* d_bias, void* stream)
+{
+    return pack_ppo_family("evg_pack_ppo", sim, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, nullptr, nullptr, nullptr, nullptr, latent, out_dim,
+                           d_w1_img, d_w2_img, nullptr, nullptr, d_w3_img, d_bias, stream);
+}
+
+int evg_pack_rppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
+                  const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent, int32_t out_dim,
+                  void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream)
+{
+    if (!d_w_ih || !d_b_ih || !d_w_hh || !d_b_hh || !d_wi_img || !d_wh_img) return fail(EVG_E_ARG, "evg_pack_rppo: null argument");
+    return pack_ppo_family("evg_pack_rppo", sim, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim,
+                           d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, stream);
+}
+
 int evg_shape_reward(EvgSim* sim, int32_t mode, const float* d_reward, const uint8_t* d_done, const float* d_obs, float* d_out,
                      void* stream)
 {

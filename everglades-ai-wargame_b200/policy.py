@@ -12,7 +12,8 @@ TMEM, bf16 operands, fp32 accumulation) on the observation tensor the step kerne
   ``FusedRPPO`` wraps a module with the reference ActorCritic's ``action_head``, ``action_gru`` and ``action_layer``.
 
 The images are what the kernels copy straight into shared memory (bf16, K-major, 128-byte swizzle; layout in
-include/evgsim.h).  Plumbing only; the networks themselves are the caller's.
+include/evgsim.h).  The constructors pack them on the host; each wrapper's ``refresh()`` re-packs them in place on the
+device (evg_pack_mlp / _ppo / _rppo) after an optimiser step.  Plumbing only; the networks themselves are the caller's.
 """
 from __future__ import annotations
 
@@ -90,15 +91,44 @@ def _check_input_width(w1, env):
         raise ValueError("the network takes %d inputs, the environment's observations have %d values" % (np.shape(w1)[1], env.obs_len))
 
 
+def _linear_params(net, n, expected):
+    """(weight, bias) of each of the `n` nn.Linear layers of a Sequential, in order."""
+    import torch
+    lin = [m for m in net if isinstance(m, torch.nn.Linear)]
+    assert len(lin) == n, "expected " + expected
+    return [t for m in lin for t in (m.weight, m.bias)]
+
+
+def _host_arrays(params):
+    return [t.detach().float().cpu().numpy() for t in params]
+
+
+def _refresh_sources(fused, net, params_of, shapes):
+    """The parameters `refresh` packs from, as device pointers: ValueError, before anything is launched, unless each is
+    a contiguous float32 tensor on the env's device of exactly the shape the wrapper's images were sized for."""
+    import torch
+    net = fused._net if net is None else net
+    if net is None:
+        raise ValueError("this wrapper was built from weights= arrays: pass the module to refresh(net)")
+    params = params_of(net)
+    env = fused.env
+    for i, (t, shape) in enumerate(zip(params, shapes)):
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != env.device:
+            raise ValueError("parameter %d must be a contiguous float32 tensor on %s, got %s%s on %s"
+                             % (i, env.device, t.dtype, "" if t.is_contiguous() else " (not contiguous)", t.device))
+        if tuple(t.shape) != shape:
+            raise ValueError("parameter %d has shape %s, the wrapper's images were built for %s" % (i, tuple(t.shape), shape))
+    return [C.c_void_p(t.data_ptr()) for t in params]
+
+
 class FusedDQN:
     """Q-network forward + decode for a BatchedEvergladesEnv: ``actions = FusedDQN(env, net)()`` reads env.obs in place."""
 
     def __init__(self, env, net=None, weights=None):
         import torch
+        self._net = net if weights is None else None
         if weights is None:
-            lin = [m for m in net if isinstance(m, torch.nn.Linear)]
-            assert len(lin) == 2, "expected Sequential(Linear, ReLU, Linear)"
-            weights = [t.detach().float().cpu().numpy() for t in (lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias)]
+            weights = _host_arrays(self._params(net))
         _check_input_width(weights[0], env)
         img1, img2, self.hidden, self.out_dim = pack_mlp(*weights)
         self.env = env
@@ -107,6 +137,23 @@ class FusedDQN:
         self._w2 = torch.from_numpy(img2).to(dev)
         self.q = torch.empty((env.num_envs, 2, self.out_dim), dtype=torch.float32, device=dev)
         self.qt = torch.empty((self.out_dim, env.num_envs * 2), dtype=torch.float32, device=dev)
+
+    @staticmethod
+    def _params(net):
+        return _linear_params(net, 2, "Sequential(Linear, ReLU, Linear)")
+
+    def refresh(self, net=None):
+        """Re-pack the weight images in place from `net` (default: the module this wrapper was built with), on the device:
+        one kernel on the env's current stream, no allocation, no host synchronisation; the images are byte for byte
+        those the constructor would build.  Call it after each optimiser step.  It can be captured in a CUDA graph, which
+        then holds the parameters' addresses: it stays valid across in-place updates (optimizer.step(), load_state_dict),
+        while replacing a parameter tensor needs a new capture.  The parameters must be contiguous float32 tensors on the
+        env's device, of the shapes the wrapper was built with (ValueError otherwise, before anything is launched)."""
+        h, o, w = self.hidden, self.out_dim, self.env.obs_len
+        w1, b1, w2, b2 = _refresh_sources(self, net, self._params, [(h, w), (h,), (o, h), (o,)])
+        env = self.env
+        _capi.check(env._lib.evg_pack_mlp(env._h, w1, b1, w2, b2, h, o, C.c_void_p(self._w1.data_ptr()),
+                                          C.c_void_p(self._w2.data_ptr()), env._stream()))
 
     def _run(self, obs, out, transposed):
         env = self.env
@@ -182,10 +229,9 @@ class FusedPPO:
 
     def __init__(self, env, net=None, weights=None, player=-1, latent=None, div=12, mod=11):
         import torch
+        self._net = net if weights is None else None
         if weights is None:
-            lin = [m for m in net if isinstance(m, torch.nn.Linear)]
-            assert len(lin) == 3, "expected Sequential(Linear, Tanh, Linear, Tanh, Linear, Tanh, Softmax)"
-            weights = [t.detach().float().cpu().numpy() for m in lin for t in (m.weight, m.bias)]
+            weights = _host_arrays(self._params(net))
         _check_input_width(weights[0], env)
         img1, img2, img3, bias, self.latent, self.out_dim = pack_ppo(*weights)
         assert latent is None or latent == self.latent, "latent %s != the weights' %d" % (latent, self.latent)
@@ -196,6 +242,19 @@ class FusedPPO:
         shape = (env.num_envs, 2) if self.player < 0 else (env.num_envs,)
         self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
         self.probs = torch.empty(shape + (self.out_dim,), dtype=torch.float32, device=dev)
+
+    @staticmethod
+    def _params(net):
+        return _linear_params(net, 3, "Sequential(Linear, Tanh, Linear, Tanh, Linear, Tanh, Softmax)")
+
+    def refresh(self, net=None):
+        """Re-pack the weight images and the bias vector in place from `net` (default: the module this wrapper was built
+        with), on the device; see FusedDQN.refresh (CUDA graphs, the ValueError checks)."""
+        L, o, w = self.latent, self.out_dim, self.env.obs_len
+        src = _refresh_sources(self, net, self._params, [(L, w), (L,), (L, L), (L,), (o, L), (o,)])
+        env = self.env
+        w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_pack_ppo(env._h, *src, L, o, w1, w2, w3, bias, env._stream()))
 
     def __call__(self, want_probs=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); fills .idx (int64 [N, 2, 7] or [N, 7]) and, with want_probs,
@@ -213,6 +272,11 @@ def rppo_weights(actor):
     """(w1, b1, w2, b2, w_ih, b_ih, w_hh, b_hh, w3, b3) float32 numpy arrays of a module with the reference ActorCritic's
     action_head (Linear, Tanh, Linear, Tanh), action_gru and action_layer (Linear, Tanh, Softmax).  ValueError for a GRU
     the kernel does not run: more than one layer, bidirectional, an input width other than the hidden width, no biases."""
+    return _host_arrays(_rppo_params(actor))
+
+
+def _rppo_params(actor):
+    """rppo_weights' parameters as the module's own tensors, after its checks."""
     import torch
     gru = actor.action_gru
     if gru.num_layers != 1 or gru.bidirectional or gru.input_size != gru.hidden_size or not gru.bias:
@@ -228,9 +292,8 @@ def rppo_weights(actor):
         raise ValueError("the GRU's width %d is outside 1..%d" % (latent, PPO_MAX_LATENT))
     if head[1].weight.shape[0] != latent:
         raise ValueError("the head's output width %d is not the GRU's %d" % (head[1].weight.shape[0], latent))
-    ts = (head[0].weight, head[0].bias, head[1].weight, head[1].bias, gru.weight_ih_l0, gru.bias_ih_l0, gru.weight_hh_l0,
-          gru.bias_hh_l0, out[0].weight, out[0].bias)
-    return [t.detach().float().cpu().numpy() for t in ts]
+    return [head[0].weight, head[0].bias, head[1].weight, head[1].bias, gru.weight_ih_l0, gru.bias_ih_l0, gru.weight_hh_l0,
+            gru.bias_hh_l0, out[0].weight, out[0].bias]
 
 
 def pack_rppo(w1, b1, w2, b2, w_ih, b_ih, w_hh, b_hh, w3, b3):
@@ -298,6 +361,7 @@ class FusedRPPO:
     def __init__(self, env, actor, player=-1, div=12, mod=11):
         import torch
         weights = rppo_weights(actor)
+        self._net = actor
         _check_input_width(weights[0], env)
         if player not in (-1, 0, 1):
             raise ValueError("player must be -1, 0 or 1, got %r" % (player,))
@@ -309,6 +373,18 @@ class FusedRPPO:
         self.hidden = torch.zeros(shape + (self.latent,), dtype=torch.float32, device=dev)
         self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
         self.probs = torch.empty(shape + (_capi.MAX_ACTIONS, self.out_dim), dtype=torch.float32, device=dev)
+
+    def refresh(self, actor=None):
+        """Re-pack the weight images and the bias vector in place from `actor` (default: the module this wrapper was built
+        with), on the device; .hidden is left as it is.  ValueError for a GRU the kernel does not run (as the constructor),
+        otherwise as FusedDQN.refresh (CUDA graphs, the checks)."""
+        L, o, w = self.latent, self.out_dim, self.env.obs_len
+        w1, b1, w2, b2, wi, bi, wh, bh, w3, b3 = _refresh_sources(
+            self, actor, _rppo_params, [(L, w), (L,), (L, L), (L,), (3 * L, L), (3 * L,), (3 * L, L), (3 * L,), (o, L), (o,)])
+        env = self.env
+        i1, i2, ii, ih, i3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_pack_rppo(env._h, w1, b1, w2, b2, w3, b3, wi, bi, wh, bh, L, o, i1, i2, ii, ih, i3, bias,
+                                           env._stream()))
 
     def __call__(self, want_probs=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); steps .hidden, fills .idx (int64 [N, 2, 7] or [N, 7]) and, with

@@ -371,6 +371,27 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
                     const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
                     float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream);
 
+/* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
+ * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo build on the host: one launch on `stream`, no host synchronisation,
+ * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
+ * Sources are device arrays in torch's layouts (contiguous, row-major): d_w1 [hidden or latent][obs_len], d_w2 / d_w3
+ * [out][in] as nn.Linear.weight, biases [out]; d_w_ih / d_w_hh [3 * latent][latent] and d_b_ih / d_b_hh [3 * latent] as
+ * nn.GRU's weight_ih_l0 ... (gates r, z, n).  The input width is the simulator's obs_len, the one the forward kernels read.
+ *   evg_pack_mlp:  d_w1_img / d_w2_img as evg_policy_mlp reads them (W1' = [W1 | b1] plus the unit of ones, W2' = [W2 | b2],
+ *                  ceil((hidden + 1) / EVG_MLP_CHUNK) chunks each).
+ *   evg_pack_ppo:  d_w1_img, d_w2_img, d_w3_img and d_bias as evg_policy_ppo reads them.
+ *   evg_pack_rppo: the same, plus d_wi_img / d_wh_img and the GRU biases in d_bias as evg_policy_rppo reads them.
+ * Every byte of every image and of d_bias is written, zero padding included.  Weights round to bf16 to nearest even
+ * (overflow to +-Inf, subnormals kept); a NaN packs to a bf16 NaN of unspecified payload.  Images and d_bias must be
+ * 16-byte aligned; hidden, latent, out_dim and obs_len are checked as the matching evg_policy_* checks them. */
+int evg_pack_mlp(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, int32_t hidden, int32_t out_dim,
+                 void* d_w1_img, void* d_w2_img, void* stream);
+int evg_pack_ppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
+                 int32_t latent, int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_w3_img, float* d_bias, void* stream);
+int evg_pack_rppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
+                  const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent, int32_t out_dim,
+                  void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream);
+
 /* Reward shaping of the reference's training scripts (utils/reward_shaping.py:17-56) on the step's outputs:
  * d_out float32 [n_envs][2].  turnNum (steps played before this one) is read from the observation's turn
  * field, so use it with EVG_AUTORESET_OFF or _TERMINAL (the observation of a finished match is the terminal one). */
