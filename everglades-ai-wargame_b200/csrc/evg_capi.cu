@@ -351,7 +351,9 @@ int evg_create(const EvgConfig* cfg, int64_t n_envs, uint64_t seed, int64_t env_
         }
     }
     s->sm_count = prop.multiProcessorCount;
-    if ((e = evg::set_step_smem(s->smem)) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
+    // the shared-memory opt-ins are per device: made on the simulator's, for the step and the policy kernels
+    if ((e = evg::set_step_smem(s->smem)) != cudaSuccess || (e = evg::set_policy_mlp_smem()) != cudaSuccess || (e = evg::set_policy_ppo_smem()) != cudaSuccess ||
+        (e = evg::set_policy_rppo_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
     int per_sm = 0;
     if ((e = evg::step_occupancy(t, s->smem, &per_sm)) != cudaSuccess || per_sm < 1) { delete s; return cuda_fail(e, "occupancy query"); }
     // persistent CTAs: a whole number of resident waves, never more CTAs than matches need
@@ -488,6 +490,44 @@ int check_fmt(const EvgSim* sim, int32_t format, const void* rows, const float* 
         if (sim->cfg.turn_limit > 32767) return fail(EVG_E_ARG, "%s: EVG_OBS_I16 cannot carry a turn counter up to %d", who, sim->cfg.turn_limit);
     }
     if (rows && (uintptr_t)rows % 16) return fail(EVG_E_ARG, "%s: observation rows must be 16-byte aligned", who);
+    return EVG_OK;
+}
+
+// evg_policy_mlp's and evg_pack_mlp's checks: the observations, the network's shape and the images fit the kernel
+int check_mlp_shape(const char* fn, const EvgSim* sim, int32_t hidden, int32_t out_dim, const void* d_w1_img, const void* d_w2_img)
+{
+    if (sim->layout.obs_len >= EVG_MLP_IN_PAD) return fail(EVG_E_ARG, "%s: observations of %d values + the bias input exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_MLP_IN_PAD);
+    if (hidden < 1 || hidden > 64 * EVG_MLP_CHUNK || out_dim < 1 || out_dim > EVG_MLP_OUT_PAD)
+        return fail(EVG_E_ARG, "%s: hidden %d / out_dim %d outside the kernel's tiling (hidden <= %d, out <= %d)", fn, hidden, out_dim, 64 * EVG_MLP_CHUNK, EVG_MLP_OUT_PAD);
+    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img) % 16) return fail(EVG_E_ARG, "%s: weight images must be 16-byte aligned", fn);
+    return EVG_OK;
+}
+
+// the same checks for the PPO actors (evg_policy_ppo / _rppo, evg_pack_ppo / _rppo); `aligned`: what the call reads in 16 B
+int check_actor_shape(const char* fn, const EvgSim* sim, int32_t latent, int32_t out_dim, std::initializer_list<const void*> aligned)
+{
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
+    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "%s: out_dim %d outside %d..%d", fn, out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
+    for (const void* p : aligned)
+        if ((uintptr_t)p % 16) return fail(EVG_E_ARG, "%s: weight images (and a packed bias vector) must be 16-byte aligned", fn);
+    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "%s: observations of %d values exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    return EVG_OK;
+}
+
+// evg_pack_ppo and evg_pack_rppo (w_ih != null): the weights of evg_policy_ppo / _rppo
+int pack_ppo_family(const char* fn, EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                    const float* d_b3, const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent,
+                    int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w3 || !d_b3 || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias)
+        return fail(EVG_E_ARG, "%s: null argument", fn);
+    if ((rc = check_actor_shape(fn, sim, latent, out_dim, {d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias}))) return rc;
+    cudaError_t e = evg::launch_pack_ppo(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim,
+                                         d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
     return EVG_OK;
 }
 
@@ -878,9 +918,7 @@ int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_
     int rc = check_sim(sim, false);
     if (rc) return rc;
     if (!d_obs || !d_w1_img || !d_w2_img || !d_q || rows < 0) return fail(EVG_E_ARG, "evg_policy_mlp: null argument");
-    if (sim->layout.obs_len >= EVG_MLP_IN_PAD) return fail(EVG_E_ARG, "evg_policy_mlp: observations of %d values + the bias input exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_MLP_IN_PAD);
-    if (hidden < 1 || hidden > 64 * EVG_MLP_CHUNK || out_dim < 1 || out_dim > EVG_MLP_OUT_PAD) return fail(EVG_E_ARG, "evg_policy_mlp: hidden %d / out_dim %d outside the kernel's tiling (out <= %d)", hidden, out_dim, EVG_MLP_OUT_PAD);
-    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img) % 16) return fail(EVG_E_ARG, "evg_policy_mlp: weight images must be 16-byte aligned");
+    if ((rc = check_mlp_shape("evg_policy_mlp", sim, hidden, out_dim, d_w1_img, d_w2_img))) return rc;
     const int n_chunks = (hidden + 1 + EVG_MLP_CHUNK - 1) / EVG_MLP_CHUNK;  // + the hidden unit that carries b2
     cudaError_t e = evg::launch_policy_mlp(d_obs, rows, sim->layout.obs_len, d_w1_img, d_w2_img, n_chunks, out_dim, d_q, q_transposed, sim->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_mlp_kernel launch");
@@ -896,11 +934,8 @@ int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* 
     if (rc) return rc;
     if (!d_obs || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias || !d_actions) return fail(EVG_E_ARG, "evg_policy_ppo: null argument");
     if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_ppo: player %d outside -1..1", player);
-    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "evg_policy_ppo: latent %d outside 1..%d", latent, EVG_PPO_MAX_LATENT);
-    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "evg_policy_ppo: out_dim %d outside %d..%d", out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
     if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_ppo: div %d / mod %d must be positive", div, mod);
-    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img | (uintptr_t)d_w3_img) % 16) return fail(EVG_E_ARG, "evg_policy_ppo: weight images must be 16-byte aligned");
-    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "evg_policy_ppo: observations of %d values exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    if ((rc = check_actor_shape("evg_policy_ppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_w3_img}))) return rc;
     cudaError_t e = evg::launch_policy_ppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
                                            d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx, d_probs, sim->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_ppo_kernel launch");
@@ -918,12 +953,8 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
         return fail(EVG_E_ARG, "evg_policy_rppo: null argument");
     if (!d_hidden) return fail(EVG_E_ARG, "evg_policy_rppo: d_hidden (the GRU state, in and out) is null");
     if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_rppo: player %d outside -1..1", player);
-    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "evg_policy_rppo: latent %d outside 1..%d", latent, EVG_PPO_MAX_LATENT);
-    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "evg_policy_rppo: out_dim %d outside %d..%d", out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
     if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_rppo: div %d / mod %d must be positive", div, mod);
-    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img | (uintptr_t)d_wi_img | (uintptr_t)d_wh_img | (uintptr_t)d_w3_img) % 16)
-        return fail(EVG_E_ARG, "evg_policy_rppo: weight images must be 16-byte aligned");
-    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "evg_policy_rppo: observations of %d values exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    if ((rc = check_actor_shape("evg_policy_rppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img}))) return rc;
     cudaError_t e = evg::launch_policy_rppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
                                             d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_hidden, d_actions, d_idx, d_probs,
                                             sim->sm_count, (cudaStream_t)stream);
@@ -938,43 +969,12 @@ int evg_pack_mlp(EvgSim* sim, const float* d_w1, const float* d_b1, const float*
     int rc = check_sim(sim, false);
     if (rc) return rc;
     if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w1_img || !d_w2_img) return fail(EVG_E_ARG, "evg_pack_mlp: null argument");
-    if (sim->layout.obs_len >= EVG_MLP_IN_PAD) return fail(EVG_E_ARG, "evg_pack_mlp: observations of %d values + the bias input exceed the %d the kernel is tiled for", sim->layout.obs_len, EVG_MLP_IN_PAD);
-    if (hidden < 1 || hidden > 64 * EVG_MLP_CHUNK || out_dim < 1 || out_dim > EVG_MLP_OUT_PAD) return fail(EVG_E_ARG, "evg_pack_mlp: hidden %d / out_dim %d outside the kernel's tiling (hidden <= %d, out <= %d)", hidden, out_dim, 64 * EVG_MLP_CHUNK, EVG_MLP_OUT_PAD);
-    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img) % 16) return fail(EVG_E_ARG, "evg_pack_mlp: weight images must be 16-byte aligned");
+    if ((rc = check_mlp_shape("evg_pack_mlp", sim, hidden, out_dim, d_w1_img, d_w2_img))) return rc;
     cudaError_t e = evg::launch_pack_mlp(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, hidden, out_dim, d_w1_img, d_w2_img, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
     sim->launches += 1;
     return EVG_OK;
 }
-
-}  // extern "C"
-
-namespace {
-
-// evg_pack_ppo and evg_pack_rppo (w_ih != null): the checks of evg_policy_ppo / _rppo that concern the weights
-int pack_ppo_family(const char* fn, EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
-                    const float* d_b3, const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent,
-                    int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream)
-{
-    int rc = check_sim(sim, false);
-    if (rc) return rc;
-    if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w3 || !d_b3 || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias)
-        return fail(EVG_E_ARG, "%s: null argument", fn);
-    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
-    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "%s: out_dim %d outside %d..%d", fn, out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
-    if (((uintptr_t)d_w1_img | (uintptr_t)d_w2_img | (uintptr_t)d_wi_img | (uintptr_t)d_wh_img | (uintptr_t)d_w3_img | (uintptr_t)d_bias) % 16)
-        return fail(EVG_E_ARG, "%s: weight images and the bias vector must be 16-byte aligned", fn);
-    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "%s: observations of %d values exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
-    cudaError_t e = evg::launch_pack_ppo(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim,
-                                         d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
-    sim->launches += 1;
-    return EVG_OK;
-}
-
-}  // namespace
-
-extern "C" {
 
 int evg_pack_ppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
                  int32_t latent, int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_w3_img, float* d_bias, void* stream)

@@ -1,5 +1,6 @@
-// evg_internal.h — device tables, resident record layout and launcher prototypes shared by
-// evg_kernels.cu (sm_100a kernels) and evg_capi.cu (the C ABI of include/evgsim.h).
+// evg_internal.h — device tables, resident record layout, the tape's Philox and launcher prototypes, shared by every
+// translation unit: the kernels (evg_kernels.cu, evg_step_tpm.cu, evg_policy_*.cu, through evg_tcgen05.cuh for the
+// tensor-core ones) and evg_capi.cu (the C ABI of include/evgsim.h).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -173,6 +174,10 @@ cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const f
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
                                int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
                                cudaStream_t stream);
+// the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
+cudaError_t set_policy_mlp_smem();
+cudaError_t set_policy_ppo_smem();
+cudaError_t set_policy_rppo_smem();
 // weight images of the three policy kernels from the float32 parameters (evg_policy_pack.cu); launch_pack_ppo packs the
 // recurrent actor's GRU as well when w_ih is not null
 cudaError_t launch_pack_mlp(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, int hidden, int out_dim,

@@ -35,9 +35,7 @@ namespace evg {
 
 namespace {
 
-constexpr int kMlpThreads = 512;
-constexpr int kTileM = 128;   // observation rows per tile
-constexpr int kInPad = 128;   // input features, padded (obs_len <= 128)
+constexpr int kInPad = kObsCols;  // input features, padded (obs_len < 128: the bias input behind them)
 constexpr int kChunk = 192;   // hidden units per chunk: 3 swizzle atoms of 64
 constexpr int kOutPad = 144;  // outputs, padded to a multiple of 16 (12 groups x 11 nodes = 132)
 
@@ -52,11 +50,10 @@ constexpr int kW1ChunkBytes = (kInPad / kAtomK) * kChunk * 128;    // 49152
 constexpr int kW2ChunkBytes = (kChunk / kAtomK) * kOutPad * 128;   // 55296
 static_assert(kSmH % 1024 == 0 && kSmW1 % 1024 == 0 && kSmW2 % 1024 == 0 && (kOutPad * 128) % 1024 == 0 && (kChunk * 128) % 1024 == 0, "swizzle atoms must be 1024-byte aligned");
 
-constexpr int kTmemCols = 512;  // power of two >= D1 (192) + D2 (144) columns
-constexpr int kTmemD1 = 0, kTmemD2 = 256;
+constexpr int kTmemD1 = 0, kTmemD2 = 256;  // D1 (192 columns) and D2 (144) in the 512 of kTmemCols
 
 // q_col_stride == 1: Q[row * q_row_stride + col] (row-major); q_row_stride == 1: Q[col * q_col_stride + row] (transposed)
-__global__ void __launch_bounds__(kMlpThreads, 1)
+__global__ void __launch_bounds__(kCtaThreads, 1)
 evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, const unsigned char* __restrict__ w1_img,
                       const unsigned char* __restrict__ w2_img, int n_chunks, int out_dim, float* __restrict__ q, int64_t q_row_stride,
                       int64_t q_col_stride)
@@ -64,20 +61,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kSmBar);  // [0] layer-1 MMAs done, [1] layer-2 MMAs done, [2] W1 image landed, [3] W2 image landed
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + kSmBar + 32);
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&bar[i])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {  // one warp allocates the tensor memory (and frees it at the end)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
+    const uint32_t tmem = cta_setup<4>(tid, bar, reinterpret_cast<uint32_t*>(smem + kSmBar + 32));
     // my row = TMEM lane 32 * (warp % 4) + lane (a warp reaches the lane quarter warp % 4); my quarter of the columns = warp / 4
     const int r = (warp & 3) * 32 + lane, quarter = warp >> 2;
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
@@ -91,36 +75,16 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
         bulk_load(smem + kSmW1, w1_img, kW1ChunkBytes, &bar[2]);
         bulk_load(smem + kSmW2, w2_img, kW2ChunkBytes, &bar[3]);
     }
-    // A: a tile's observations -> bf16, swizzled.  Every thread owns 4 of the tile's 2048 16-byte chunks (8 features each):
-    // all 32 loads are issued together into registers (one DRAM round trip), converted and stored later; feature
-    // `in_dim` is the constant 1 that carries the bias, rows and features beyond that are zero.
-    float af[kTileM * (kInPad / 8) / kMlpThreads][8];
-    auto load_a = [&](int64_t row0, int nrows) {
-#pragma unroll
-        for (int it = 0; it < kTileM * (kInPad / 8) / kMlpThreads; ++it) {
-            const int i = tid + it * kMlpThreads, ar = i >> 4, k0 = (i & 15) * 8;
-            const float* src = obs + (row0 + ar) * in_dim + k0;
-#pragma unroll
-            for (int e = 0; e < 8; ++e) af[it][e] = (ar < nrows && k0 + e < in_dim) ? __ldcs(src + e) : (k0 + e == in_dim ? 1.f : 0.f);
-        }
-    };
-    auto store_a = [&]() {
-#pragma unroll
-        for (int it = 0; it < kTileM * (kInPad / 8) / kMlpThreads; ++it) {
-            const int i = tid + it * kMlpThreads, ar = i >> 4, k0 = (i & 15) * 8;
-            *reinterpret_cast<uint4*>(smem + kSmA + swz_offset(kTileM, ar, k0)) =
-                make_uint4(pack_bf16(af[it][0], af[it][1]), pack_bf16(af[it][2], af[it][3]), pack_bf16(af[it][4], af[it][5]), pack_bf16(af[it][6], af[it][7]));
-        }
-    };
+    ObsTile<true> a_tile;  // A: feature in_dim is the constant 1 that carries b1
     int64_t step = 0;
     bool l1_queued = false;  // the coming tile's first layer-1 MMAs were issued at the end of the previous tile
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int64_t row0 = tile * kTileM;
         const int nrows = rows - row0 < kTileM ? (int)(rows - row0) : kTileM;
         if (tile == (int64_t)blockIdx.x) {  // the first tile: later ones are fetched and converted under the previous tile's last chunk
-            load_a(row0, nrows);
-            store_a();
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the tensor core's reads
+            a_tile.load(tid, obs, row0, rows, in_dim, -1);
+            a_tile.store(tid, smem + kSmA);
+            fence_async_smem();
             __syncthreads();
         }
         for (int c = 0; c < n_chunks; ++c, ++step) {
@@ -129,7 +93,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             // ones are queued right behind the previous chunk's layer 2 (below), so that their latency is not paid again
             auto issue_layer1 = [&](uint32_t parity) {
                 mbar_wait(&bar[2], parity);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
 #pragma unroll
                 for (int k = 0; k < kInPad / 16; ++k) {  // within a swizzle atom the start address advances by 32 bytes per K = 16
                     const uint32_t offA = (k >> 2) * (kTileM * 128) + (k & 3) * 32, offB = (k >> 2) * (kChunk * 128) + (k & 3) * 32;
@@ -142,13 +106,10 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             ph_w1 ^= 1;
             mbar_wait(&bar[0], ph_m1);  // D1 complete (and, the tensor pipe being in order, the previous step's layer 2: H is free)
             ph_m1 ^= 1;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             if (tid == 0 && step + 1 < n_steps) bulk_load(smem + kSmW1, w1_img + (size_t)cn * kW1ChunkBytes, kW1ChunkBytes, &bar[2]);
             const bool fetch_next_a = c + 1 == n_chunks && tile + gridDim.x < n_tiles;  // this tile's last layer-1 MMAs have read A: it is free
-            if (fetch_next_a) {
-                const int64_t nrow0 = (tile + gridDim.x) * kTileM;
-                load_a(nrow0, rows - nrow0 < kTileM ? (int)(rows - nrow0) : kTileM);  // in flight under the epilogue below
-            }
+            if (fetch_next_a) a_tile.load(tid, obs, (tile + gridDim.x) * kTileM, rows, in_dim, -1);  // in flight under the epilogue below
             // ---- hidden activations of my row, my 48 of the chunk's 192 columns: TMEM -> registers -> ReLU, bf16 -> swizzled H
             {
                 constexpr int kLd = kChunk / 4 / 16;  // tensor-memory loads of 16 columns per thread: all issued, then one wait
@@ -156,7 +117,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
                 const int jq1 = quarter * (kChunk / 4);
 #pragma unroll
                 for (int t = 0; t < kLd; ++t) tmem_ld16(lane_base + kTmemD1 + jq1 + 16 * t, v[t]);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                tmem_wait_ld();
 #pragma unroll
                 for (int t = 0; t < kLd; ++t) {
 #pragma unroll
@@ -169,13 +130,13 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
                     }
                 }
             }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            fence_async_smem();
+            tc_fence_before();
             __syncthreads();
             // ---- layer 2: D2 += H . W2c^T
             if (tid == 0) {
                 mbar_wait(&bar[3], ph_w2);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
 #pragma unroll
                 for (int k = 0; k < kChunk / 16; ++k) {
                     const uint32_t offA = (k >> 2) * (kTileM * 128) + (k & 3) * 32, offB = (k >> 2) * (kOutPad * 128) + (k & 3) * 32;
@@ -188,8 +149,8 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             }
             ph_w2 ^= 1;
             if (fetch_next_a) {  // the next tile's A, converted while layer 2 runs
-                store_a();
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                a_tile.store(tid, smem + kSmA);
+                fence_async_smem();
                 __syncthreads();
                 // ... and its first layer-1 MMAs queued now: they only write D1, so they run under this tile's Q store
                 if (tid == 0) issue_layer1(ph_w1);
@@ -197,7 +158,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             }
             mbar_wait(&bar[1], ph_m2);  // the W2 buffer is free again; after the last chunk D2 is complete
             ph_m2 ^= 1;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             if (tid == 0 && step + 1 < n_steps) bulk_load(smem + kSmW2, w2_img + (size_t)cn * kW2ChunkBytes, kW2ChunkBytes, &bar[3]);
         }
         // ---- Q = D2: my row, my quarter of the columns (36 = 16 + 16 + 4)
@@ -208,8 +169,8 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             uint32_t v[2][16], v4[4];
             tmem_ld16(lane_base + kTmemD2 + jq, v[0]);
             tmem_ld16(lane_base + kTmemD2 + jq + 16, v[1]);
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n" : "=r"(v4[0]), "=r"(v4[1]), "=r"(v4[2]), "=r"(v4[3]) : "r"(lane_base + kTmemD2 + jq + 32));
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_ld4(lane_base + kTmemD2 + jq + 32, v4);
+            tmem_wait_ld();
 #pragma unroll
             for (int j0 = 0; j0 < 32; j0 += 16) {
 #pragma unroll
@@ -220,10 +181,10 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             for (int e = 0; e < 4; ++e, qp += q_col_stride)
                 if (live && jq + 32 + e < out_dim) *qp = __uint_as_float(v4[e]);
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncthreads();  // the next tile's first MMAs overwrite D1 / D2, its conversion overwrites A
     }
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols));
+    cta_teardown(tid, tmem);
 }
 
 }  // namespace
@@ -231,19 +192,11 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
 cudaError_t launch_policy_mlp(const float* obs, int64_t rows, int in_dim, const void* w1_img, const void* w2_img, int n_chunks, int out_dim, float* q,
                               int transposed, int sm_count, cudaStream_t stream)
 {
-    if (rows <= 0) return cudaSuccess;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(evg_policy_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
-        if (e != cudaSuccess) return e;
-        attr_set = true;
-    }
-    const int64_t tiles = (rows + kTileM - 1) / kTileM;
-    const unsigned grid = (unsigned)(tiles < sm_count ? tiles : sm_count);
-    evg_policy_mlp_kernel<<<grid, kMlpThreads, kSmBytes, stream>>>(obs, rows, in_dim, reinterpret_cast<const unsigned char*>(w1_img),
-                                                                   reinterpret_cast<const unsigned char*>(w2_img), n_chunks, out_dim, q,
-                                                                   transposed ? 1 : out_dim, transposed ? rows : 1);
-    return cudaGetLastError();
+    return launch_persistent(evg_policy_mlp_kernel, rows, sm_count, kSmBytes, stream, obs, rows, in_dim, reinterpret_cast<const unsigned char*>(w1_img),
+                             reinterpret_cast<const unsigned char*>(w2_img), n_chunks, out_dim, q, (int64_t)(transposed ? 1 : out_dim),
+                             (int64_t)(transposed ? rows : 1));
 }
+
+cudaError_t set_policy_mlp_smem() { return cudaFuncSetAttribute(evg_policy_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
 
 }  // namespace evg

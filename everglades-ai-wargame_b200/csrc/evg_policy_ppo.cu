@@ -37,8 +37,6 @@ namespace evg {
 
 namespace {
 
-constexpr int kPpoThreads = 512;
-constexpr int kTileM = 128;                 // observation rows per tile
 constexpr int kInPad = EVG_PPO_IN_PAD;      // input features, padded (obs_len < 128)
 constexpr int kMaxL = EVG_PPO_MAX_LATENT;   // latent width bound: 4 swizzle atoms of H, N <= 256 per MMA
 constexpr int kOutPad = EVG_PPO_OUT_PAD;    // outputs, padded to a multiple of 16 (132 -> 144)
@@ -57,49 +55,21 @@ static_assert(kSmH % 1024 == 0 && kSmW % 1024 == 0 && kSlotBytes % 1024 == 0 && 
 static_assert(kOutPad * kTileM * 4 <= kSmW, "the probabilities must fit over A and H");
 static_assert(kSmBytes <= 227 * 1024, "shared memory");
 
-constexpr int kTmemCols = 512;
 constexpr int kTmemD1 = 0, kTmemD2 = 256;  // D3 reuses D1's columns (read out before layer 3 is issued)
 
-struct PpoArgs {
-    const float* obs;
-    const unsigned char* w1;
-    const unsigned char* w2;
-    const unsigned char* w3;
-    const float* bias;
-    const uint32_t* records;
-    int8_t* actions;
-    int64_t* idx;
-    float* probs;
-    int64_t rows;  // n_envs * (player < 0 ? 2 : 1)
-    int player, in_dim, lp, nk, out_dim, div, mod, rec_words;
-    uint32_t env_base, seed_lo, seed_hi;
-};
-
-__global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __grid_constant__ PpoArgs a)
+// nk: chunks of 128 K-columns of layers 2 and 3
+__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __grid_constant__ ActorArgs a, const int nk)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kSmBar);  // [0] / [1] weight slot 0 / 1 landed, [2] a layer's MMAs done
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + kSmBar + 24);
     float* sb = reinterpret_cast<float*>(smem + kSmBias);
     float* ps = reinterpret_cast<float*>(smem + kSmP);
-    for (int i = tid; i < kBiasFloats; i += kPpoThreads) sb[i] = a.bias[i];
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&bar[i])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
+    for (int i = tid; i < kBiasFloats; i += kCtaThreads) sb[i] = a.bias[i];
+    const uint32_t tmem = cta_setup<3>(tid, bar, reinterpret_cast<uint32_t*>(smem + kSmBar + 24));
     const int r = (warp & 3) * 32 + lane, quarter = warp >> 2;
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    const int lp = a.lp, nk = a.nk, n_pieces = 1 + 2 * nk;
+    const int lp = a.lp, n_pieces = 1 + 2 * nk;
     const uint32_t idesc_l = make_idesc(kTileM, lp), idesc_o = make_idesc(kTileM, kOutPad);
     const uint32_t sA = smem_u32(smem + kSmA), sH = smem_u32(smem + kSmH), sW = smem_u32(smem + kSmW);
     const int64_t n_tiles = (a.rows + kTileM - 1) / kTileM;
@@ -127,7 +97,7 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
     };
     auto wait_piece = [&](int64_t s) {
         mbar_wait(&bar[s & 1], (uint32_t)((s >> 1) & 1));
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
     };
     // one layer's MMAs into TMEM column `tcol`: A = the activations from shared memory (k0 = first K step of the piece),
     // B = the piece in slot s & 1 ([rows_b x 128 K-columns] at most)
@@ -144,59 +114,18 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
     auto wait_layer = [&]() {
         mbar_wait(&bar[2], ph_m);
         ph_m ^= 1;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
     };
-    // a hidden layer's epilogue: my row, my 16-column groups (quarter, quarter + 4, ...): H = bf16(tanh(D + b))
-    auto epilogue_hidden = [&](uint32_t tcol, const float* b) {
-#pragma unroll 1
-        for (int j0 = 16 * quarter; j0 < lp; j0 += 64) {
-            uint32_t v[16];
-            tmem_ld16(lane_base + tcol + j0, v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int g = 0; g < 2; ++g) {
-                uint32_t w[4];
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const int j = j0 + 8 * g + 2 * e;
-                    w[e] = pack_bf16(tanhf(__uint_as_float(v[8 * g + 2 * e]) + b[j]), tanhf(__uint_as_float(v[8 * g + 2 * e + 1]) + b[j + 1]));
-                }
-                *reinterpret_cast<uint4*>(smem + kSmH + swz_offset(kTileM, r, j0 + 8 * g)) = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the tensor core
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-    };
-    // A: a tile's observations -> bf16, swizzled; every thread owns 4 of the tile's 2048 16-byte chunks (8 features each)
-    float af[kTileM * (kInPad / 8) / kPpoThreads][8];
-    auto load_a = [&](int64_t row0) {
-#pragma unroll
-        for (int it = 0; it < kTileM * (kInPad / 8) / kPpoThreads; ++it) {
-            const int i = tid + it * kPpoThreads, ar = i >> 4, k0 = (i & 15) * 8;
-            const int64_t row = row0 + ar;
-            const float* src = a.obs + (a.player < 0 ? row : 2 * row + a.player) * a.in_dim + k0;
-#pragma unroll
-            for (int e = 0; e < 8; ++e) af[it][e] = (row < a.rows && k0 + e < a.in_dim) ? __ldcs(src + e) : 0.f;
-        }
-    };
-    auto store_a = [&]() {
-#pragma unroll
-        for (int it = 0; it < kTileM * (kInPad / 8) / kPpoThreads; ++it) {
-            const int i = tid + it * kPpoThreads, ar = i >> 4, k0 = (i & 15) * 8;
-            *reinterpret_cast<uint4*>(smem + kSmA + swz_offset(kTileM, ar, k0)) =
-                make_uint4(pack_bf16(af[it][0], af[it][1]), pack_bf16(af[it][2], af[it][3]), pack_bf16(af[it][4], af[it][5]), pack_bf16(af[it][6], af[it][7]));
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    };
+    ObsTile<false> a_tile;  // A
 
     if (tid == 0) {
         load_piece(0);
         load_piece(1);
     }
     if (my_tiles > 0) {
-        load_a((int64_t)blockIdx.x * kTileM);
-        store_a();
+        a_tile.load(tid, a.obs, (int64_t)blockIdx.x * kTileM, a.rows, a.in_dim, a.player);
+        a_tile.store(tid, smem + kSmA);
+        fence_async_smem();
     }
     __syncthreads();
     int64_t s0 = 0;  // this tile's first weight piece
@@ -206,26 +135,26 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
         const int lk = lp / 16;  // K steps of layers 2 and 3
         // ---- layer 1
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             issue(kTmemD1, sA, s0, 0, kInPad / 16, lp, idesc_l);
             umma_commit(&bar[2]);
         }
         wait_layer();
         if (tid == 0) load_piece(s0 + 2);
-        epilogue_hidden(kTmemD1, sb);
+        epilogue_tanh_bias(smem + kSmH, lane_base + kTmemD1, sb, r, quarter, lp);
         // ---- layer 2
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             for (int c = 0; c < nk; ++c) issue(kTmemD2, sH, s0 + 1 + c, 8 * c, lk < 8 * c + 8 ? lk : 8 * c + 8, lp, idesc_l);
             umma_commit(&bar[2]);
         }
         wait_layer();
         if (tid == 0)
             for (int c = 0; c < nk; ++c) load_piece(s0 + 3 + c);
-        epilogue_hidden(kTmemD2, sb + kMaxL);
+        epilogue_tanh_bias(smem + kSmH, lane_base + kTmemD2, sb + kMaxL, r, quarter, lp);
         // ---- layer 3
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             for (int c = 0; c < nk; ++c) issue(kTmemD1, sH, s0 + 1 + nk + c, 8 * c, lk < 8 * c + 8 ? lk : 8 * c + 8, kOutPad, idesc_o);
             umma_commit(&bar[2]);
         }
@@ -233,7 +162,7 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
         if (tid == 0)
             for (int c = 0; c < nk; ++c) load_piece(s0 + 3 + nk + c);
         const bool next = tile + gridDim.x < n_tiles;
-        if (next) load_a((tile + gridDim.x) * kTileM);  // in flight under the epilogue and the sampling
+        if (next) a_tile.load(tid, a.obs, (tile + gridDim.x) * kTileM, a.rows, a.in_dim, a.player);  // in flight under the epilogue and the sampling
         // ---- e = exp(tanh(D3 + b3)) of my row, my 16-column groups, into ps[j][row] (A and H are free: layer 3 has retired)
         {
             constexpr int kG = (kOutPad / 16 + 3) / 4;
@@ -241,7 +170,7 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
 #pragma unroll
             for (int i = 0; i < kG; ++i)
                 if (quarter + 4 * i < kOutPad / 16) tmem_ld16(lane_base + kTmemD1 + 16 * (quarter + 4 * i), v[i]);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_wait_ld();
 #pragma unroll
             for (int i = 0; i < kG; ++i) {
                 if (quarter + 4 * i >= kOutPad / 16) continue;
@@ -252,18 +181,17 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
                 }
             }
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncthreads();
         // ---- softmax and the 7 draws: one thread per row
         if (tid < kTileM && tid < nrows) {
             const int64_t i = row0 + tid;
-            const int64_t env = a.player < 0 ? i >> 1 : i;
-            const int p = a.player < 0 ? (int)(i & 1) : a.player;
-            const uint32_t* rec = a.records + env * a.rec_words;
-            const uint32_t turn = rec[kRecTurn], episode = rec[kRecEpisode], g = a.env_base + (uint32_t)env;
-            uint32_t w[8];
-            philox4x32_10(g, turn, (uint32_t)p, 3u | episode << 8, a.seed_lo, a.seed_hi, w);
-            philox4x32_10(g, turn, (uint32_t)p | 1u << 8, 3u | episode << 8, a.seed_lo, a.seed_hi, w + 4);
+            const ActorRow row = actor_row(a, i);
+            const uint32_t* rec = a.records + row.env * a.rec_words;
+            const uint32_t turn = rec[kRecTurn], episode = rec[kRecEpisode];
+            uint32_t w[2][4];
+            draw_block(a, row, turn, episode, 0, w[0]);
+            draw_block(a, row, turn, episode, 1, w[1]);
             float* pr = ps + tid;
             const int out_dim = a.out_dim;
             float sum = 0.f;
@@ -278,11 +206,10 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
                 total += q;
                 if (gp) gp[j] = q;
             }
-            uint16_t* out = reinterpret_cast<uint16_t*>(a.actions + (env * 2 + p) * (EVG_MAX_ACTIONS * 2));
             int64_t* ip = a.idx ? a.idx + i * EVG_MAX_ACTIONS : nullptr;
 #pragma unroll
             for (int k = 0; k < EVG_MAX_ACTIONS; ++k) {
-                const float x = (float)(w[k] >> 8) * 0x1p-24f * total;
+                const float x = draw_uniform(w[k >> 2][k & 3]) * total;
                 float c = 0.f, t = 0.f, c_last = 0.f;
                 int sel = -1, last = -1;
 #pragma unroll 4
@@ -299,15 +226,18 @@ __global__ void __launch_bounds__(kPpoThreads, 1) evg_policy_ppo_kernel(const __
                 pr[sel * kTileM] = -0.f;
                 total = t;
                 if (ip) ip[k] = sel;
-                out[k] = (uint16_t)(((uint32_t)(sel / a.div) & 0xFFu) | ((uint32_t)(sel % a.mod) & 0xFFu) << 8);
+                store_action(a, row, k, sel);
             }
         }
         __syncthreads();  // the probabilities are read: A may be overwritten
-        if (next) store_a();
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        if (next) {
+            a_tile.store(tid, smem + kSmA);
+            fence_async_smem();
+        }
+        tc_fence_before();
         __syncthreads();
     }
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols));
+    cta_teardown(tid, tmem);
 }
 
 }  // namespace
@@ -316,39 +246,10 @@ cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const fl
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
                               int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream)
 {
-    PpoArgs a;
-    a.obs = obs;
-    a.w1 = reinterpret_cast<const unsigned char*>(w1_img);
-    a.w2 = reinterpret_cast<const unsigned char*>(w2_img);
-    a.w3 = reinterpret_cast<const unsigned char*>(w3_img);
-    a.bias = bias;
-    a.records = records;
-    a.actions = actions;
-    a.idx = idx;
-    a.probs = probs;
-    a.rows = n_envs * (player < 0 ? 2 : 1);
-    a.player = player;
-    a.in_dim = t.obs_len;
-    a.lp = (latent + 15) / 16 * 16;
-    a.nk = (a.lp + 127) / 128;
-    a.out_dim = out_dim;
-    a.div = div;
-    a.mod = mod;
-    a.rec_words = t.rec_words8 * 2;
-    a.env_base = t.env_base;
-    a.seed_lo = t.seed_lo;
-    a.seed_hi = t.seed_hi;
-    if (a.rows <= 0) return cudaSuccess;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(evg_policy_ppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
-        if (e != cudaSuccess) return e;
-        attr_set = true;
-    }
-    const int64_t tiles = (a.rows + kTileM - 1) / kTileM;
-    const unsigned grid = (unsigned)(tiles < sm_count ? tiles : sm_count);
-    evg_policy_ppo_kernel<<<grid, kPpoThreads, kSmBytes, stream>>>(a);
-    return cudaGetLastError();
+    const ActorArgs a = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
+    return launch_persistent(evg_policy_ppo_kernel, a.rows, sm_count, kSmBytes, stream, a, (a.lp + 127) / 128);
 }
+
+cudaError_t set_policy_ppo_smem() { return cudaFuncSetAttribute(evg_policy_ppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
 
 }  // namespace evg

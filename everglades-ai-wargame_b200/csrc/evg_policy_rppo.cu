@@ -39,8 +39,6 @@ namespace evg {
 
 namespace {
 
-constexpr int kRppoThreads = 512;
-constexpr int kTileM = 128;                 // observation rows per tile
 constexpr int kInPad = EVG_PPO_IN_PAD;      // input features, padded (obs_len < 128)
 constexpr int kMaxL = EVG_PPO_MAX_LATENT;   // latent width bound: 4 swizzle atoms of X / H
 constexpr int kOutPad = EVG_PPO_OUT_PAD;    // outputs, padded to a multiple of 16 (132 -> 144)
@@ -65,66 +63,28 @@ constexpr int kSmBytes = kSmBar + (2 * kSlots + 1) * 8 + 8;
 static_assert(kSmH % 1024 == 0 && kSmW % 1024 == 0 && kSlotBytes % 1024 == 0 && kSmBar % 8 == 0, "operand blocks must be 1024-byte aligned");
 static_assert(kSmBytes <= 227 * 1024, "shared memory");
 
-constexpr int kTmemCols = 512;
 constexpr int kTmemZ = 128, kTmemNi = 256, kTmemNh = 384;  // r at 0; D1 / D2 / D3 at 0, e / p at kTmemE
 constexpr int kTmemE = 256;
 
-struct RppoArgs {
-    const float* obs;
-    const unsigned char* w1;
-    const unsigned char* w2;
+struct RppoArgs : ActorArgs {
     const unsigned char* wi;
     const unsigned char* wh;
-    const unsigned char* w3;
-    const float* bias;
-    const uint32_t* records;
     float* hidden;
-    int8_t* actions;
-    int64_t* idx;
-    float* probs;
-    int64_t rows;  // n_envs * (player < 0 ? 2 : 1)
-    int player, in_dim, latent, lp, ka, nrb, out_dim, div, mod, rec_words;
-    uint32_t env_base, seed_lo, seed_hi;
+    int latent, ka, nrb;
 };
-
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&v)[4])
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr));
-}
-
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n" ::"r"(taddr),
-        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]),
-        "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-}
-
-// has phase `parity` of an mbarrier completed?  (no wait)
-__device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity)
-{
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                 : "=r"(done)
-                 : "r"(smem_u32(bar)), "r"(parity)
-                 : "memory");
-    return done != 0;
-}
 
 __device__ __forceinline__ float sigmoid(float v) { return __frcp_rn(1.f + expf(-v)); }  // = 1 / (1 + e^-v), correctly rounded
 
-__global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const __grid_constant__ RppoArgs a)
+__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const __grid_constant__ RppoArgs a)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* full = reinterpret_cast<uint64_t*>(smem + kSmBar);  // [s]: slot s landed
     uint64_t* empty = full + kSlots;                              // [s]: the MMAs reading slot s retired
     uint64_t* done = empty + kSlots;                              // a phase's MMAs retired
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(done + 1);
     float* sb = reinterpret_cast<float*>(smem + kSmBias);
     float* red = reinterpret_cast<float*>(smem + kSmRed);
-    for (int i = tid; i < kMaxL; i += kRppoThreads) {
+    for (int i = tid; i < kMaxL; i += kCtaThreads) {
         sb[kB1 + i] = a.bias[kB1 + i];
         sb[kB2 + i] = a.bias[kB2 + i];
         sb[kBr + i] = a.bias[kImgBih + i] + a.bias[kImgBhh + i];
@@ -133,18 +93,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
         sb[kBhn + i] = a.bias[kImgBhh + 2 * kMaxL + i];
         if (i < kOutPad) sb[kB3 + i] = a.bias[kB3 + i];
     }
-    if (tid == 0) {
-        for (int i = 0; i < 2 * kSlots + 1; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&full[i])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
+    const uint32_t tmem = cta_setup<2 * kSlots + 1>(tid, full, reinterpret_cast<uint32_t*>(done + 1));
     const int r = (warp & 3) * 32 + lane, quarter = warp >> 2;
     const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const int lp = a.lp, ka = a.ka, nrb = a.nrb, latent = a.latent;
@@ -158,7 +107,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
     const int total = my_tiles * per_tile;  // pieces of this CTA: < 2^31 for any batch that fits in memory
 
     // the source and size of every piece of a tile, decoded once per CTA: the producer only looks them up
-    for (int q0 = tid; q0 < per_tile; q0 += kRppoThreads) {
+    for (int q0 = tid; q0 < per_tile; q0 += kCtaThreads) {
         int q = q0, rows, rb, c;
         const unsigned char* m;
         if (q < n1) {
@@ -202,7 +151,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
             load_piece(loaded++);
         }
         mbar_wait(&full[slot], (uint32_t)((s / kSlots) & 1));
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t b_base = sW + (uint32_t)(slot * kSlotBytes), idesc = make_idesc(kTileM, nh);
         const int ks = k_cols / 16 - 4 * c < 4 ? k_cols / 16 - 4 * c : 4;
         for (int kk = 0; kk < ks; ++kk)
@@ -215,33 +164,10 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
     auto wait_done = [&]() {
         mbar_wait(done, ph);
         ph ^= 1;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (tid == 0) refill();
     };
     auto rows_of = [&](int rb) { return lp - kPieceRows * rb < kPieceRows ? lp - kPieceRows * rb : kPieceRows; };
-    // a head layer's epilogue: my row, my 16-column groups: X = bf16(tanh(D + b))
-    auto epilogue_head = [&](const float* b) {
-#pragma unroll 1
-        for (int j0 = 16 * quarter; j0 < lp; j0 += 64) {
-            uint32_t v[16];
-            tmem_ld16(lane_base + j0, v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int g = 0; g < 2; ++g) {
-                uint32_t w[4];
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const int j = j0 + 8 * g + 2 * e;
-                    w[e] = pack_bf16(tanhf(__uint_as_float(v[8 * g + 2 * e]) + b[j]), tanhf(__uint_as_float(v[8 * g + 2 * e + 1]) + b[j + 1]));
-                }
-                *reinterpret_cast<uint4*>(smem + kSmX + swz_offset(kTileM, r, j0 + 8 * g)) = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the tensor core
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-    };
-
     // the fp32 state h of my row, columns j = 16 (quarter + 4 i) + [0, 16): units below 128 (i = 0, 1) in registers for all 7
     // steps of a tile; units 128..255 (i = 2, 3, only when L > 128) in my row of d_hidden itself, which the CTA owns for the
     // whole call (64 registers of state would not fit beside the rest at 512 threads).  Padding units (L <= j < Lp) and the
@@ -282,8 +208,8 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
             h_load(i, v);
             h_to_smem(i, v);
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        fence_async_smem();
+        tc_fence_before();
         __syncthreads();
     };
 
@@ -293,26 +219,13 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
         const int nrows = a.rows - row0 < kTileM ? (int)(a.rows - row0) : kTileM;
         // ---- the observation tile -> bf16 into H; h0 of my row into registers (0 at turn 0)
         {
-            constexpr int kIt = kTileM * (kInPad / 8) / kRppoThreads;
-            float f[kIt][8];
-#pragma unroll
-            for (int it = 0; it < kIt; ++it) {
-                const int i = tid + it * kRppoThreads, ar = i >> 4, k0 = (i & 15) * 8;
-                const int64_t row = row0 + ar;
-                const float* src = a.obs + (a.player < 0 ? row : 2 * row + a.player) * a.in_dim + k0;
-#pragma unroll
-                for (int e = 0; e < 8; ++e) f[it][e] = (row < a.rows && k0 + e < a.in_dim) ? __ldcs(src + e) : 0.f;
-            }
-#pragma unroll
-            for (int it = 0; it < kIt; ++it) {
-                const int i = tid + it * kRppoThreads, ar = i >> 4, k0 = (i & 15) * 8;
-                *reinterpret_cast<uint4*>(smem + kSmH + swz_offset(kTileM, ar, k0)) =
-                    make_uint4(pack_bf16(f[it][0], f[it][1]), pack_bf16(f[it][2], f[it][3]), pack_bf16(f[it][4], f[it][5]), pack_bf16(f[it][6], f[it][7]));
-            }
+            ObsTile<false> obs_tile;
+            obs_tile.load(tid, a.obs, row0, a.rows, a.in_dim, a.player);
+            obs_tile.store(tid, smem + kSmH);
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_async_smem();
         const int64_t my_row = row0 + r;
-        const int64_t my_env = a.player < 0 ? my_row >> 1 : my_row;
+        const int64_t my_env = actor_row(a, my_row).env;
         live = r < nrows;
         hrow = a.hidden + my_row * latent;
         const bool fresh = !live || a.records[my_env * a.rec_words + kRecTurn] == 0;
@@ -324,25 +237,25 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                 if (i < 2) hs[i][e] = (!fresh && j < latent) ? hrow[j] : 0.f;
                 else if (fresh && live && j < latent) hrow[j] = 0.f;
             }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncthreads();
         // ---- the action head
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             for (int rb = 0; rb < nrb; ++rb)
                 for (int c = 0; c < 2; ++c) issue(kPieceRows * rb, sH, c, rows_of(rb), kInPad, c > 0);
             umma_commit(done);
         }
         wait_done();
-        epilogue_head(sb + kB1);
+        epilogue_tanh_bias(smem + kSmX, lane_base, sb + kB1, r, quarter, lp);
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             for (int rb = 0; rb < nrb; ++rb)
                 for (int c = 0; c < ka; ++c) issue(kPieceRows * rb, sX, c, rows_of(rb), lp, c > 0);
             umma_commit(done);
         }
         wait_done();
-        epilogue_head(sb + kB2);  // X = x for the 7 steps (layer 2 has retired)
+        epilogue_tanh_bias(smem + kSmX, lane_base, sb + kB2, r, quarter, lp);  // X = x for the 7 steps (layer 2 has retired)
         store_h(4);               // H = bf16(h0) (layer 1 has retired: the observations are read)
 #pragma unroll 1
         for (int k = 0; k < EVG_MAX_ACTIONS; ++k) {
@@ -350,7 +263,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
 #pragma unroll 1
             for (int rb = 0; rb < nrb; ++rb) {
                 if (tid == 0) {
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tc_fence_after();
                     const int nh = rows_of(rb);
                     for (int g = 0; g < 3; ++g)
                         for (int c = 0; c < ka; ++c) issue(128 * g, sX, c, nh, lp, c > 0);
@@ -373,7 +286,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                         tmem_ld4(col + kTmemZ + 4 * g, vz);
                         tmem_ld4(col + kTmemNi + 4 * g, vn);
                         tmem_ld4(col + kTmemNh + 4 * g, vh);
-                        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                        tmem_wait_ld();
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
                             const int j = j0 + 4 * g + e;
@@ -386,13 +299,13 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                     h_keep(i, hv);
                     if (rb == nrb - 1) h_to_smem(i, hv);  // every MMA reading H has retired
                 }
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+                tc_fence_before();
                 __syncthreads();  // the gates are read: the next pass may overwrite them
             }
             store_h(2 * (nrb - 1));  // the earlier pass's part of H (the last pass's epilogue wrote its own)
             // ---- D3 = H . W3^T, e = exp(tanh(D3 + b3)) back into TMEM
             if (tid == 0) {
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 for (int rb = 0; rb < 2; ++rb)
                     for (int c = 0; c < ka; ++c) issue(kPieceRows * rb, sH, c, rb ? kOutPad - kPieceRows : kPieceRows, lp, c > 0);
                 umma_commit(done);
@@ -408,7 +321,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                     if (gi >= kOutPad / 16) continue;
                     uint32_t v[16];
                     tmem_ld16(lane_base + 16 * gi, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 16; ++e) {
                         const int j = 16 * gi + e;
@@ -419,7 +332,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                     tmem_st16(lane_base + kTmemE + 16 * gi, v);
                 }
                 red[quarter * kTileM + r] = part;
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+                tmem_wait_st();
                 __syncthreads();
                 const float sum = ((red[r] + red[kTileM + r]) + red[2 * kTileM + r]) + red[3 * kTileM + r];
                 float* gp = (a.probs && live) ? a.probs + (my_row * EVG_MAX_ACTIONS + k) * a.out_dim : nullptr;
@@ -429,7 +342,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                     if (gi >= kOutPad / 16) continue;
                     uint32_t v[16];
                     tmem_ld16(lane_base + kTmemE + 16 * gi, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 16; ++e) {
                         const int j = 16 * gi + e;
@@ -440,10 +353,10 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                     tmem_st16(lane_base + kTmemE + 16 * gi, v);
                 }
             }
-            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tmem_wait_st();
+            tc_fence_before();
             __syncthreads();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc_fence_after();
             // ---- the draw: one thread per row (warps 0-3 = TMEM lanes 0-127, whole warps for tcgen05.ld): T and the
             // prefix walk are the sampler's sequential ascending sums
             if (warp < 4) {
@@ -453,24 +366,24 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                 for (int gi = 0; gi < n_groups; ++gi) {
                     uint32_t v[16];
                     tmem_ld16(lane_base + kTmemE + 16 * gi, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 16; ++e) total += __uint_as_float(v[e]);  // p = 0 past out_dim adds nothing
                 }
                 const uint32_t turn = live ? a.records[my_env * a.rec_words + kRecTurn] : 0u;
                 const uint32_t episode = live ? a.records[my_env * a.rec_words + kRecEpisode] : 0u;
-                const int p_me = a.player < 0 ? (int)(my_row & 1) : a.player;
+                const ActorRow me{my_env, actor_row(a, my_row).player};  // (my_env kept: 128 registers without spills)
                 uint32_t w[4];
-                philox4x32_10(a.env_base + (uint32_t)my_env, turn, (uint32_t)p_me | (uint32_t)(k >> 2) << 8, 3u | episode << 8, a.seed_lo, a.seed_hi, w);
+                draw_block(a, me, turn, episode, k >> 2, w);
                 const uint32_t wk = (k & 3) == 0 ? w[0] : (k & 3) == 1 ? w[1] : (k & 3) == 2 ? w[2] : w[3];
-                const float x = (float)(wk >> 8) * 0x1p-24f * total;
+                const float x = draw_uniform(wk) * total;
                 float c = 0.f;
                 int sel = -1;
 #pragma unroll 1
                 for (int gi = 0; gi < n_groups; ++gi) {
                     uint32_t v[16];
                     tmem_ld16(lane_base + kTmemE + 16 * gi, v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 16; ++e) {
                         const int j = 16 * gi + e;
@@ -484,11 +397,10 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                 if (sel < 0) sel = a.out_dim - 1;
                 if (live) {
                     if (a.idx) a.idx[my_row * EVG_MAX_ACTIONS + k] = sel;
-                    uint16_t* out = reinterpret_cast<uint16_t*>(a.actions + (my_env * 2 + p_me) * (EVG_MAX_ACTIONS * 2));
-                    out[k] = (uint16_t)(((uint32_t)(sel / a.div) & 0xFFu) | ((uint32_t)(sel % a.mod) & 0xFFu) << 8);
+                    store_action(a, me, k, sel);
                 }
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tc_fence_before();
             __syncthreads();  // D3 and p are read: the next step's gates may overwrite them
         }
         // ---- the final h of my row (units 128.. are in place already)
@@ -502,7 +414,7 @@ __global__ void __launch_bounds__(kRppoThreads, 1) evg_policy_rppo_kernel(const 
                 }
         }
     }
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols));
+    cta_teardown(tid, tmem);
 }
 
 }  // namespace
@@ -513,43 +425,16 @@ cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const f
                                cudaStream_t stream)
 {
     RppoArgs a;
-    a.obs = obs;
-    a.w1 = reinterpret_cast<const unsigned char*>(w1_img);
-    a.w2 = reinterpret_cast<const unsigned char*>(w2_img);
+    static_cast<ActorArgs&>(a) = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
     a.wi = reinterpret_cast<const unsigned char*>(wi_img);
     a.wh = reinterpret_cast<const unsigned char*>(wh_img);
-    a.w3 = reinterpret_cast<const unsigned char*>(w3_img);
-    a.bias = bias;
-    a.records = records;
     a.hidden = hidden;
-    a.actions = actions;
-    a.idx = idx;
-    a.probs = probs;
-    a.rows = n_envs * (player < 0 ? 2 : 1);
-    a.player = player;
-    a.in_dim = t.obs_len;
     a.latent = latent;
-    a.lp = (latent + 15) / 16 * 16;
     a.ka = (latent + kAtomK - 1) / kAtomK;
     a.nrb = (a.lp + kPieceRows - 1) / kPieceRows;
-    a.out_dim = out_dim;
-    a.div = div;
-    a.mod = mod;
-    a.rec_words = t.rec_words8 * 2;
-    a.env_base = t.env_base;
-    a.seed_lo = t.seed_lo;
-    a.seed_hi = t.seed_hi;
-    if (a.rows <= 0) return cudaSuccess;
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(evg_policy_rppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
-        if (e != cudaSuccess) return e;
-        attr_set = true;
-    }
-    const int64_t tiles = (a.rows + kTileM - 1) / kTileM;
-    const unsigned grid = (unsigned)(tiles < sm_count ? tiles : sm_count);
-    evg_policy_rppo_kernel<<<grid, kRppoThreads, kSmBytes, stream>>>(a);
-    return cudaGetLastError();
+    return launch_persistent(evg_policy_rppo_kernel, a.rows, sm_count, kSmBytes, stream, a);
 }
+
+cudaError_t set_policy_rppo_smem() { return cudaFuncSetAttribute(evg_policy_rppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
 
 }  // namespace evg

@@ -1,12 +1,21 @@
-// evg_tcgen05.cuh — the 5th-generation tensor-core plumbing (tcgen05 MMAs into TMEM, mbarriers, bulk copies, the
-// 128-byte-swizzled K-major operand layout) shared by the fused policy kernels evg_policy_mlp.cu and evg_policy_ppo.cu.
+// evg_tcgen05.cuh — the skeleton shared by the three fused policy kernels (evg_policy_mlp.cu, evg_policy_ppo.cu,
+// evg_policy_rppo.cu): the 5th-generation tensor-core plumbing (tcgen05 MMAs into TMEM, mbarriers, bulk copies, the
+// 128-byte-swizzled K-major operand layout), the CTA's setup and teardown, the observation-tile stager, the hidden-layer
+// epilogue of the PPO actors, their draw plumbing, and the persistent-grid launch.
 #pragma once
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include "evg_internal.h"
+
 namespace evg {
 
-constexpr int kAtomK = 64;  // bf16 elements in one 128-byte swizzle row
+constexpr int kAtomK = 64;       // bf16 elements in one 128-byte swizzle row
+constexpr int kTileM = 128;      // observation rows per tile (UMMA M = 128: TMEM lane i holds row i of the accumulators)
+constexpr int kCtaThreads = 512; // four threads per row, one per quarter of the columns
+constexpr int kObsCols = 128;    // observation columns of the A tile (EVG_MLP_IN_PAD = EVG_PPO_IN_PAD)
+constexpr int kTmemCols = 512;   // every policy kernel allocates the SM's whole tensor memory: one CTA per SM
+static_assert(EVG_MLP_IN_PAD == kObsCols && EVG_PPO_IN_PAD == kObsCols, "the observation tile is 128 columns wide");
 
 // K-major operand tile with 128-byte swizzle: element (row r, column k) of a [rows x K] bf16 matrix lives in atom k / 64
 // (a block of rows x 128 bytes), at row r, 16-byte chunk ((k % 64) / 8) ^ (r % 8)
@@ -15,8 +24,88 @@ __host__ __device__ inline int swz_offset(int rows, int r, int k)
     return (k / kAtomK) * rows * 128 + r * 128 + ((((k % kAtomK) >> 3) ^ (r & 7)) << 4) + (k & 7) * 2;
 }
 
+// the fields evg_policy_ppo_kernel and evg_policy_rppo_kernel share (filled by actor_args)
+struct ActorArgs {
+    const float* obs;
+    const unsigned char* w1;
+    const unsigned char* w2;
+    const unsigned char* w3;
+    const float* bias;
+    const uint32_t* records;
+    int8_t* actions;
+    int64_t* idx;
+    float* probs;
+    int64_t rows;  // n_envs * (player < 0 ? 2 : 1)
+    int player, in_dim, lp, out_dim, div, mod, rec_words;
+    uint32_t env_base, seed_lo, seed_hi;
+};
+
+inline ActorArgs actor_args(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+                            const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
+                            int8_t* actions, int64_t* idx, float* probs)
+{
+    ActorArgs a;
+    a.obs = obs;
+    a.w1 = reinterpret_cast<const unsigned char*>(w1_img);
+    a.w2 = reinterpret_cast<const unsigned char*>(w2_img);
+    a.w3 = reinterpret_cast<const unsigned char*>(w3_img);
+    a.bias = bias;
+    a.records = records;
+    a.actions = actions;
+    a.idx = idx;
+    a.probs = probs;
+    a.rows = n_envs * (player < 0 ? 2 : 1);
+    a.player = player;
+    a.in_dim = t.obs_len;
+    a.lp = (latent + 15) / 16 * 16;
+    a.out_dim = out_dim;
+    a.div = div;
+    a.mod = mod;
+    a.rec_words = t.rec_words8 * 2;
+    a.env_base = t.env_base;
+    a.seed_lo = t.seed_lo;
+    a.seed_hi = t.seed_hi;
+    return a;
+}
+
 #ifdef __CUDACC__
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+// ordering of tensor-core work around thread synchronisation, and of generic-proxy shared-memory writes before the
+// tensor core (async proxy) reads them
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// The CTA's start: thread 0 initialises kBars mbarriers (arrival count 1), warp 0 allocates the tensor memory into
+// *tmem_slot and gives up the allocation permit; returns the TMEM base address, visible to every thread.  This and the
+// helpers below take the kernel's own tid = threadIdx.x rather than reading it again: a second read hid tid < 512 from
+// the compiler, and the recurrent actor's whole schedule changed with it (1.6 % slower on a B200 at 1000 W).
+template <int kBars>
+__device__ __forceinline__ uint32_t cta_setup(int tid, uint64_t* bar, uint32_t* tmem_slot)
+{
+    if (tid == 0) {
+#pragma unroll
+        for (int i = 0; i < kBars; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&bar[i])));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (tid < 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    return *tmem_slot;
+}
+
+// the CTA's end: warp 0 frees the tensor memory it allocated
+__device__ __forceinline__ void cta_teardown(int tid, uint32_t tmem)
+{
+    if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols));
+}
 
 // shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start address >> 4 [0:14), leading byte offset >> 4
 // [16:30) (unused for a swizzled K-major operand), stride byte offset >> 4 [32:46) = 1024 B between 8-row groups,
@@ -62,6 +151,22 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity)
     }
 }
 
+// has phase `parity` of an mbarrier completed?  (no wait)
+__device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity)
+{
+    uint32_t done;
+    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
+                 : "=r"(done)
+                 : "r"(smem_u32(bar)), "r"(parity)
+                 : "memory");
+    return done != 0;
+}
+
+__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&v)[4])
+{
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr));
+}
+
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
 {
     asm volatile(
@@ -69,6 +174,15 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
           "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
         : "r"(taddr));
+}
+
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16])
+{
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n" ::"r"(taddr),
+        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]),
+        "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
+        : "memory");
 }
 
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
@@ -84,6 +198,97 @@ __device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t b
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
                  "r"(smem_u32(bar))
                  : "memory");
+}
+
+// A tile of 128 observation rows -> bf16, K-major, 128-byte swizzle, 128 columns.  Every thread owns 4 of the tile's
+// 2048 16-byte chunks (8 features each): load() issues all 32 loads together into registers (one DRAM round trip), so
+// that they can be in flight under other work; store() converts and writes them.  Tile row ar is batch row row0 + ar,
+// which reads observation row (player < 0 ? row : 2 row + player).  Rows past `rows` and features past in_dim are 0,
+// except feature in_dim, which is the constant 1 that carries the first layer's bias when kBiasColumn.
+template <bool kBiasColumn>
+struct ObsTile {
+    static constexpr int kIt = kTileM * (kObsCols / 8) / kCtaThreads;
+    float f[kIt][8];
+
+    __device__ __forceinline__ void load(int tid, const float* obs, int64_t row0, int64_t rows, int in_dim, int player)
+    {
+#pragma unroll
+        for (int it = 0; it < kIt; ++it) {
+            const int i = tid + it * kCtaThreads, ar = i >> 4, k0 = (i & 15) * 8;
+            const int64_t row = row0 + ar;
+            const float* src = obs + (player < 0 ? row : 2 * row + player) * in_dim + k0;
+#pragma unroll
+            for (int e = 0; e < 8; ++e) f[it][e] = (row < rows && k0 + e < in_dim) ? __ldcs(src + e) : (kBiasColumn && k0 + e == in_dim ? 1.f : 0.f);
+        }
+    }
+    __device__ __forceinline__ void store(int tid, unsigned char* dst) const
+    {
+#pragma unroll
+        for (int it = 0; it < kIt; ++it) {
+            const int i = tid + it * kCtaThreads, ar = i >> 4, k0 = (i & 15) * 8;
+            *reinterpret_cast<uint4*>(dst + swz_offset(kTileM, ar, k0)) =
+                make_uint4(pack_bf16(f[it][0], f[it][1]), pack_bf16(f[it][2], f[it][3]), pack_bf16(f[it][4], f[it][5]), pack_bf16(f[it][6], f[it][7]));
+        }
+    }
+};
+
+// a PPO actor's hidden-layer epilogue: row r, the 16-column groups 16 quarter, + 64, ... below lp of the accumulators at
+// TMEM address `taddr` (the thread's lane base + the layer's column): dst = bf16(tanh(D + b)), swizzled; then dst is made
+// visible to the tensor core and the CTA synchronises
+__device__ __forceinline__ void epilogue_tanh_bias(unsigned char* dst, uint32_t taddr, const float* b, int r, int quarter, int lp)
+{
+#pragma unroll 1
+    for (int j0 = 16 * quarter; j0 < lp; j0 += 64) {
+        uint32_t v[16];
+        tmem_ld16(taddr + j0, v);
+        tmem_wait_ld();
+#pragma unroll
+        for (int g = 0; g < 2; ++g) {
+            uint32_t w[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const int j = j0 + 8 * g + 2 * e;
+                w[e] = pack_bf16(tanhf(__uint_as_float(v[8 * g + 2 * e]) + b[j]), tanhf(__uint_as_float(v[8 * g + 2 * e + 1]) + b[j + 1]));
+            }
+            *reinterpret_cast<uint4*>(dst + swz_offset(kTileM, r, j0 + 8 * g)) = make_uint4(w[0], w[1], w[2], w[3]);
+        }
+    }
+    fence_async_smem();
+    tc_fence_before();
+    __syncthreads();
+}
+
+// row i of an actor's batch: (match, player) = (i / 2, i % 2) when both players are played, else (i, player)
+struct ActorRow {
+    int64_t env;
+    int player;
+};
+__device__ __forceinline__ ActorRow actor_row(const ActorArgs& a, int64_t i) { return {a.player < 0 ? i >> 1 : i, a.player < 0 ? (int)(i & 1) : a.player}; }
+
+// the draws of a row (match env, player p) at the turn and episode of the match's record, on the tape's domain 3
+// (DESIGN.md §2): the uniform of draw k comes from word k % 4 of Philox block k / 4
+__device__ __forceinline__ void draw_block(const ActorArgs& a, ActorRow row, uint32_t turn, uint32_t episode, int block, uint32_t (&w)[4])
+{
+    philox4x32_10(a.env_base + (uint32_t)row.env, turn, (uint32_t)row.player | (uint32_t)block << 8, 3u | episode << 8, a.seed_lo, a.seed_hi, w);
+}
+__device__ __forceinline__ float draw_uniform(uint32_t word) { return (float)(word >> 8) * 0x1p-24f; }
+
+// action row k of (match env, player p) for flat index sel: (sel / div, sel % mod)
+__device__ __forceinline__ void store_action(const ActorArgs& a, ActorRow row, int k, int sel)
+{
+    uint16_t* out = reinterpret_cast<uint16_t*>(a.actions + (row.env * 2 + row.player) * (EVG_MAX_ACTIONS * 2));
+    out[k] = (uint16_t)(((uint32_t)(sel / a.div) & 0xFFu) | ((uint32_t)(sel % a.mod) & 0xFFu) << 8);
+}
+
+// the fused policy kernels are persistent over 128-row tiles: at most one CTA per SM (each takes all of its tensor
+// memory), never more CTAs than tiles
+template <typename... Params, typename... Args>
+cudaError_t launch_persistent(void (*kernel)(Params...), int64_t rows, int sm_count, int smem, cudaStream_t stream, Args... args)
+{
+    if (rows <= 0) return cudaSuccess;
+    const int64_t tiles = (rows + kTileM - 1) / kTileM;
+    kernel<<<(unsigned)(tiles < sm_count ? tiles : sm_count), kCtaThreads, smem, stream>>>(args...);
+    return cudaGetLastError();
 }
 #endif
 

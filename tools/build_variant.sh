@@ -1,12 +1,11 @@
 #!/bin/bash
 # Build the library under another name with extra -D flags: kernel A/B runs without touching the in-tree libevgsim.so.
 #   tools/build_variant.sh NAME [-DEVG_TPM_STAGE=32 -DEVG_TPM_MIN_CTAS=3 ...]   ->  build/libevgsim_NAME.so
-# Select it with EVGSIM_LIB=build/libevgsim_NAME.so (see tools/ab_variants.sh).
+# Select it with EVGSIM_LIB=build/libevgsim_NAME.so (see tools/ab_variants.sh).  The sources and nvcc flags are those of
+# __graft_entry__.build().
 set -e
 cd "$(dirname "$0")/.."
 name=$1; shift
 mkdir -p build
-C=everglades-ai-wargame_b200/csrc
-/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -shared "$@" \
-    -o build/libevgsim_$name.so $C/evg_kernels.cu $C/evg_step_tpm.cu $C/evg_policy_mlp.cu $C/evg_capi.cu
+python3 -c 'import sys, __graft_entry__ as g; g.compile_library(sys.argv[1], sys.argv[2:], force=True)' "build/libevgsim_$name.so" "$@"
 echo built build/libevgsim_$name.so
