@@ -559,11 +559,10 @@ int evg_reset_fmt(EvgSim* sim, int32_t format, const uint8_t* d_mask, void* d_ro
 
 int evg_reset(EvgSim* sim, const uint8_t* d_mask, float* d_obs, void* stream) { return evg_reset_fmt(sim, EVG_OBS_F32, d_mask, d_obs, nullptr, stream); }
 
-// first/count: the whole batch (0, n_envs), or a 128-aligned sub-range for the thread-per-match kernel (evg_step_host's
-// chunks; all the per-match arrays are offset here, the kernel adds `first` to the global match ids)
-static int step_impl(EvgSim* sim, int agent0, int agent1, const int8_t* d_actions, int8_t* d_actions_out, void* d_obs,
-                     float* d_reward, uint8_t* d_done, uint8_t* d_status, int32_t* d_scores, void* stream, int64_t first = 0,
-                     int64_t count = -1, int obs_fmt = EVG_OBS_F32, int sched_slot = 0, int n_turns = 1)
+// the step kernels' arguments for the whole batch
+static evg::StepArgs step_args(EvgSim* sim, int agent0, int agent1, const int8_t* d_actions, int8_t* d_actions_out, void* d_obs,
+                               float* d_reward, uint8_t* d_done, uint8_t* d_status, int32_t* d_scores, int obs_fmt, int sched_slot,
+                               int n_turns)
 {
     evg::StepArgs a;
     a.n_turns = n_turns;
@@ -586,6 +585,17 @@ static int step_impl(EvgSim* sim, int agent0, int agent1, const int8_t* d_action
     a.tables_dev = sim->tables_dev;
     a.oconst_dev = sim->oconst_dev;
     a.env_first = 0;
+    return a;
+}
+
+// first/count: the whole batch (0, n_envs), or a 128-aligned sub-range for the thread-per-match kernel (evg_step_host's
+// chunks; all the per-match arrays are offset here, the kernel adds `first` to the global match ids)
+static int step_impl(EvgSim* sim, int agent0, int agent1, const int8_t* d_actions, int8_t* d_actions_out, void* d_obs,
+                     float* d_reward, uint8_t* d_done, uint8_t* d_status, int32_t* d_scores, void* stream, int64_t first = 0,
+                     int64_t count = -1, int obs_fmt = EVG_OBS_F32, int sched_slot = 0, int n_turns = 1)
+{
+    evg::StepArgs a = step_args(sim, agent0, agent1, d_actions, d_actions_out, d_obs, d_reward, d_done, d_status, d_scores, obs_fmt,
+                                sched_slot, n_turns);
     if (count >= 0) {
         const evg::Tables& t = sim->tables;
         a.records += first * t.rec_words8 * 2;
@@ -663,25 +673,7 @@ int evg_rollout(EvgSim* sim, int32_t agent_p0, int32_t agent_p1, int32_t n_turns
     }
     if (sim->use_tpm)  // one launch: a CTA keeps each of its batches in shared memory for all n_turns
         return step_impl(sim, agent_p0, agent_p1, d_actions, d_actions, d_obs, d_reward, d_done, d_status, d_scores, stream, 0, -1, EVG_OBS_F32, 0, n_turns);
-    evg::StepArgs a;
-    memset(&a, 0, sizeof(a));
-    a.agent[0] = agent_p0;
-    a.agent[1] = agent_p1;
-    a.actions = d_actions;
-    a.actions_out = d_actions;
-    a.records = (uint32_t*)sim->bound[EVG_BIND_RECORDS];
-    a.health = (double*)sim->bound[EVG_BIND_HEALTH];
-    a.stats = (unsigned long long*)sim->bound[EVG_BIND_STATS];
-    a.agent_state = (uint2*)sim->bound[EVG_BIND_AGENTS];
-    a.obs = d_obs;
-    a.obs_fmt = EVG_OBS_F32;
-    a.reward = d_reward;
-    a.done = d_done;
-    a.status = d_status;
-    a.scores = d_scores;
-    a.n_envs = sim->n_envs;
-    a.tables_dev = sim->tables_dev;
-    a.oconst_dev = sim->oconst_dev;
+    const evg::StepArgs a = step_args(sim, agent_p0, agent_p1, d_actions, d_actions, d_obs, d_reward, d_done, d_status, d_scores, EVG_OBS_F32, 0, n_turns);
     cudaError_t e = evg::launch_rollout(sim->tables, a, n_turns, sim->grid, sim->smem, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_rollout_kernel launch");
     sim->launches += 1;

@@ -86,27 +86,11 @@ struct alignas(16) Tables {
 
 constexpr int kLossD = 32;
 constexpr int kAgentMaxNodes = 15;  // nibble-packed node permutation of the on-device random agent
-#ifndef EVG_TPM_THREADS
-#define EVG_TPM_THREADS 128
-#endif
-constexpr int kTpmThreads = EVG_TPM_THREADS;
+constexpr int kTpmThreads = 128;
 constexpr int kTpmSmallThreads = 32;  // the one-warp-per-CTA instantiation for small batches (compile-time map only)
-#ifndef EVG_TPM_STAGE
-#define EVG_TPM_STAGE 32
-#endif
-#ifndef EVG_TPM_MIN_CTAS
-#define EVG_TPM_MIN_CTAS 3
-#endif
-#ifndef EVG_TPM_LITE_MIN_CTAS
-#define EVG_TPM_LITE_MIN_CTAS 14  // resident one-warp CTAs per SM the LITE instantiation is compiled for (register cap 144)
-#endif
-#ifndef EVG_TPM_SYNC
-#define EVG_TPM_SYNC 1  // CTA barriers at the phase boundaries named by EVG_TPM_SYNC_MASK (0: free-running warps)
-#endif
-#ifndef EVG_TPM_PIPE
-#define EVG_TPM_PIPE 1
-#endif
-constexpr int kTpmStage = EVG_TPM_STAGE;  // observation staging window per match, 32-bit words (16 or 32)
+constexpr int kTpmMinCtas = 3;        // resident 128-thread CTAs per SM the thread-per-match kernel is compiled for
+constexpr int kTpmLiteMinCtas = 14;   // resident one-warp CTAs per SM the LITE instantiation is compiled for (register cap 144)
+constexpr int kTpmStage = 32;         // observation staging window per match, 32-bit words
 
 // device statistics accumulators (uint64 each); matches EvgEpisodeStats minus env_turns
 // ST_FOUGHT: unit slots of the groups that took part in combat (every match-turn, finished or not): the health term of
@@ -217,6 +201,18 @@ cudaError_t launch_step_tpm(const Tables& t, const StepArgs& a, int threads, siz
 #else
 #define EVG_CHECK(cond) ((void)0)
 #endif
+
+// Map size of a step kernel: compile-time (NODES > 0, DemoMap's 11 for the instantiated fast paths) or read from the
+// tables (0).  The record size is in 8-byte units, as in Tables::rec_words8.
+template <int NODES>
+struct Geo {
+    const Tables& S;
+    __device__ __forceinline__ explicit Geo(const Tables& s) : S(s) {}
+    __device__ __forceinline__ int n_nodes() const { return NODES ? NODES : S.n_nodes; }
+    __device__ __forceinline__ int nn() const { return n_nodes() + 1; }
+    __device__ __forceinline__ int obs_len() const { return 1 + 4 * n_nodes() + 5 * EVG_NUM_GROUPS; }
+    __device__ __forceinline__ int rec_words8() const { return NODES ? ((kRecNode0 + NODES) * 4 + 31) / 32 * 4 : S.rec_words8; }
+};
 
 // Philox4x32-10 (Salmon et al., SC'11); same function as oracle/tape.py, oracle/evg_oracle.c.
 __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,

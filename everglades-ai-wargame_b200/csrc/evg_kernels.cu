@@ -51,17 +51,6 @@ __device__ __forceinline__ WarpSmem carve(unsigned char* base, const Tables& S)
     return W;
 }
 
-// Compile-time map size (NODES > 0: DemoMap's 11 is the instantiated fast path) or run-time (0).
-template <int NODES>
-struct Dim {
-    const Tables& S;
-    __device__ __forceinline__ explicit Dim(const Tables& s) : S(s) {}
-    __device__ __forceinline__ int n_nodes() const { return NODES ? NODES : S.n_nodes; }
-    __device__ __forceinline__ int nn() const { return n_nodes() + 1; }
-    __device__ __forceinline__ int obs_len() const { return 1 + 4 * n_nodes() + 5 * EVG_NUM_GROUPS; }
-    __device__ __forceinline__ int rec_words8() const { return NODES ? ((kRecNode0 + NODES) * 4 + 31) / 32 * 4 : S.rec_words8; }
-};
-
 // Per-(side,node) sums over the groups LISTED at the node (node.groups[pid]: location == node and
 // not destroyed).  One shared-memory atomic per group packs three reductions:
 //   [0:10)  units of all listed groups, moving or not   (board_state opponent count, server.py:446-449)
@@ -71,7 +60,7 @@ template <int NODES>
 __device__ __forceinline__ void node_accumulate(const Tables& S, const WarpSmem& W, int lane, bool is_grp, int side,
                                                 uint32_t w0, uint32_t w1)
 {
-    const Dim<NODES> D(S);
+    const Geo<NODES> D(S);
     const int nn = D.nn();
     for (int i = lane; i < 2 * nn; i += 32) W.acc[i] = 0;
     __syncwarp();
@@ -93,7 +82,7 @@ __device__ __forceinline__ void pack_obs(const Tables& S, const WarpSmem& W, int
                                          uint32_t w0, uint32_t w1, uint32_t nw, uint32_t turn, float* out, int fmt = EVG_OBS_F32,
                                          bool done = false, int status = 0, float r0 = 0.f, float r1 = 0.f)
 {
-    const Dim<NODES> D(S);
+    const Geo<NODES> D(S);
     const int L = D.obs_len(), nn = D.nn();
     if (fmt == EVG_OBS_WIRE) {
         uint32_t* sw = reinterpret_cast<uint32_t*>(W.obs);
@@ -157,7 +146,7 @@ template <int NODES>
 __device__ __forceinline__ void step_match(const Tables& S, const WarpSmem& W, const StepArgs& A, int64_t env, int lane,
                                            unsigned long long* cta_stats)
 {
-    const Dim<NODES> D(S);
+    const Geo<NODES> D(S);
     const int n_nodes = D.n_nodes(), nn = D.nn(), rec_words8 = D.rec_words8();
     const bool is_grp = lane < kGroupLanes;
     const int side = lane >= EVG_NUM_GROUPS ? 1 : 0;

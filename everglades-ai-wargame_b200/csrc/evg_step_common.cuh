@@ -4,16 +4,6 @@
 
 namespace evg {
 
-template <int NODES>
-struct Geo {
-    const Tables& S;
-    __device__ __forceinline__ explicit Geo(const Tables& s) : S(s) {}
-    __device__ __forceinline__ int n_nodes() const { return NODES ? NODES : S.n_nodes; }
-    __device__ __forceinline__ int nn() const { return n_nodes() + 1; }
-    __device__ __forceinline__ int obs_len() const { return 1 + 4 * n_nodes() + 5 * EVG_NUM_GROUPS; }
-    __device__ __forceinline__ int rw() const { return NODES ? ((kRecNode0 + NODES) * 4 + 31) / 32 * 8 : S.rec_words8 * 2; }
-};
-
 // numpy's pairwise float64 sum (np.sum at server.py:481) over hv[0..size), size <= MAXSZ <= 16.
 template <int MAXSZ>
 __device__ __forceinline__ double np_sum_regs(const double (&hv)[MAXSZ], int size)

@@ -30,52 +30,17 @@
 // independently, so (1) ONE CTA barrier per batch, before the observation phase, keeps a CTA's four warps on the
 // same instructions through the longest straight-line code, (2) code that a launch never executes lives in
 // another instantiation (AGENTS) or out of line (statistics, partial warps, resets), (3) loops stay rolled where
-// unrolling buys little.  The knobs below exist for A/B builds (tools/build_variant.sh); defaults are the
-// measured best.
+// unrolling buys little.  The unroll factors, the barrier site, the request point of the record pipeline and the
+// occupancy targets were each chosen by measurement (DESIGN.md section 4.1, profiles/README.md); the unroll factors
+// and the observation split quote their timings where they are set.
 //
 // Reference semantics are cited per phase (server.py / env.py as in evg_kernels.cu); the checker is
 // oracle/evg_oracle.c.
-#include <cstdlib>
-
 #include "evg_step_common.cuh"
 
-#ifndef EVG_TPM_MOVE_UNROLL
-#define EVG_TPM_MOVE_UNROLL 1  // (1: 0.4965 ms, 2: 0.4983, 3: 0.5016, 4: 0.5078 per 1 Mi match-turns; footprint beats overlap)
-#endif
-#ifndef EVG_TPM_STORE_UNROLL
-#define EVG_TPM_STORE_UNROLL 8  // record store, 16 chunks per lane (8: 0.4882 ms, 4: 0.4904, 2: 0.4922, 16: 0.4924)
-#endif
-#ifndef EVG_TPM_STREAM_UNROLL
-#define EVG_TPM_STREAM_UNROLL 4  // streaming loop of an observation window, 16 iterations (4: 0.4924 ms, 8: 0.4942, 16: 0.4965, 2: 0.4971)
-#endif
-#ifndef EVG_TPM_CAPTURE_UNROLL
-#define EVG_TPM_CAPTURE_UNROLL 1
-#endif
-#ifndef EVG_TPM_SYNC_MASK
-#define EVG_TPM_SYNC_MASK 8  // which of the phase boundaries carry a CTA barrier: bit 3 = before the observation phase (measured best, profiles/README.md)
-#endif
-#if EVG_TPM_SYNC
-#define EVG_PHASE_SYNC(i) do { if ((EVG_TPM_SYNC_MASK >> (i)) & 1) __syncthreads(); } while (0)
-#else
-#define EVG_PHASE_SYNC(i) ((void)0)
-#endif
-
-#ifndef EVG_TPM_OBS_SPLIT
-#define EVG_TPM_OBS_SPLIT 2  // groups a 32-word observation window is packed in (1, 2 or 4; 2 measured best: 0.5004 vs 0.5024 / 0.5044 ms)
-#endif
-
-#ifndef EVG_TPM_REQUEST_AT
-#define EVG_TPM_REQUEST_AT 1  // where the next batch's records are requested: 0 before the observation phase, 1 before movement
-#endif
-
-#ifndef EVG_TPM_SEG
-#define EVG_TPM_SEG 1
-#endif
 namespace evg {
 
 namespace {
-
-constexpr int kMoveUnroll = EVG_TPM_MOVE_UNROLL, kCaptureUnroll = EVG_TPM_CAPTURE_UNROLL, kStreamUnroll = EVG_TPM_STREAM_UNROLL, kStoreUnroll = EVG_TPM_STORE_UNROLL;
 
 // game_init state (server.py:133-209) for one match: its record row in shared memory (the health refill is the warp's
 // job: refill_health below)
@@ -167,7 +132,7 @@ __device__ __noinline__ void load_rows_direct(const StepArgs& A, uint32_t* wrow,
 // WIRE: the observation output is the packed wire row of include/evgsim.h (EVG_OBS_WIRE: 128 bytes per match on DemoMap,
 // both players' observations + rewards + done in one cache line) instead of float32[2][obs_len] (840 bytes)
 template <int NODES, int MAXSZ, typename HistT, int PITCH, bool AGENTS, int THREADS, bool WIRE = false, bool ROLL = false>
-__global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_CTAS : EVG_TPM_LITE_MIN_CTAS) evg_step_tpm_kernel(const __grid_constant__ Tables T, const __grid_constant__ StepArgs A)
+__global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? kTpmMinCtas : kTpmLiteMinCtas) evg_step_tpm_kernel(const __grid_constant__ Tables T, const __grid_constant__ StepArgs A)
 {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -186,9 +151,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
     // CTA that runs one or two batches has no use for, gives its 71 registers back.
     constexpr bool LITE = THREADS == kTpmSmallThreads;
     // SEG (compile-time map): combat applies damage in segments of 8 unit slots, a group of 9..MAXSZ slots on two lanes
-    constexpr bool SEG = NODES != 0 && EVG_TPM_SEG != 0 && MAXSZ > 8;
+    constexpr bool SEG = NODES != 0 && MAXSZ > 8;
     constexpr int HVN = SEG ? 8 : MAXSZ;
-    constexpr bool PIPE = NODES != 0 && EVG_TPM_PIPE != 0 && !LITE && !ROLL;  // (a rollout loads records once per K turns: the pipeline's 71 registers are worth more to its turns)
+    constexpr bool PIPE = NODES != 0 && !LITE && !ROLL;  // (a rollout loads records once per K turns: the pipeline's 71 registers are worth more to its turns)
     uint4 nxt[16];
     uint32_t nxa[7];
     bool have = false;
@@ -208,7 +173,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
     // leaves the SMs with the cheap batches idle at the end.  Thread 0 draws the batch after next from a global counter
     // ahead of the one CTA barrier of a batch and publishes it in shared memory; the counter pair (handed out, CTAs
     // finished) resets itself when the last CTA leaves.
-    static_assert(EVG_TPM_SYNC && ((EVG_TPM_SYNC_MASK >> 3) & 1), "the batch hand-over uses the barrier before the observation phase");
     // (the two hand-over slots live in the CTA's copy of the tables: static shared memory would come off the opt-in limit)
     uint32_t first_draw = 0;
     if (!LITE && threadIdx.x == 0) first_draw = gridDim.x + atomicAdd(&A.sched[0], 1u);
@@ -224,7 +188,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
     const Tables& S = *tables_ptr;
     if (!LITE) __syncthreads();  // the run-time-sized instantiations read their sizes from the staged tables
     const Geo<NODES> G(S);
-    const int n_nodes = G.n_nodes(), nn = G.nn(), RW = G.rw(), OL = G.obs_len();
+    const int n_nodes = G.n_nodes(), nn = G.nn(), RW = G.rec_words8() * 2, OL = G.obs_len();
     // the observation entries that never change (a third of them: the nodes' DEFENSE/OBSERVE flags in each viewer's
     // numbering and the groups' unit types) were converted to float once, by evg_bind (A.oconst_dev: 2*OL floats, then per
     // [player][viewer slot] the node's two flags); a CTA keeps a copy in shared memory, LITE reads them in place
@@ -290,7 +254,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
         load_rows_direct<NODES>(A, wrow, P, RW, RWU, warp_env0, nvalid, lane, !PIPE, next_batch * THREADS + warp * 32);
     }
     __syncwarp();
-    EVG_PHASE_SYNC(0);
 
     uint32_t turn = 0, episode = 0;
     int s0 = 0, s1 = 0, status = 0;
@@ -443,7 +406,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
             const uint32_t tot = __reduce_add_sync(0xFFFFFFFFu, my_slots);
             if (lane == 0 && tot) atomicAdd(&A.stats[ST_FOUGHT], (unsigned long long)tot);
         }
-        EVG_PHASE_SYNC(1);
         // the warp's work list = concatenation of the matches' fighting groups (then their second draw blocks); a
         // round takes whole matches (a match has <= 32 items), so draws and apply of one match stay in one round and the
         // round's histograms fit the warp's pool: match m owns entries [upre[m] - upre[m_begin], +b0+b1)
@@ -618,10 +580,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
         }
     }
 
-    EVG_PHASE_SYNC(2);
-#if EVG_TPM_REQUEST_AT == 1
-    if (PIPE && last) have = request(next_batch);
-#endif
+    if (PIPE && last) have = request(next_batch);  // in flight through movement, capture and the observations
     if (valid) {
         // ---- movement (server.py:656-706) fused with the per-(side,node) sums capture and observations need:
         //   [0:10) units of all listed groups (:446-449), [10:24) count*control of non-moving groups (:718-724),
@@ -654,7 +613,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
                 pts = (int)(cnt * (gm >> 16));
                 any_alive |= live;
             };
-#pragma unroll kMoveUnroll
+            // rolled: the footprint costs more than the overlap buys (unrolled 1: 0.4965 ms, 2: 0.4983, 3: 0.5016,
+            // 4: 0.5078 per 1 Mi match-turns)
+#pragma unroll 1
             for (int g = 0; g < EVG_NUM_GROUPS; ++g) {
                 uint32_t va, la, vb, lb;
                 int pa, pb;
@@ -672,7 +633,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
         // ---- capture (server.py:708-767; current_turn > 0 here) and node scoring (server.py:298-310)
         bool basecap = false;
         const int capture_bonus = S.capture_bonus;
-#pragma unroll kCaptureUnroll
+#pragma unroll 1
         for (int n = 1; n <= n_nodes; ++n) {
             const uint32_t nw = R[kRecNode0 + n - 1];
             int cs = (int)(int16_t)(nw & 0xFFFFu), cb = (int)(int8_t)((nw >> 16) & 0xFFu);
@@ -747,11 +708,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
     }
     }  // turns of a rollout
 
-#if EVG_TPM_REQUEST_AT == 0
-    if (PIPE) have = request(next_batch);  // in flight across the barrier
-#endif
     if (!LITE && threadIdx.x == 0) sched[par] = gridDim.x + atomicAdd(&A.sched[0], 1u);  // the batch after next
-    EVG_PHASE_SYNC(3);
+    // the CTA's one barrier of a batch: it keeps the four warps on the same instructions through the observation code,
+    // and the batch hand-over relies on it (sched[par], written above, is read below by every thread)
+    __syncthreads();
     const int64_t after_next = LITE ? next_batch + gridDim.x : (int64_t)sched[par];
     par ^= 1;
 
@@ -817,11 +777,13 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
 #pragma unroll
         for (int c = 0; c < (NODES ? kFastChunks : nchunks); ++c) {
             if (valid) {
-                // reads first (they can be merged and overlapped), then the staging stores — in EVG_TPM_OBS_SPLIT groups per
-                // window: fewer values alive at once next to the 71 registers of the record pipeline
-                constexpr int GP = SP / EVG_TPM_OBS_SPLIT;  // pairs per group
+                // reads first (they can be merged and overlapped), then the staging stores — in kSplit groups per window:
+                // fewer values alive at once next to the 71 registers of the record pipeline (2 groups: 0.5004 ms, 1: 0.5024,
+                // 4: 0.5044)
+                constexpr int kSplit = 2;
+                constexpr int GP = SP / kSplit;  // pairs per group
 #pragma unroll
-                for (int h = 0; h < EVG_TPM_OBS_SPLIT; ++h) {
+                for (int h = 0; h < kSplit; ++h) {
                     uint32_t vals[2 * GP];
 #pragma unroll
                     for (int k = 0; k < 2 * GP; ++k) {
@@ -839,7 +801,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
                 const uint32_t* srow = wrow + stage_off + 2 * cp;
                 uint32_t* orow = obs_base + 2 * pr;
                 if (nvalid == 32) {  // whole warp: no per-match predicates
-#pragma unroll kStreamUnroll
+                    // 16 iterations, unrolled by 4: 0.4924 ms (8: 0.4942, 16: 0.4965, 2: 0.4971)
+#pragma unroll 4
                     for (int it = 0; it < 32 / MPI; ++it) {
                         const int m = MPI * it + sub;
                         const uint2 v = *reinterpret_cast<const uint2*>(srow + (size_t)m * P);
@@ -867,7 +830,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
     }
     __syncwarp();
 
-    EVG_PHASE_SYNC(4);
     // ---- cooperative, coalesced store of the records (the padding words are written as zeros)
     {
         const int q4 = RW / 4;
@@ -886,7 +848,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
             g4[f] = make_uint4(a.x, a.y, b.x, b.y);
         };
         if (NODES && nvalid == 32) {
-#pragma unroll kStoreUnroll
+            // 16 chunks per lane, unrolled by 8: 0.4882 ms (4: 0.4904, 2: 0.4922, 16: 0.4924)
+#pragma unroll 8
             for (int i = 0; i < (NODES ? 16 : 1); ++i) put(pl + 32 * i);
         } else {
 #pragma unroll 1
@@ -912,8 +875,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == kTpmThreads ? EVG_TPM_MIN_
 // DemoMap row: 62 record words + the staging window, pitch / 2 odd
 constexpr int kFastPitch = (((62 + kTpmStage) / 2) & 1) ? 62 + kTpmStage : 62 + kTpmStage + 2;
 
-// which instantiation serves this config
+// which family of instantiations serves this config
 enum Variant { V_FAST = 0, V_GENERIC8, V_GENERIC16 };
+using TpmKernel = void (*)(Tables, StepArgs);
 
 Variant pick(const Tables& t)
 {
@@ -922,97 +886,67 @@ Variant pick(const Tables& t)
     return t.tpm_hist16 ? V_GENERIC16 : V_GENERIC8;
 }
 
+// The kernel that serves a launch of one variant's kernel family, nullptr for a combination that is not instantiated.
+// The compile-time map leaves the agents' code out of a plain step (AGENTS = false) and has no wire-row instantiation
+// with scripted agents: no C ABI entry point fuses the agents into a step that writes wire rows (evg_step_agents and
+// evg_rollout write float32).  The run-time-sized kernels carry the agents' code in every instantiation.
+template <int NODES, int MAXSZ, typename HistT, int PITCH, int THREADS>
+TpmKernel family_kernel(bool agents, bool wire, bool roll)
+{
+    constexpr bool PLAIN_AGENTS = NODES == 0;
+    if (wire) return roll || (agents && !PLAIN_AGENTS) ? nullptr : evg_step_tpm_kernel<NODES, MAXSZ, HistT, PITCH, PLAIN_AGENTS, THREADS, true>;
+    if (roll) return evg_step_tpm_kernel<NODES, MAXSZ, HistT, PITCH, true, THREADS, false, true>;
+    if (agents) return evg_step_tpm_kernel<NODES, MAXSZ, HistT, PITCH, true, THREADS>;
+    return evg_step_tpm_kernel<NODES, MAXSZ, HistT, PITCH, PLAIN_AGENTS, THREADS>;
+}
+
+// The one table of thread-per-match instantiations: one-warp CTAs exist for the compile-time map only
+TpmKernel tpm_kernel(Variant v, int threads, bool agents, bool wire, bool roll)
+{
+    if (threads == kTpmSmallThreads) return v == V_FAST ? family_kernel<11, 12, uint8_t, kFastPitch, kTpmSmallThreads>(agents, wire, roll) : nullptr;
+    switch (v) {
+        case V_FAST: return family_kernel<11, 12, uint8_t, kFastPitch, kTpmThreads>(agents, wire, roll);
+        case V_GENERIC8: return family_kernel<0, 16, uint8_t, 0, kTpmThreads>(agents, wire, roll);
+        default: return family_kernel<0, 16, uint16_t, 0, kTpmThreads>(agents, wire, roll);
+    }
+}
+
 }  // namespace
 
 bool tpm_has_small(const Tables& t) { return pick(t) == V_FAST; }
 
-static size_t tpm_smem_bytes(const Tables& t, int threads)
+cudaError_t tpm_prepare(const Tables& t, int threads, size_t* smem_out, int* blocks_per_sm)
 {
     // the one-warp CTAs keep neither the tables nor the constant observation entries in shared memory (LITE).
     // DemoMap, 128-thread CTAs: 65,696 B; three CTAs + the driver's 1 KiB each = 195.5 KiB, inside the SM's 196 KiB
     // shared-memory configuration.  One more KB per CTA selects the 228 KiB configuration, L1 drops from 60 to 28 KiB
     // and the step kernel loses 15 % (DESIGN.md section 4.4): do not grow this.
-    size_t smem = (threads == kTpmSmallThreads ? 0 : (size_t)t.sm_tables_bytes + (size_t)oconst_bytes(t.n_nodes)) +
-                  (size_t)(threads / 32) * (32 * t.tpm_pitch + 64 * (t.n_nodes + 1) + t.tpm_pool_words) * 4;
-    if (const char* pad = getenv("EVG_TPM_SMEM_PAD")) smem += (size_t)atoi(pad);  // occupancy experiments (profiles/README.md)
-    return smem;
-}
-
-cudaError_t tpm_prepare(const Tables& t, int threads, size_t* smem_out, int* blocks_per_sm)
-{
-    const size_t smem = tpm_smem_bytes(t, threads);
+    const size_t smem = (threads == kTpmSmallThreads ? 0 : (size_t)t.sm_tables_bytes + (size_t)oconst_bytes(t.n_nodes)) +
+                        (size_t)(threads / 32) * (32 * t.tpm_pitch + 64 * (t.n_nodes + 1) + t.tpm_pool_words) * 4;
     *smem_out = smem;
+    const Variant v = pick(t);
+    const TpmKernel plain = tpm_kernel(v, threads, false, false, false);
+    if (!plain) return cudaErrorInvalidValue;
     cudaError_t e;
     int limit = 0;
     if ((e = optin_smem_limit(smem, &limit)) != cudaSuccess) return e;
-#define EVG_TPM_ATTR(...) \
-    if ((e = cudaFuncSetAttribute(evg_step_tpm_kernel<__VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize, limit)) != cudaSuccess) return e;
-    if (threads == kTpmSmallThreads) {
-        if (pick(t) != V_FAST) return cudaErrorInvalidValue;
-        EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, false, kTpmSmallThreads)
-        EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, true, kTpmSmallThreads)
-        EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, true, kTpmSmallThreads, false, true)
-        EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, false, kTpmSmallThreads, true)
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, evg_step_tpm_kernel<11, 12, uint8_t, kFastPitch, false, kTpmSmallThreads>,
-                                                             threads, smem);
-    }
-    EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, false, kTpmThreads)
-    EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, true, kTpmThreads)
-    EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, true, kTpmThreads, false, true)
-    EVG_TPM_ATTR(0, 16, uint8_t, 0, true, kTpmThreads, false, true)
-    EVG_TPM_ATTR(0, 16, uint16_t, 0, true, kTpmThreads, false, true)
-    EVG_TPM_ATTR(11, 12, uint8_t, kFastPitch, false, kTpmThreads, true)
-    EVG_TPM_ATTR(0, 16, uint8_t, 0, true, kTpmThreads)
-    EVG_TPM_ATTR(0, 16, uint16_t, 0, true, kTpmThreads)
-    EVG_TPM_ATTR(0, 16, uint8_t, 0, true, kTpmThreads, true)
-    EVG_TPM_ATTR(0, 16, uint16_t, 0, true, kTpmThreads, true)
-#undef EVG_TPM_ATTR
-    switch (pick(t)) {
-        case V_FAST: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, evg_step_tpm_kernel<11, 12, uint8_t, kFastPitch, false, kTpmThreads>, kTpmThreads, smem); break;
-        case V_GENERIC8: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, evg_step_tpm_kernel<0, 16, uint8_t, 0, true, kTpmThreads>, kTpmThreads, smem); break;
-        default: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, evg_step_tpm_kernel<0, 16, uint16_t, 0, true, kTpmThreads>, kTpmThreads, smem); break;
-    }
-    return e;
+    for (int c = 0; c < 8; ++c)  // every (agents, wire, roll) this simulator can launch with
+        if (const TpmKernel k = tpm_kernel(v, threads, c & 1, c & 2, c & 4))
+            if ((e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, limit)) != cudaSuccess) return e;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, plain, threads, smem);
 }
 
-// The float32 observation vector is the default output; the wire row (EVG_OBS_WIRE) has its own instantiations.  The
-// compile-time DemoMap kernel with scripted agents AND wire rows is not instantiated: that combination takes the
-// run-time-sized kernel, which serves every configuration.
+// The float32 observation vector is the default output; the wire row (EVG_OBS_WIRE) has its own instantiations.
 cudaError_t launch_step_tpm(const Tables& t, const StepArgs& a, int threads, size_t smem, int max_grid, cudaStream_t stream)
 {
-    const bool agents = a.agent[0] != EVG_AGENT_EXTERNAL || a.agent[1] != EVG_AGENT_EXTERNAL;
-    const bool wire = a.obs_fmt == EVG_OBS_WIRE;
     const bool roll = a.n_turns > 1;  // (evg_rollout: both players scripted, float32 observations)
-    if (roll && (wire || a.agent[0] == EVG_AGENT_EXTERNAL || a.agent[1] == EVG_AGENT_EXTERNAL)) return cudaErrorInvalidValue;
-    Variant v = pick(t);
-    if (v == V_FAST && agents && wire) {
-        v = V_GENERIC8;
-        threads = kTpmThreads;
-        smem = tpm_smem_bytes(t, threads);
-    }
+    if (roll && (a.agent[0] == EVG_AGENT_EXTERNAL || a.agent[1] == EVG_AGENT_EXTERNAL)) return cudaErrorInvalidValue;
+    const TpmKernel k = tpm_kernel(pick(t), threads, a.agent[0] != EVG_AGENT_EXTERNAL || a.agent[1] != EVG_AGENT_EXTERNAL,
+                                   a.obs_fmt == EVG_OBS_WIRE, roll);
+    if (!k) return cudaErrorInvalidValue;
     const int64_t nb = (a.n_envs + threads - 1) / threads;
     const unsigned grid = (unsigned)(nb < max_grid ? nb : max_grid);
-#define EVG_TPM_LAUNCH(...) evg_step_tpm_kernel<__VA_ARGS__><<<grid, threads, smem, stream>>>(t, a)
-    if (v == V_FAST && threads == kTpmSmallThreads) {
-        if (wire) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, false, kTpmSmallThreads, true);
-        else if (roll) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, true, kTpmSmallThreads, false, true);
-        else if (agents) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, true, kTpmSmallThreads);
-        else EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, false, kTpmSmallThreads);
-    } else if (v == V_FAST) {
-        if (wire) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, false, kTpmThreads, true);
-        else if (roll) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, true, kTpmThreads, false, true);
-        else if (agents) EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, true, kTpmThreads);
-        else EVG_TPM_LAUNCH(11, 12, uint8_t, kFastPitch, false, kTpmThreads);
-    } else if (v == V_GENERIC8) {
-        if (wire) EVG_TPM_LAUNCH(0, 16, uint8_t, 0, true, kTpmThreads, true);
-        else if (roll) EVG_TPM_LAUNCH(0, 16, uint8_t, 0, true, kTpmThreads, false, true);
-        else EVG_TPM_LAUNCH(0, 16, uint8_t, 0, true, kTpmThreads);
-    } else {
-        if (wire) EVG_TPM_LAUNCH(0, 16, uint16_t, 0, true, kTpmThreads, true);
-        else if (roll) EVG_TPM_LAUNCH(0, 16, uint16_t, 0, true, kTpmThreads, false, true);
-        else EVG_TPM_LAUNCH(0, 16, uint16_t, 0, true, kTpmThreads);
-    }
-#undef EVG_TPM_LAUNCH
+    k<<<grid, threads, smem, stream>>>(t, a);
     return cudaGetLastError();
 }
 

@@ -114,8 +114,9 @@ def test_step_host_compact_formats_through_the_chunk_pipeline(evg, cfg, fmt):
 
 
 def test_wire_with_fused_agents_takes_the_runtime_sized_kernel(evg, cfg, monkeypatch):
-    """Not an instantiated combination on the compile-time DemoMap kernel; the C ABI has no entry point for it either
-    (evg_step_agents writes float32), so this only pins the launcher's choice through evg_step_fmt's twin."""
+    """Scripted agents fused into a wire-row step are not instantiated on the compile-time DemoMap kernel, and no C ABI
+    entry point asks for them (evg_step_agents and evg_rollout write float32; the launcher refuses the combination).  The
+    wire step with rows from outside (here: random_actions) takes the DemoMap wire instantiation of 128-thread CTAs."""
     monkeypatch.setenv("EVG_STEP_KERNEL", "tpm")
     env = evg.BatchedEvergladesEnv(512, seed=1, config=cfg)
     env.reset()

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Build the library under another name with extra -D flags: kernel A/B runs without touching the in-tree libevgsim.so.
-#   tools/build_variant.sh NAME [-DEVG_TPM_STAGE=32 -DEVG_TPM_MIN_CTAS=3 ...]   ->  build/libevgsim_NAME.so
+#   tools/build_variant.sh NAME [-DEVG_CHECKED ...]   ->  build/libevgsim_NAME.so
 # Select it with EVGSIM_LIB=build/libevgsim_NAME.so (see tools/ab_variants.sh).  The sources and nvcc flags are those of
 # __graft_entry__.build().
 set -e
