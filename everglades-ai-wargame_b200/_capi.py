@@ -170,6 +170,11 @@ SYMBOLS = [
     ("evg_policy_mlp", C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
     ("evg_policy_ppo", C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     ("evg_policy_rppo", C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    ("evg_policy_mlp_fmt", C.c_int, [_P, C.c_int32, _P, C.c_int64, _P, _P, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
+    ("evg_policy_ppo_fmt", C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
+    ("evg_policy_rppo_fmt", C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                      _P, _P, _P, _P, _P]),
+    ("evg_wire_expand", C.c_int, [_P, _P, C.c_int64, _P, C.c_int64, C.c_int32, _P, _P, _P, _P]),
     ("evg_pack_mlp", C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     ("evg_pack_ppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_pack_rppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),

@@ -2,6 +2,7 @@
 // Validates the config, derives the device tables and launch geometry, and forwards every call to
 // the kernels of evg_kernels.cu.  Owns no device memory: all arrays are the caller's (evg_bind).
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
@@ -235,6 +236,18 @@ int check_sim(const EvgSim* s, bool need_bound)
     cudaError_t e = cudaSetDevice(s->device);
     if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
     return EVG_OK;
+}
+
+// where the wire-row expansion of a bound simulator finds the map's constant entries and player 1's node numbering
+evg::WireSrc wire_src(const EvgSim* s)
+{
+    evg::WireSrc w;
+    w.oconst = s->oconst_dev;
+    w.p1_map = reinterpret_cast<const uint8_t*>(s->tables_dev) + offsetof(evg::Tables, p1_map);
+    w.n_nodes = s->tables.n_nodes;
+    w.obs_len = s->tables.obs_len;
+    w.words = evg::wire_bytes(s->tables.n_nodes) / 4;
+    return w;
 }
 
 }  // namespace
@@ -904,16 +917,60 @@ int evg_decode_indices(EvgSim* sim, const int64_t* d_idx, int32_t div, int32_t m
     return EVG_OK;
 }
 
-int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_w1_img, const void* d_w2_img, int32_t hidden, int32_t out_dim,
-                   float* d_q, int32_t q_transposed, void* stream)
+// the observations of a policy call: float32 (wire = null) or, EVG_OBS_WIRE, rows whose expansion reads the bound tables
+static int policy_source(const char* fn, const EvgSim* sim, int32_t format, const void* d_obs, evg::WireSrc* wire, bool* use_wire)
+{
+    if (format != EVG_OBS_F32 && format != EVG_OBS_WIRE) return fail(EVG_E_ARG, "%s: observation format %d (EVG_OBS_F32 or EVG_OBS_WIRE)", fn, format);
+    *use_wire = format == EVG_OBS_WIRE;
+    if (!*use_wire) return EVG_OK;
+    if (!sim->is_bound) return fail(EVG_E_STATE, "%s: evg_bind() must be called before reading wire rows", fn);
+    if ((uintptr_t)d_obs % 16) return fail(EVG_E_ARG, "%s: wire rows must be 16-byte aligned", fn);
+    *wire = wire_src(sim);
+    return EVG_OK;
+}
+
+int evg_policy_mlp_fmt(EvgSim* sim, int32_t format, const void* d_obs, int64_t rows, const void* d_w1_img, const void* d_w2_img, int32_t hidden,
+                       int32_t out_dim, float* d_q, int32_t q_transposed, void* stream)
 {
     int rc = check_sim(sim, false);
     if (rc) return rc;
     if (!d_obs || !d_w1_img || !d_w2_img || !d_q || rows < 0) return fail(EVG_E_ARG, "evg_policy_mlp: null argument");
+    evg::WireSrc ws;
+    bool wire;
+    if ((rc = policy_source("evg_policy_mlp", sim, format, d_obs, &ws, &wire))) return rc;
+    if (wire && rows % 2) return fail(EVG_E_ARG, "evg_policy_mlp: %lld observation rows: wire rows hold both players, the count must be even", (long long)rows);
     if ((rc = check_mlp_shape("evg_policy_mlp", sim, hidden, out_dim, d_w1_img, d_w2_img))) return rc;
     const int n_chunks = (hidden + 1 + EVG_MLP_CHUNK - 1) / EVG_MLP_CHUNK;  // + the hidden unit that carries b2
-    cudaError_t e = evg::launch_policy_mlp(d_obs, rows, sim->layout.obs_len, d_w1_img, d_w2_img, n_chunks, out_dim, d_q, q_transposed, sim->sm_count, (cudaStream_t)stream);
+    cudaError_t e = evg::launch_policy_mlp(d_obs, rows, sim->layout.obs_len, d_w1_img, d_w2_img, n_chunks, out_dim, d_q, q_transposed, sim->sm_count,
+                                           (cudaStream_t)stream, wire ? &ws : nullptr);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_mlp_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_w1_img, const void* d_w2_img, int32_t hidden, int32_t out_dim,
+                   float* d_q, int32_t q_transposed, void* stream)
+{
+    return evg_policy_mlp_fmt(sim, EVG_OBS_F32, d_obs, rows, d_w1_img, d_w2_img, hidden, out_dim, d_q, q_transposed, stream);
+}
+
+int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                       const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions,
+                       int64_t* d_idx, float* d_probs, void* stream)
+{
+    int rc = check_sim(sim, true);  // the draws read turn and episode from the bound records
+    if (rc) return rc;
+    if (!d_obs || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias || !d_actions) return fail(EVG_E_ARG, "evg_policy_ppo: null argument");
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_ppo: player %d outside -1..1", player);
+    if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_ppo: div %d / mod %d must be positive", div, mod);
+    evg::WireSrc ws;
+    bool wire;
+    if ((rc = policy_source("evg_policy_ppo", sim, format, d_obs, &ws, &wire))) return rc;
+    if ((rc = check_actor_shape("evg_policy_ppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_w3_img}))) return rc;
+    cudaError_t e = evg::launch_policy_ppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
+                                           d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx, d_probs, sim->sm_count, (cudaStream_t)stream,
+                                           wire ? &ws : nullptr);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_ppo_kernel launch");
     sim->launches += 1;
     return EVG_OK;
 }
@@ -922,22 +979,13 @@ int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* 
                    const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions, int64_t* d_idx,
                    float* d_probs, void* stream)
 {
-    int rc = check_sim(sim, true);  // the draws read turn and episode from the bound records
-    if (rc) return rc;
-    if (!d_obs || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias || !d_actions) return fail(EVG_E_ARG, "evg_policy_ppo: null argument");
-    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_ppo: player %d outside -1..1", player);
-    if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_ppo: div %d / mod %d must be positive", div, mod);
-    if ((rc = check_actor_shape("evg_policy_ppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_w3_img}))) return rc;
-    cudaError_t e = evg::launch_policy_ppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
-                                           d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx, d_probs, sim->sm_count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_ppo_kernel launch");
-    sim->launches += 1;
-    return EVG_OK;
+    return evg_policy_ppo_fmt(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx,
+                              d_probs, stream);
 }
 
-int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_wi_img,
-                    const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
-                    float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
+int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                        const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim,
+                        int32_t div, int32_t mod, float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
 {
     int rc = check_sim(sim, true);  // the draws and the turn-0 reset of the state read the bound records
     if (rc) return rc;
@@ -946,11 +994,40 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
     if (!d_hidden) return fail(EVG_E_ARG, "evg_policy_rppo: d_hidden (the GRU state, in and out) is null");
     if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_rppo: player %d outside -1..1", player);
     if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_rppo: div %d / mod %d must be positive", div, mod);
+    evg::WireSrc ws;
+    bool wire;
+    if ((rc = policy_source("evg_policy_rppo", sim, format, d_obs, &ws, &wire))) return rc;
     if ((rc = check_actor_shape("evg_policy_rppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img}))) return rc;
     cudaError_t e = evg::launch_policy_rppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
                                             d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_hidden, d_actions, d_idx, d_probs,
-                                            sim->sm_count, (cudaStream_t)stream);
+                                            sim->sm_count, (cudaStream_t)stream, wire ? &ws : nullptr);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_rppo_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_wi_img,
+                    const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
+                    float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
+{
+    return evg_policy_rppo_fmt(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod,
+                               d_hidden, d_actions, d_idx, d_probs, stream);
+}
+
+int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64_t* d_index, int64_t n_out, int32_t player, float* d_obs,
+                    float* d_reward, uint8_t* d_done, void* stream)
+{
+    int rc = check_sim(sim, true);  // the constant entries and p1_map are in the bound tables
+    if (rc) return rc;
+    if (!d_rows || !d_obs) return fail(EVG_E_ARG, "evg_wire_expand: null argument");
+    if (n_rows < 0 || n_out < 0) return fail(EVG_E_ARG, "evg_wire_expand: negative row count");
+    if (!d_index && n_out != n_rows) return fail(EVG_E_ARG, "evg_wire_expand: without an index n_out (%lld) must equal n_rows (%lld)", (long long)n_out, (long long)n_rows);
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_wire_expand: player %d outside -1..1", player);
+    if (((uintptr_t)d_rows | (uintptr_t)d_obs) % 16 || (uintptr_t)d_index % 8 || (uintptr_t)d_reward % 4)
+        return fail(EVG_E_ARG, "evg_wire_expand: rows and obs must be 16-byte aligned, index 8-byte, reward 4-byte");
+    cudaError_t e = evg::launch_wire_expand(wire_src(sim), (const uint32_t*)d_rows, n_rows, d_index, n_out, player, d_obs, d_reward, d_done,
+                                            (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_wire_expand_kernel launch");
     sim->launches += 1;
     return EVG_OK;
 }

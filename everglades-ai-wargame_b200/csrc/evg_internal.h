@@ -133,6 +133,16 @@ __host__ __device__ inline int oconst_bytes(int n_nodes)
 // bytes of one match's wire row (include/evgsim.h, EVG_OBS_WIRE)
 __host__ __device__ inline int wire_bytes(int n_nodes) { return (EVG_WIRE_NODE0 + 4 * n_nodes + 3 * kGroupLanes + 8 + 15) / 16 * 16; }
 
+// What expanding a wire row into the float32 observation vector needs besides the row (evg_wire_expand.cu and the policy
+// kernels' wire stager): the simulator's constant entries (oconst_bytes layout, StepArgs::oconst_dev) and player 1's node
+// numbering (Tables::p1_map), both in the simulator's bound tables on the device
+struct WireSrc {
+    const float* oconst;
+    const uint8_t* p1_map;
+    int32_t n_nodes, obs_len;
+    int32_t words;  // 32-bit words of a row
+};
+
 // Kernels that need more than 48 KB of dynamic shared memory are opted in up to the DEVICE limit, not up to what one
 // simulator needs: the attribute is per function, and simulators of different configurations share the functions.
 inline cudaError_t optin_smem_limit(size_t needed, int* limit)
@@ -149,15 +159,19 @@ cudaError_t launch_step(const Tables& t, const StepArgs& a, int grid, size_t sme
 cudaError_t launch_rollout(const Tables& t, const StepArgs& a, int n_turns, int grid, size_t smem, cudaStream_t stream);
 cudaError_t launch_reset(const Tables& t, uint32_t* records, double* health, const uint8_t* mask, void* obs, int obs_fmt,
                          int64_t n_envs, int grid, size_t smem, cudaStream_t stream);
-cudaError_t launch_policy_mlp(const float* obs, int64_t rows, int in_dim, const void* w1_img, const void* w2_img, int n_chunks, int out_dim, float* q,
-                              int transposed, int sm_count, cudaStream_t stream);
-cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+// the policy launchers read float32 observations from `obs`, or wire rows when `wire` is not null
+cudaError_t launch_policy_mlp(const void* obs, int64_t rows, int in_dim, const void* w1_img, const void* w2_img, int n_chunks, int out_dim, float* q,
+                              int transposed, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
+cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
-                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream);
-cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
+cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
                                int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
-                               cudaStream_t stream);
+                               cudaStream_t stream, const WireSrc* wire = nullptr);
+// wire rows -> float32 observations, reward and done (evg_wire_expand.cu); index / reward / done may be null
+cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n_rows, const int64_t* index, int64_t n_out, int player,
+                               float* obs, float* reward, uint8_t* done, cudaStream_t stream);
 // the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();
@@ -213,6 +227,48 @@ struct Geo {
     __device__ __forceinline__ int obs_len() const { return 1 + 4 * n_nodes() + 5 * EVG_NUM_GROUPS; }
     __device__ __forceinline__ int rec_words8() const { return NODES ? ((kRecNode0 + NODES) * 4 + 31) / 32 * 4 : S.rec_words8; }
 };
+
+// Entry f (< obs_len) of player p's observation vector from a wire row (evgsim.wire.expand): every dynamic entry is one
+// field of one 32-bit word of the row — the turn and a node's control state are the low halves of words 0 and x (node id
+// x in real numbering), a unit count or a group byte is one byte — and the rest is a constant of the map (oconst).
+// wire_entry() says which word and how to read it; wire_value() reads it.  Only the group location of player 1 needs a
+// table lookup on the row's data (p1_map, clamped into the table for rows the step did not write).
+enum : uint32_t { kWireConst = 0, kWireU16, kWireS16, kWireByte, kWireLoc, kWireLocP1, kWireMoving };
+
+__device__ __forceinline__ int wire_entry(const WireSrc& w, int p, int f, uint32_t& op, uint32_t& shift)
+{
+    const int n = w.n_nodes;
+    shift = 0;
+    if (f == 0) {
+        op = kWireU16;
+        return 0;
+    }
+    if (f <= 4 * n) {  // node slot k of the viewer: DEFENSE, OBSERVE, control state, the OTHER player's units
+        const int k = (f - 1) >> 2, j = (f - 1) & 3;
+        op = j < 2 ? kWireConst : j == 2 ? kWireS16 : kWireByte;
+        shift = 8 * (3 - p);
+        return p ? __ldg(w.p1_map + k + 1) : k + 1;
+    }
+    const int t = f - 1 - 4 * n, g = t / 5, j = t - 5 * g;  // group g: location, type, avg health, moving, units alive
+    const int b = EVG_WIRE_NODE0 + 4 * n + 3 * (EVG_NUM_GROUPS * p + g) + (j == 2 ? 1 : j == 4 ? 2 : 0);
+    op = j == 1 ? kWireConst : j == 0 ? (p ? kWireLocP1 : kWireLoc) : j == 3 ? kWireMoving : kWireByte;
+    shift = 8 * (b & 3);
+    return b >> 2;
+}
+
+__device__ __forceinline__ float wire_value(const WireSrc& w, int p, int f, uint32_t op, uint32_t shift, uint32_t word)
+{
+    const uint32_t byte = (word >> shift) & 0xFFu;
+    switch (op) {
+        case kWireU16: return (float)(word & 0xFFFFu);
+        case kWireS16: return (float)(int16_t)(word & 0xFFFFu);
+        case kWireByte: return (float)byte;
+        case kWireLoc: return (float)(byte & 63u);
+        case kWireLocP1: return (float)__ldg(w.p1_map + min(byte & 63u, (uint32_t)(kNN - 1)));
+        case kWireMoving: return (float)(byte >> 6);
+        default: return __ldg(w.oconst + p * w.obs_len + f);
+    }
+}
 
 // Philox4x32-10 (Salmon et al., SC'11); same function as oracle/tape.py, oracle/evg_oracle.c.
 __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,

@@ -53,10 +53,12 @@ static_assert(kSmH % 1024 == 0 && kSmW1 % 1024 == 0 && kSmW2 % 1024 == 0 && (kOu
 constexpr int kTmemD1 = 0, kTmemD2 = 256;  // D1 (192 columns) and D2 (144) in the 512 of kTmemCols
 
 // q_col_stride == 1: Q[row * q_row_stride + col] (row-major); q_row_stride == 1: Q[col * q_col_stride + row] (transposed)
+// kWire: obs holds wire rows (ws), observation row i = (match i / 2, player i % 2); else float32 rows
+template <bool kWire>
 __global__ void __launch_bounds__(kCtaThreads, 1)
-evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, const unsigned char* __restrict__ w1_img,
+evg_policy_mlp_kernel(const void* __restrict__ obs, int64_t rows, int in_dim, const unsigned char* __restrict__ w1_img,
                       const unsigned char* __restrict__ w2_img, int n_chunks, int out_dim, float* __restrict__ q, int64_t q_row_stride,
-                      int64_t q_col_stride)
+                      int64_t q_col_stride, const __grid_constant__ WireSrc ws)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -75,15 +77,15 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
         bulk_load(smem + kSmW1, w1_img, kW1ChunkBytes, &bar[2]);
         bulk_load(smem + kSmW2, w2_img, kW2ChunkBytes, &bar[3]);
     }
-    ObsTile<true> a_tile;  // A: feature in_dim is the constant 1 that carries b1
+    Stager<kWire, true> a_tile;  // A: feature in_dim is the constant 1 that carries b1
     int64_t step = 0;
     bool l1_queued = false;  // the coming tile's first layer-1 MMAs were issued at the end of the previous tile
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int64_t row0 = tile * kTileM;
         const int nrows = rows - row0 < kTileM ? (int)(rows - row0) : kTileM;
         if (tile == (int64_t)blockIdx.x) {  // the first tile: later ones are fetched and converted under the previous tile's last chunk
-            a_tile.load(tid, obs, row0, rows, in_dim, -1);
-            a_tile.store(tid, smem + kSmA);
+            a_tile.load(tid, obs, row0, rows, in_dim, -1, ws);
+            a_tile.store(tid, smem + kSmA, in_dim, -1, ws);
             fence_async_smem();
             __syncthreads();
         }
@@ -109,7 +111,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             tc_fence_after();
             if (tid == 0 && step + 1 < n_steps) bulk_load(smem + kSmW1, w1_img + (size_t)cn * kW1ChunkBytes, kW1ChunkBytes, &bar[2]);
             const bool fetch_next_a = c + 1 == n_chunks && tile + gridDim.x < n_tiles;  // this tile's last layer-1 MMAs have read A: it is free
-            if (fetch_next_a) a_tile.load(tid, obs, (tile + gridDim.x) * kTileM, rows, in_dim, -1);  // in flight under the epilogue below
+            if (fetch_next_a) a_tile.load(tid, obs, (tile + gridDim.x) * kTileM, rows, in_dim, -1, ws);  // in flight under the epilogue below
             // ---- hidden activations of my row, my 48 of the chunk's 192 columns: TMEM -> registers -> ReLU, bf16 -> swizzled H
             {
                 constexpr int kLd = kChunk / 4 / 16;  // tensor-memory loads of 16 columns per thread: all issued, then one wait
@@ -149,7 +151,7 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
             }
             ph_w2 ^= 1;
             if (fetch_next_a) {  // the next tile's A, converted while layer 2 runs
-                a_tile.store(tid, smem + kSmA);
+                a_tile.store(tid, smem + kSmA, in_dim, -1, ws);
                 fence_async_smem();
                 __syncthreads();
                 // ... and its first layer-1 MMAs queued now: they only write D1, so they run under this tile's Q store
@@ -189,14 +191,18 @@ evg_policy_mlp_kernel(const float* __restrict__ obs, int64_t rows, int in_dim, c
 
 }  // namespace
 
-cudaError_t launch_policy_mlp(const float* obs, int64_t rows, int in_dim, const void* w1_img, const void* w2_img, int n_chunks, int out_dim, float* q,
-                              int transposed, int sm_count, cudaStream_t stream)
+cudaError_t launch_policy_mlp(const void* obs, int64_t rows, int in_dim, const void* w1_img, const void* w2_img, int n_chunks, int out_dim, float* q,
+                              int transposed, int sm_count, cudaStream_t stream, const WireSrc* wire)
 {
-    return launch_persistent(evg_policy_mlp_kernel, rows, sm_count, kSmBytes, stream, obs, rows, in_dim, reinterpret_cast<const unsigned char*>(w1_img),
-                             reinterpret_cast<const unsigned char*>(w2_img), n_chunks, out_dim, q, (int64_t)(transposed ? 1 : out_dim),
-                             (int64_t)(transposed ? rows : 1));
+    return launch_persistent(wire ? evg_policy_mlp_kernel<true> : evg_policy_mlp_kernel<false>, rows, sm_count, kSmBytes, stream, obs, rows, in_dim,
+                             reinterpret_cast<const unsigned char*>(w1_img), reinterpret_cast<const unsigned char*>(w2_img), n_chunks, out_dim, q,
+                             (int64_t)(transposed ? 1 : out_dim), (int64_t)(transposed ? rows : 1), wire ? *wire : WireSrc{});
 }
 
-cudaError_t set_policy_mlp_smem() { return cudaFuncSetAttribute(evg_policy_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
+cudaError_t set_policy_mlp_smem()
+{
+    cudaError_t e = cudaFuncSetAttribute(evg_policy_mlp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(evg_policy_mlp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+}
 
 }  // namespace evg

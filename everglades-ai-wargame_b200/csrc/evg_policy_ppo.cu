@@ -58,7 +58,9 @@ static_assert(kSmBytes <= 227 * 1024, "shared memory");
 constexpr int kTmemD1 = 0, kTmemD2 = 256;  // D3 reuses D1's columns (read out before layer 3 is issued)
 
 // nk: chunks of 128 K-columns of layers 2 and 3
-__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __grid_constant__ ActorArgs a, const int nk)
+// kWire: the observations are wire rows (ws), else float32
+template <bool kWire>
+__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __grid_constant__ ActorArgs a, const int nk, const __grid_constant__ WireSrc ws)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -116,15 +118,15 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
         ph_m ^= 1;
         tc_fence_after();
     };
-    ObsTile<false> a_tile;  // A
+    Stager<kWire, false> a_tile;  // A
 
     if (tid == 0) {
         load_piece(0);
         load_piece(1);
     }
     if (my_tiles > 0) {
-        a_tile.load(tid, a.obs, (int64_t)blockIdx.x * kTileM, a.rows, a.in_dim, a.player);
-        a_tile.store(tid, smem + kSmA);
+        a_tile.load(tid, a.obs, (int64_t)blockIdx.x * kTileM, a.rows, a.in_dim, a.player, ws);
+        a_tile.store(tid, smem + kSmA, a.in_dim, a.player, ws);
         fence_async_smem();
     }
     __syncthreads();
@@ -162,7 +164,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
         if (tid == 0)
             for (int c = 0; c < nk; ++c) load_piece(s0 + 3 + nk + c);
         const bool next = tile + gridDim.x < n_tiles;
-        if (next) a_tile.load(tid, a.obs, (tile + gridDim.x) * kTileM, a.rows, a.in_dim, a.player);  // in flight under the epilogue and the sampling
+        if (next) a_tile.load(tid, a.obs, (tile + gridDim.x) * kTileM, a.rows, a.in_dim, a.player, ws);  // in flight under the epilogue and the sampling
         // ---- e = exp(tanh(D3 + b3)) of my row, my 16-column groups, into ps[j][row] (A and H are free: layer 3 has retired)
         {
             constexpr int kG = (kOutPad / 16 + 3) / 4;
@@ -231,7 +233,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
         }
         __syncthreads();  // the probabilities are read: A may be overwritten
         if (next) {
-            a_tile.store(tid, smem + kSmA);
+            a_tile.store(tid, smem + kSmA, a.in_dim, a.player, ws);
             fence_async_smem();
         }
         tc_fence_before();
@@ -242,14 +244,19 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
 
 }  // namespace
 
-cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
-                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream)
+                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream, const WireSrc* wire)
 {
     const ActorArgs a = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
-    return launch_persistent(evg_policy_ppo_kernel, a.rows, sm_count, kSmBytes, stream, a, (a.lp + 127) / 128);
+    return launch_persistent(wire ? evg_policy_ppo_kernel<true> : evg_policy_ppo_kernel<false>, a.rows, sm_count, kSmBytes, stream, a,
+                             (a.lp + 127) / 128, wire ? *wire : WireSrc{});
 }
 
-cudaError_t set_policy_ppo_smem() { return cudaFuncSetAttribute(evg_policy_ppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
+cudaError_t set_policy_ppo_smem()
+{
+    cudaError_t e = cudaFuncSetAttribute(evg_policy_ppo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(evg_policy_ppo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+}
 
 }  // namespace evg

@@ -75,7 +75,9 @@ struct RppoArgs : ActorArgs {
 
 __device__ __forceinline__ float sigmoid(float v) { return __frcp_rn(1.f + expf(-v)); }  // = 1 / (1 + e^-v), correctly rounded
 
-__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const __grid_constant__ RppoArgs a)
+// kWire: the observations are wire rows (ws), else float32
+template <bool kWire>
+__global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const __grid_constant__ RppoArgs a, const __grid_constant__ WireSrc ws)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -219,9 +221,9 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
         const int nrows = a.rows - row0 < kTileM ? (int)(a.rows - row0) : kTileM;
         // ---- the observation tile -> bf16 into H; h0 of my row into registers (0 at turn 0)
         {
-            ObsTile<false> obs_tile;
-            obs_tile.load(tid, a.obs, row0, a.rows, a.in_dim, a.player);
-            obs_tile.store(tid, smem + kSmH);
+            Stager<kWire, false> obs_tile;
+            obs_tile.load(tid, a.obs, row0, a.rows, a.in_dim, a.player, ws);
+            obs_tile.store(tid, smem + kSmH, a.in_dim, a.player, ws);
         }
         fence_async_smem();
         const int64_t my_row = row0 + r;
@@ -419,10 +421,10 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
 
 }  // namespace
 
-cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
                                int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
-                               cudaStream_t stream)
+                               cudaStream_t stream, const WireSrc* wire)
 {
     RppoArgs a;
     static_cast<ActorArgs&>(a) = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
@@ -432,9 +434,14 @@ cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const f
     a.latent = latent;
     a.ka = (latent + kAtomK - 1) / kAtomK;
     a.nrb = (a.lp + kPieceRows - 1) / kPieceRows;
-    return launch_persistent(evg_policy_rppo_kernel, a.rows, sm_count, kSmBytes, stream, a);
+    return launch_persistent(wire ? evg_policy_rppo_kernel<true> : evg_policy_rppo_kernel<false>, a.rows, sm_count, kSmBytes, stream, a,
+                             wire ? *wire : WireSrc{});
 }
 
-cudaError_t set_policy_rppo_smem() { return cudaFuncSetAttribute(evg_policy_rppo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes); }
+cudaError_t set_policy_rppo_smem()
+{
+    cudaError_t e = cudaFuncSetAttribute(evg_policy_rppo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(evg_policy_rppo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+}
 
 }  // namespace evg

@@ -6,6 +6,8 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "evg_internal.h"
 
 namespace evg {
@@ -26,7 +28,7 @@ __host__ __device__ inline int swz_offset(int rows, int r, int k)
 
 // the fields evg_policy_ppo_kernel and evg_policy_rppo_kernel share (filled by actor_args)
 struct ActorArgs {
-    const float* obs;
+    const void* obs;  // float32 observations or wire rows
     const unsigned char* w1;
     const unsigned char* w2;
     const unsigned char* w3;
@@ -40,7 +42,7 @@ struct ActorArgs {
     uint32_t env_base, seed_lo, seed_hi;
 };
 
-inline ActorArgs actor_args(const Tables& t, const uint32_t* records, const float* obs, int64_t n_envs, int player, const void* w1_img,
+inline ActorArgs actor_args(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                             const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
                             int8_t* actions, int64_t* idx, float* probs)
 {
@@ -210,8 +212,9 @@ struct ObsTile {
     static constexpr int kIt = kTileM * (kObsCols / 8) / kCtaThreads;
     float f[kIt][8];
 
-    __device__ __forceinline__ void load(int tid, const float* obs, int64_t row0, int64_t rows, int in_dim, int player)
+    __device__ __forceinline__ void load(int tid, const void* src_obs, int64_t row0, int64_t rows, int in_dim, int player, const WireSrc&)
     {
+        const float* obs = static_cast<const float*>(src_obs);
 #pragma unroll
         for (int it = 0; it < kIt; ++it) {
             const int i = tid + it * kCtaThreads, ar = i >> 4, k0 = (i & 15) * 8;
@@ -221,7 +224,7 @@ struct ObsTile {
             for (int e = 0; e < 8; ++e) f[it][e] = (row < rows && k0 + e < in_dim) ? __ldcs(src + e) : (kBiasColumn && k0 + e == in_dim ? 1.f : 0.f);
         }
     }
-    __device__ __forceinline__ void store(int tid, unsigned char* dst) const
+    __device__ __forceinline__ void store(int tid, unsigned char* dst, int, int, const WireSrc&) const
     {
 #pragma unroll
         for (int it = 0; it < kIt; ++it) {
@@ -231,6 +234,71 @@ struct ObsTile {
         }
     }
 };
+
+// The same tile from wire rows (EVG_OBS_WIRE): tile row ar = batch row row0 + ar is (match, player) = (row / 2, row % 2)
+// when player < 0, else (row, player), and its values are what evg_wire_expand writes (wire_entry / wire_value).  The
+// 16 threads that build a tile row (a half-warp: 8 features each) load its match's row together, word j + 16 q into
+// thread j (kWords = 3 covers the 160-byte rows of a 16-node map; words past the row are not read): 8 bytes in flight per
+// thread and tile row on DemoMap, 12 at 16 nodes, against the 32 of the float32 stager.  store() takes each entry's word
+// from the thread that holds it with a shuffle inside the half-warp, so the stager needs no shared memory of its own.
+// A thread's 8 features and its player are the same for every tile row it builds, so each entry's source is worked out
+// once per store() and used for all kIt rows.
+template <bool kBiasColumn>
+struct WireTile {
+    static constexpr int kIt = ObsTile<kBiasColumn>::kIt;
+    static constexpr int kWords = 3;
+    uint32_t w[kIt][kWords];
+    uint32_t live;  // bit it: the tile row of iteration it is a batch row
+
+    __device__ __forceinline__ void load(int tid, const void* src_rows, int64_t row0, int64_t rows, int, int player, const WireSrc& ws)
+    {
+        const uint32_t* base = static_cast<const uint32_t*>(src_rows);
+        const int j = tid & 15;
+        live = 0;
+#pragma unroll
+        for (int it = 0; it < kIt; ++it) {
+            const int64_t row = row0 + ((tid + it * kCtaThreads) >> 4);
+            const uint32_t* src = base + (player < 0 ? row >> 1 : row) * ws.words + j;
+            if (row < rows) live |= 1u << it;
+#pragma unroll
+            for (int q = 0; q < kWords; ++q) w[it][q] = (row < rows && j + 16 * q < ws.words) ? __ldcs(src + 16 * q) : 0u;
+        }
+    }
+    __device__ __forceinline__ void store(int tid, unsigned char* dst, int in_dim, int player, const WireSrc& ws) const
+    {
+        const int k0 = (tid & 15) * 8, p = player < 0 ? (tid >> 4) & 1 : player;
+        uint32_t packed[kIt][4];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+            const int k = k0 + e;
+            uint32_t op = kWireConst, shift = 0;
+            const int wi = k < in_dim ? wire_entry(ws, p, k, op, shift) : 0;
+            const float pad = kBiasColumn && k == in_dim ? 1.f : 0.f;
+            const float cst = k < in_dim && op == kWireConst ? wire_value(ws, p, k, op, 0, 0u) : pad;
+#pragma unroll
+            for (int it = 0; it < kIt; ++it) {
+                uint32_t word = 0;
+#pragma unroll
+                for (int q = 0; q < kWords; ++q) {
+                    const uint32_t v = __shfl_sync(0xFFFFFFFFu, w[it][q], wi & 15, 16);
+                    if ((wi >> 4) == q) word = v;
+                }
+                const float x = !(live >> it & 1u) ? pad : op == kWireConst ? cst : wire_value(ws, p, k, op, shift, word);
+                const uint32_t b = pack_bf16(x, 0.f) & 0xFFFFu;
+                packed[it][e >> 1] = (e & 1) ? packed[it][e >> 1] | b << 16 : b;
+            }
+        }
+#pragma unroll
+        for (int it = 0; it < kIt; ++it) {
+            const int ar = (tid + it * kCtaThreads) >> 4;
+            *reinterpret_cast<uint4*>(dst + swz_offset(kTileM, ar, k0)) = make_uint4(packed[it][0], packed[it][1], packed[it][2], packed[it][3]);
+        }
+    }
+};
+
+// the observation stager of a policy kernel: float32 observations, or wire rows (kWire)
+template <bool kWire, bool kBiasColumn>
+using Stager = std::conditional_t<kWire, WireTile<kBiasColumn>, ObsTile<kBiasColumn>>;
 
 // a PPO actor's hidden-layer epilogue: row r, the 16-column groups 16 quarter, + 64, ... below lp of the accumulators at
 // TMEM address `taddr` (the thread's lane base + the layer's column): dst = bf16(tanh(D + b)), swizzled; then dst is made

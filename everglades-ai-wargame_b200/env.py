@@ -384,6 +384,51 @@ class BatchedEvergladesEnv:
                                                C.c_void_p(self.obs.data_ptr()), C.c_void_p(out.data_ptr()), self._stream()))
         return out
 
+    def expand_wire(self, rows, index=None, player=-1, out=None, reward=None, done=None):
+        """Wire rows uint8 [M, row_bytes] (obs_rows('wire') of some turn, or rows stored since) -> the float32
+        observations on the device, bit for bit what the step writes in the f32 format (evg_wire_expand).  Output row i
+        expands rows[index[i]] (index: int64 [K] on the device; None: row i), so a replay memory expands a sampled
+        minibatch in one launch; an index outside [0, M) gives a row of zeros (reward 0, done 0).  player -1: float32
+        [K, 2, L]; 0 or 1: [K, L].  reward (float32 [K, 2]) and done (uint8 [K]) are filled when given.  Returns `out`
+        (allocated when None).  ValueError, before anything is launched, for a tensor of the wrong dtype, width, shape or
+        device, or one that is not contiguous."""
+        torch = _torch()
+        rb = int(self._lib.evg_obs_row_bytes(self._h, _capi.OBS_WIRE))
+
+        def need(name, t, dtype, shape):
+            if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != self.device or not t.is_contiguous() \
+                    or (shape is not None and tuple(t.shape) != shape):
+                raise ValueError("%s must be a contiguous %s tensor%s on %s, got %s" % (
+                    name, dtype, "" if shape is None else " of shape %s" % (shape,), self.device,
+                    "%s %s%s on %s" % (t.dtype, tuple(t.shape), "" if t.is_contiguous() else " (not contiguous)", t.device)
+                    if isinstance(t, torch.Tensor) else type(t).__name__))
+
+        need("rows", rows, torch.uint8, None)
+        if rows.dim() != 2 or rows.shape[1] != rb:
+            raise ValueError("rows must be [M, %d] wire rows of this map, got shape %s" % (rb, tuple(rows.shape)))
+        if player not in (-1, 0, 1):
+            raise ValueError("player must be -1, 0 or 1, got %r" % (player,))
+        if index is not None:
+            need("index", index, torch.int64, None)
+            if index.dim() != 1:
+                raise ValueError("index must be one-dimensional, got shape %s" % (tuple(index.shape),))
+        k = rows.shape[0] if index is None else index.shape[0]
+        shape = (k, 2, self.obs_len) if player < 0 else (k, self.obs_len)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        need("out", out, torch.float32, shape)
+        if reward is not None:
+            need("reward", reward, torch.float32, (k, 2))
+        if done is not None:
+            need("done", done, torch.uint8, (k,))
+
+        def ptr(t):
+            return None if t is None else C.c_void_p(t.data_ptr())
+
+        _capi.check(self._lib.evg_wire_expand(self._h, ptr(rows), rows.shape[0], ptr(index), k, int(player), ptr(out), ptr(reward),
+                                              ptr(done), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ snapshots
     def get_state(self, first=0, count=None):
         """numpy structured array (dtype _capi.env_state_dtype()) of matches [first, first+count)."""

@@ -121,6 +121,28 @@ def _refresh_sources(fused, net, params_of, shapes):
     return [C.c_void_p(t.data_ptr()) for t in params]
 
 
+def _wire_rows(env, obs, obs_format):
+    """The observations a fused policy reads: (format code, tensor).  'f32' is env.obs; 'wire' is env.obs_rows('wire'),
+    or `obs` when given, a contiguous uint8 [num_envs, row_bytes] tensor on the env's device (ValueError otherwise, and
+    for a map whose observations do not fit the kernels' 128 input columns, before anything is launched)."""
+    import torch
+    if obs_format not in ("f32", "wire"):
+        raise ValueError("obs_format must be 'f32' or 'wire', got %r" % (obs_format,))
+    if obs_format == "f32":
+        return _capi.OBS_F32, obs
+    if env.obs_len >= PPO_IN_PAD:
+        raise ValueError("observations of %d values do not fit the %d input columns of the fused kernels" % (env.obs_len, PPO_IN_PAD))
+    rb = int(env._lib.evg_obs_row_bytes(env._h, _capi.OBS_WIRE))
+    if obs is None:
+        return _capi.OBS_WIRE, env.obs_rows("wire")
+    if not isinstance(obs, torch.Tensor) or obs.dtype != torch.uint8 or not obs.is_contiguous() or obs.device != env.device \
+            or tuple(obs.shape) != (env.num_envs, rb):
+        raise ValueError("wire rows must be a contiguous uint8 tensor of shape (%d, %d) on %s, got %s" % (
+            env.num_envs, rb, env.device, "%s %s%s on %s" % (obs.dtype, tuple(obs.shape), "" if obs.is_contiguous() else " (not contiguous)",
+                                                          obs.device) if isinstance(obs, torch.Tensor) else type(obs).__name__))
+    return _capi.OBS_WIRE, obs
+
+
 class FusedDQN:
     """Q-network forward + decode for a BatchedEvergladesEnv: ``actions = FusedDQN(env, net)()`` reads env.obs in place."""
 
@@ -155,34 +177,37 @@ class FusedDQN:
         _capi.check(env._lib.evg_pack_mlp(env._h, w1, b1, w2, b2, h, o, C.c_void_p(self._w1.data_ptr()),
                                           C.c_void_p(self._w2.data_ptr()), env._stream()))
 
-    def _run(self, obs, out, transposed):
+    def _run(self, obs, out, transposed, obs_format="f32"):
         env = self.env
+        fmt, obs = _wire_rows(env, obs, obs_format)
         if obs is None:
             obs = env.obs
-        else:  # the kernel reads num_envs * 2 rows of obs_len float32 values from obs.data_ptr(), whatever obs is
+        elif fmt == _capi.OBS_F32:  # the kernel reads num_envs * 2 rows of obs_len float32 values from obs.data_ptr(), whatever obs is
             import torch
             if obs.dtype != torch.float32 or not obs.is_contiguous() or obs.device != env.device \
                     or obs.numel() != env.num_envs * 2 * env.obs_len:
                 raise ValueError("obs must be a contiguous float32 tensor of %d x 2 x %d values on %s, got %s %s%s on %s"
                                  % (env.num_envs, env.obs_len, env.device, obs.dtype, tuple(obs.shape),
                                     "" if obs.is_contiguous() else " (not contiguous)", obs.device))
-        _capi.check(env._lib.evg_policy_mlp(env._h, C.c_void_p(obs.data_ptr()), env.num_envs * 2, C.c_void_p(self._w1.data_ptr()),
-                                            C.c_void_p(self._w2.data_ptr()), self.hidden, self.out_dim, C.c_void_p(out.data_ptr()),
-                                            int(transposed), env._stream()))
+        _capi.check(env._lib.evg_policy_mlp_fmt(env._h, fmt, C.c_void_p(obs.data_ptr()), env.num_envs * 2, C.c_void_p(self._w1.data_ptr()),
+                                                C.c_void_p(self._w2.data_ptr()), self.hidden, self.out_dim, C.c_void_p(out.data_ptr()),
+                                                int(transposed), env._stream()))
         return out
 
-    def forward(self, obs=None):
-        """Q-values float32 [N, 2, out] for `obs` (default: the environment's own observation tensor)."""
-        return self._run(obs, self.q, False)
+    def forward(self, obs=None, obs_format="f32"):
+        """Q-values float32 [N, 2, out] for `obs` (default: the environment's own observation tensor).  obs_format 'wire':
+        the wire rows of env.obs_rows('wire'), or `obs` as uint8 [N, row_bytes] rows (e.g. a replay minibatch gathered
+        with index_select); the Q-values are bit for bit those of the float32 observations the rows expand to."""
+        return self._run(obs, self.q, False, obs_format)
 
-    def forward_t(self, obs=None):
+    def forward_t(self, obs=None, obs_format="f32"):
         """The same Q-values transposed, float32 [out, N * 2]: what the decode reads coalesced."""
-        return self._run(obs, self.qt, True)
+        return self._run(obs, self.qt, True, obs_format)
 
-    def __call__(self):
+    def __call__(self, obs_format="f32"):
         """Action rows int8 [N, 2, 7, 2] for both players: forward, then DQNAgent.filter_actions on the device."""
         env = self.env
-        qt = self.forward_t()
+        qt = self.forward_t(obs_format=obs_format)
         assert self.out_dim % _capi.NUM_GROUPS == 0
         _capi.check(env._lib.evg_decode_dqn_layout(env._h, C.c_void_p(qt.data_ptr()), self.out_dim // _capi.NUM_GROUPS, -1, 1,
                                                    C.c_void_p(env._actions.data_ptr()), env._stream()))
@@ -222,8 +247,8 @@ def reference_forward_ppo(obs, w1, b1, w2, b2, w3, b3):
 
 class FusedPPO:
     """PPO actor forward + PPOAgent.get_action's sampling for a BatchedEvergladesEnv, in one kernel:
-    ``actions = FusedPPO(env, net)()`` reads env.obs in place (so the env must be stepped in the f32 format) and writes
-    env._actions.  The draws come from the tape (seed, global match id, turn, episode, player), not from torch's
+    ``actions = FusedPPO(env, net)()`` reads env.obs in place (or, with obs_format='wire', the env's wire rows) and
+    writes env._actions.  The draws come from the tape (seed, global match id, turn, episode, player), not from torch's
     generator: the rows do not depend on batch size, sharding or call order.  `player` -1 plays both sides, 0 or 1 only
     that side's rows (the other side's rows are left as they are, e.g. for a scripted opponent)."""
 
@@ -256,15 +281,18 @@ class FusedPPO:
         w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
         _capi.check(env._lib.evg_pack_ppo(env._h, *src, L, o, w1, w2, w3, bias, env._stream()))
 
-    def __call__(self, want_probs=False):
+    def __call__(self, want_probs=False, obs_format="f32"):
         """Action rows int8 [N, 2, 7, 2] (env._actions); fills .idx (int64 [N, 2, 7] or [N, 7]) and, with want_probs,
-        .probs (float32 [N, 2, out] or [N, out])."""
+        .probs (float32 [N, 2, out] or [N, out]).  obs_format 'wire' reads env.obs_rows('wire') (the env stepped with
+        obs_format='wire'), with results bit for bit those of the float32 observations."""
         env = self.env
+        fmt, obs = _wire_rows(env, None, obs_format)
+        obs = env.obs if obs is None else obs
         w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
-        _capi.check(env._lib.evg_policy_ppo(env._h, C.c_void_p(env.obs.data_ptr()), self.player, w1, w2, w3, bias, self.latent,
-                                            self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
-                                            C.c_void_p(self.idx.data_ptr()), C.c_void_p(self.probs.data_ptr()) if want_probs else None,
-                                            env._stream()))
+        _capi.check(env._lib.evg_policy_ppo_fmt(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, w3, bias, self.latent,
+                                                self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
+                                                C.c_void_p(self.idx.data_ptr()), C.c_void_p(self.probs.data_ptr()) if want_probs else None,
+                                                env._stream()))
         return env._actions
 
 
@@ -350,7 +378,7 @@ def reference_forward_rppo(obs, h0, weights, bf16=True):
 
 class FusedRPPO:
     """PPO's recurrent actor + its 7 draws for a BatchedEvergladesEnv, in one kernel: ``actions = FusedRPPO(env, actor)()``
-    reads env.obs in place (the env must be stepped in the f32 format), steps the GRU state ``.hidden`` and writes
+    reads env.obs in place (or, with obs_format='wire', the env's wire rows), steps the GRU state ``.hidden`` and writes
     env._actions.  ``.hidden`` (float32 [N, 2, L], or [N, L] for one player; zero at construction) is read and written
     back by every call, and a row restarts from zero when its match's record is at turn 0 (after reset() and after an
     automatic reset): under AUTORESET_TERMINAL / _NEXT that is the ``hidden *= 1 - done`` mask of a torch rollout.  Under
@@ -386,13 +414,16 @@ class FusedRPPO:
         _capi.check(env._lib.evg_pack_rppo(env._h, w1, b1, w2, b2, w3, b3, wi, bi, wh, bh, L, o, i1, i2, ii, ih, i3, bias,
                                            env._stream()))
 
-    def __call__(self, want_probs=False):
+    def __call__(self, want_probs=False, obs_format="f32"):
         """Action rows int8 [N, 2, 7, 2] (env._actions); steps .hidden, fills .idx (int64 [N, 2, 7] or [N, 7]) and, with
-        want_probs, .probs (float32 [N, 2, 7, out] or [N, 7, out]: step k's distribution)."""
+        want_probs, .probs (float32 [N, 2, 7, out] or [N, 7, out]: step k's distribution).  obs_format 'wire' reads
+        env.obs_rows('wire'), as FusedPPO does."""
         env = self.env
+        fmt, obs = _wire_rows(env, None, obs_format)
+        obs = env.obs if obs is None else obs
         w1, w2, wi, wh, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
-        _capi.check(env._lib.evg_policy_rppo(env._h, C.c_void_p(env.obs.data_ptr()), self.player, w1, w2, wi, wh, w3, bias, self.latent,
-                                             self.out_dim, self.div, self.mod, C.c_void_p(self.hidden.data_ptr()),
-                                             C.c_void_p(env._actions.data_ptr()), C.c_void_p(self.idx.data_ptr()),
-                                             C.c_void_p(self.probs.data_ptr()) if want_probs else None, env._stream()))
+        _capi.check(env._lib.evg_policy_rppo_fmt(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, wi, wh, w3, bias, self.latent,
+                                                 self.out_dim, self.div, self.mod, C.c_void_p(self.hidden.data_ptr()),
+                                                 C.c_void_p(env._actions.data_ptr()), C.c_void_p(self.idx.data_ptr()),
+                                                 C.c_void_p(self.probs.data_ptr()) if want_probs else None, env._stream()))
         return env._actions

@@ -371,6 +371,36 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
                     const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
                     float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream);
 
+/* The three policy calls above with the observations in `format` (EVG_OBS_*); with EVG_OBS_F32 they ARE those calls.
+ * EVG_OBS_WIRE: d_obs holds wire rows (evg_obs_row_bytes(sim, EVG_OBS_WIRE) bytes each, 16-byte aligned) — the rows
+ * evg_step_fmt wrote, or any rows of the same map (a replay minibatch) — and the kernels stage from them exactly the
+ * bf16 operands they stage from the float32 vector evg_wire_expand would write, so every output is bit for bit that of
+ * the float32 call on the expanded rows.  The actors read n_envs rows (match m's row is row m); evg_policy_mlp_fmt reads
+ * rows / 2 of them (observation row i = player i % 2 of wire row i / 2; rows must be even).  Needs evg_bind (the rows
+ * expand through the bound tables).  EVG_OBS_I16 and unknown formats return EVG_E_ARG. */
+int evg_policy_mlp_fmt(EvgSim* sim, int32_t format, const void* d_obs, int64_t rows, const void* d_w1_img, const void* d_w2_img, int32_t hidden,
+                       int32_t out_dim, float* d_q, int32_t q_transposed, void* stream);
+int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                       const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions,
+                       int64_t* d_idx, float* d_probs, void* stream);
+int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                        const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim,
+                        int32_t div, int32_t mod, float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream);
+
+/* Wire rows -> the float32 observation vector on the device (csrc/evg_wire_expand.cu), bit for bit what the step writes
+ * in EVG_OBS_F32 and what evgsim.wire.expand computes on the host; for training consumers that store the rows (a replay or
+ * rollout memory: 128 bytes per match on DemoMap against 840) and expand a sampled minibatch.
+ *   d_rows:   n_rows wire rows of this simulator's map (16-byte aligned).
+ *   d_index:  int64 [n_out]: output row i expands source row d_index[i] (duplicates and any order allowed); NULL: output
+ *             row i expands row i, and n_out must equal n_rows.  An index outside [0, n_rows) never faults: that output
+ *             row is all zeros, its reward 0 and its done flag 0.
+ *   player:   -1: d_obs float32 [n_out][2][obs_len]; 0 or 1: d_obs float32 [n_out][obs_len], that player's vector only.
+ *   d_reward (optional): float32 [n_out][2];  d_done (optional): uint8 [n_out].
+ * d_obs 16-byte aligned.  The constant entries (node flags, unit types) and player 1's node numbering come from the bound
+ * tables (needs evg_bind).  A row the step did not write expands to unspecified values, without a fault. */
+int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64_t* d_index, int64_t n_out, int32_t player, float* d_obs,
+                    float* d_reward, uint8_t* d_done, void* stream);
+
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
  * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).

@@ -16,7 +16,9 @@ turn (forward, sampling, decode, step) in a CUDA graph.  The observation tensor 
 step.  --fused runs the network in libevgsim's tcgen05 kernels instead of torch: DQN's forward in evg_policy_mlp (then
 evg_decode_dqn), PPO's forward, sampling and unravel in evg_policy_ppo, the recurrent actor's head, GRU steps, draws
 and unravel in evg_policy_rppo, which also carries the hidden state and zeroes it when a match starts over (their draws
-come from the simulator's tape, not from torch's generator).  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
+come from the simulator's tape, not from torch's generator).  --obs wire (with --fused) steps the simulator in the wire
+format and the fused kernel reads those rows (128 B per match instead of 840); --opponent puts a scripted agent
+(env.agent_actions) on player 1's side, the fused network plays player 0.  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
 """
 import argparse
 import json
@@ -81,7 +83,12 @@ def main():
     ap.add_argument("--graph", action="store_true", help="replay the turn (forward, decode, step) from a CUDA graph")
     ap.add_argument("--fused", action="store_true",
                     help="the policy runs in libevgsim's fused tcgen05 kernels (evg_policy_mlp / evg_policy_ppo / evg_policy_rppo, bf16 operands) instead of torch")
+    ap.add_argument("--obs", default="f32", choices=["f32", "wire"], help="observation format of the step and the fused policy's input")
+    ap.add_argument("--opponent", default="none", choices=["none", "random", "base_rush", "swarm"],
+                    help="with --fused: a scripted agent plays player 1, the network player 0")
     args = ap.parse_args()
+    if (args.obs == "wire" or args.opponent != "none") and not args.fused:
+        ap.error("--obs wire and --opponent need --fused")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -93,16 +100,25 @@ def main():
     first, _ = evgsim.shard_range(E * world, rank, world)
     env = evgsim.BatchedEvergladesEnv(E, device=local, seed=0, auto_reset=evgsim._capi.AUTORESET_TERMINAL, env_id_offset=first)
     net = build_policy(args.policy, dtype, env.device)
-    env.reset()
+    env.reset(obs_format=args.obs)
     hidden = torch.zeros((1, 2 * E, 128), dtype=dtype, device=env.device) if args.policy == "rppo" and not args.fused else None
 
     fused = None
     if args.fused:  # the recurrent actor's kernel keeps its own state (fused.hidden) and resets it at turn 0
         from evgsim import policy as evp
-        fused = {"dqn": evp.FusedDQN, "ppo": evp.FusedPPO, "rppo": evp.FusedRPPO}[args.policy](env, net.float())
+        cls = {"dqn": evp.FusedDQN, "ppo": evp.FusedPPO, "rppo": evp.FusedRPPO}[args.policy]
+        fused = cls(env, net.float()) if args.policy == "dqn" or args.opponent == "none" else cls(env, net.float(), player=0)
+    opponent = {"none": None, "random": evgsim._capi.AGENT_RANDOM, "base_rush": evgsim._capi.AGENT_BASE_RUSH,
+                "swarm": evgsim._capi.AGENT_SWARM}[args.opponent]
 
     def turn():
-        env.step(fused() if fused is not None else policy_actions(env, net, args.policy, dtype, hidden))
+        if fused is None:
+            env.step(policy_actions(env, net, args.policy, dtype, hidden))
+        else:
+            actions = fused(obs_format=args.obs)
+            if opponent is not None:  # player 1's rows from the scripted agent, player 0's from the network
+                env.agent_actions(evgsim._capi.AGENT_EXTERNAL, opponent)
+            env.step(actions, obs_format=args.obs)
         if hidden is not None:  # a finished match starts over with a fresh hidden state
             hidden.mul_((1 - env.done).to(dtype).repeat_interleave(2).view(1, -1, 1))
 
@@ -135,7 +151,7 @@ def main():
     stats = evgsim.gather_episode_stats(env.episode_stats(), device=env.device) if world > 1 else env.episode_stats()
     if rank == 0:
         sec = float(ms.item()) / 1e3
-        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % {"dqn": "evg_policy_mlp", "ppo": "evg_policy_ppo", "rppo": "evg_policy_rppo"}[args.policy] if args.fused else args.dtype, "fused_forward": bool(args.fused),
+        print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % {"dqn": "evg_policy_mlp", "ppo": "evg_policy_ppo", "rppo": "evg_policy_rppo"}[args.policy] if args.fused else args.dtype, "fused_forward": bool(args.fused), "obs_format": args.obs, "opponent": args.opponent,
                           "cuda_graph": bool(args.graph),
                           "n_gpus": world, "envs_per_gpu": E, "turns": args.turns, "env_turns_per_s": E * world * args.turns / sec,
                           "ms_per_turn": sec * 1e3 / args.turns, "episodes": stats["episodes"], "wins": stats["wins"], "ties": stats["ties"]}))
