@@ -954,9 +954,9 @@ int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_
     return evg_policy_mlp_fmt(sim, EVG_OBS_F32, d_obs, rows, d_w1_img, d_w2_img, hidden, out_dim, d_q, q_transposed, stream);
 }
 
-int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
-                       const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions,
-                       int64_t* d_idx, float* d_probs, void* stream)
+int evg_policy_ppo_logp(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                        const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions,
+                        int64_t* d_idx, float* d_probs, float* d_logp, void* stream)
 {
     int rc = check_sim(sim, true);  // the draws read turn and episode from the bound records
     if (rc) return rc;
@@ -968,24 +968,33 @@ int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t p
     if ((rc = policy_source("evg_policy_ppo", sim, format, d_obs, &ws, &wire))) return rc;
     if ((rc = check_actor_shape("evg_policy_ppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_w3_img}))) return rc;
     cudaError_t e = evg::launch_policy_ppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
-                                           d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx, d_probs, sim->sm_count, (cudaStream_t)stream,
-                                           wire ? &ws : nullptr);
+                                           d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx, d_probs, d_logp, sim->sm_count,
+                                           (cudaStream_t)stream, wire ? &ws : nullptr);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_ppo_kernel launch");
     sim->launches += 1;
     return EVG_OK;
+}
+
+int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                       const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions,
+                       int64_t* d_idx, float* d_probs, void* stream)
+{
+    return evg_policy_ppo_logp(sim, format, d_obs, player, d_w1_img, d_w2_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx,
+                               d_probs, nullptr, stream);
 }
 
 int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_w3_img,
                    const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod, int8_t* d_actions, int64_t* d_idx,
                    float* d_probs, void* stream)
 {
-    return evg_policy_ppo_fmt(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx,
-                              d_probs, stream);
+    return evg_policy_ppo_logp(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_actions, d_idx,
+                               d_probs, nullptr, stream);
 }
 
-int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
-                        const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim,
-                        int32_t div, int32_t mod, float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
+int evg_policy_rppo_logp(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                         const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent,
+                         int32_t out_dim, int32_t div, int32_t mod, float* d_hidden, float* d_hidden_in, int8_t* d_actions,
+                         int64_t* d_idx, float* d_probs, float* d_logp, void* stream)
 {
     int rc = check_sim(sim, true);  // the draws and the turn-0 reset of the state read the bound records
     if (rc) return rc;
@@ -994,24 +1003,37 @@ int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t 
     if (!d_hidden) return fail(EVG_E_ARG, "evg_policy_rppo: d_hidden (the GRU state, in and out) is null");
     if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_rppo: player %d outside -1..1", player);
     if (div < 1 || mod < 1) return fail(EVG_E_ARG, "evg_policy_rppo: div %d / mod %d must be positive", div, mod);
+    if (d_hidden_in && latent > 0) {  // the kernel reads d_hidden after it has written d_hidden_in
+        const uintptr_t bytes = (uintptr_t)(sim->n_envs * (player < 0 ? 2 : 1) * latent) * sizeof(float);
+        const uintptr_t h = (uintptr_t)d_hidden, hi = (uintptr_t)d_hidden_in;
+        if (hi < h + bytes && h < hi + bytes) return fail(EVG_E_ARG, "evg_policy_rppo: d_hidden_in overlaps d_hidden");
+    }
     evg::WireSrc ws;
     bool wire;
     if ((rc = policy_source("evg_policy_rppo", sim, format, d_obs, &ws, &wire))) return rc;
     if ((rc = check_actor_shape("evg_policy_rppo", sim, latent, out_dim, {d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img}))) return rc;
     cudaError_t e = evg::launch_policy_rppo(sim->tables, (const uint32_t*)sim->bound[EVG_BIND_RECORDS], d_obs, sim->n_envs, player, d_w1_img, d_w2_img,
-                                            d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_hidden, d_actions, d_idx, d_probs,
-                                            sim->sm_count, (cudaStream_t)stream, wire ? &ws : nullptr);
+                                            d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod, d_hidden, d_hidden_in, d_actions,
+                                            d_idx, d_probs, d_logp, sim->sm_count, (cudaStream_t)stream, wire ? &ws : nullptr);
     if (e != cudaSuccess) return cuda_fail(e, "evg_policy_rppo_kernel launch");
     sim->launches += 1;
     return EVG_OK;
+}
+
+int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                        const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim,
+                        int32_t div, int32_t mod, float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
+{
+    return evg_policy_rppo_logp(sim, format, d_obs, player, d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod,
+                                d_hidden, nullptr, d_actions, d_idx, d_probs, nullptr, stream);
 }
 
 int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img, const void* d_wi_img,
                     const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
                     float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream)
 {
-    return evg_policy_rppo_fmt(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div, mod,
-                               d_hidden, d_actions, d_idx, d_probs, stream);
+    return evg_policy_rppo_logp(sim, EVG_OBS_F32, d_obs, player, d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, latent, out_dim, div,
+                                mod, d_hidden, nullptr, d_actions, d_idx, d_probs, nullptr, stream);
 }
 
 int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64_t* d_index, int64_t n_out, int32_t player, float* d_obs,

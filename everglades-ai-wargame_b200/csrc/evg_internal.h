@@ -164,11 +164,12 @@ cudaError_t launch_policy_mlp(const void* obs, int64_t rows, int in_dim, const v
                               int transposed, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
 cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
-                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
+                              int8_t* actions, int64_t* idx, float* probs, float* logp, int sm_count, cudaStream_t stream,
+                              const WireSrc* wire = nullptr);
 cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
-                               int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
-                               cudaStream_t stream, const WireSrc* wire = nullptr);
+                               int out_dim, int div, int mod, float* hidden, float* hidden_in, int8_t* actions, int64_t* idx, float* probs,
+                               float* logp, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
 // wire rows -> float32 observations, reward and done (evg_wire_expand.cu); index / reward / done may be null
 cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n_rows, const int64_t* index, int64_t n_out, int player,
                                float* obs, float* reward, uint8_t* done, cudaStream_t stream);

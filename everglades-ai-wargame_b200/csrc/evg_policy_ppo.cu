@@ -59,7 +59,9 @@ constexpr int kTmemD1 = 0, kTmemD2 = 256;  // D3 reuses D1's columns (read out b
 
 // nk: chunks of 128 K-columns of layers 2 and 3
 // kWire: the observations are wire rows (ws), else float32
-template <bool kWire>
+// kLogp: a.logp may be written (the instantiation without it is the kernel as it was before d_logp existed: the extra
+//        registers of the draw loop slowed the wire call that does not ask for it)
+template <bool kWire, bool kLogp>
 __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __grid_constant__ ActorArgs a, const int nk, const __grid_constant__ WireSrc ws)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -209,6 +211,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
                 if (gp) gp[j] = q;
             }
             int64_t* ip = a.idx ? a.idx + i * EVG_MAX_ACTIONS : nullptr;
+            float* lq = kLogp && a.logp ? a.logp + i * EVG_MAX_ACTIONS : nullptr;
 #pragma unroll
             for (int k = 0; k < EVG_MAX_ACTIONS; ++k) {
                 const float x = draw_uniform(w[k >> 2][k & 3]) * total;
@@ -225,6 +228,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
                     c = cn;
                 }
                 if (sel < 0) { sel = last; t = c_last; }
+                if (lq) lq[k] = logf(pr[sel * kTileM] / total);  // total: this draw's T
                 pr[sel * kTileM] = -0.f;
                 total = t;
                 if (ip) ip[k] = sel;
@@ -246,17 +250,21 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_ppo_kernel(const __
 
 cudaError_t launch_policy_ppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                               const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
-                              int8_t* actions, int64_t* idx, float* probs, int sm_count, cudaStream_t stream, const WireSrc* wire)
+                              int8_t* actions, int64_t* idx, float* probs, float* logp, int sm_count, cudaStream_t stream, const WireSrc* wire)
 {
-    const ActorArgs a = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
-    return launch_persistent(wire ? evg_policy_ppo_kernel<true> : evg_policy_ppo_kernel<false>, a.rows, sm_count, kSmBytes, stream, a,
-                             (a.lp + 127) / 128, wire ? *wire : WireSrc{});
+    const ActorArgs a = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs, logp);
+    auto* kernel = wire ? (logp ? evg_policy_ppo_kernel<true, true> : evg_policy_ppo_kernel<true, false>)
+                        : (logp ? evg_policy_ppo_kernel<false, true> : evg_policy_ppo_kernel<false, false>);
+    return launch_persistent(kernel, a.rows, sm_count, kSmBytes, stream, a, (a.lp + 127) / 128, wire ? *wire : WireSrc{});
 }
 
 cudaError_t set_policy_ppo_smem()
 {
-    cudaError_t e = cudaFuncSetAttribute(evg_policy_ppo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
-    return e != cudaSuccess ? e : cudaFuncSetAttribute(evg_policy_ppo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    cudaError_t e = cudaSuccess;
+    for (auto* kernel : {evg_policy_ppo_kernel<false, false>, evg_policy_ppo_kernel<true, false>, evg_policy_ppo_kernel<false, true>,
+                         evg_policy_ppo_kernel<true, true>})
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    return e;
 }
 
 }  // namespace evg

@@ -70,13 +70,16 @@ struct RppoArgs : ActorArgs {
     const unsigned char* wi;
     const unsigned char* wh;
     float* hidden;
+    float* hidden_in;  // [rows][L]: the state each row started this call from (null: not written)
     int latent, ka, nrb;
 };
 
 __device__ __forceinline__ float sigmoid(float v) { return __frcp_rn(1.f + expf(-v)); }  // = 1 / (1 + e^-v), correctly rounded
 
 // kWire: the observations are wire rows (ws), else float32
-template <bool kWire>
+// kExtra: a.logp / a.hidden_in may be written (the instantiation without them is the kernel as it was before they
+//         existed: the draw loop's stores of T and p_j slowed the call that does not ask for them by 4-10 %)
+template <bool kWire, bool kExtra>
 __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const __grid_constant__ RppoArgs a, const __grid_constant__ WireSrc ws)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -231,14 +234,22 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
         live = r < nrows;
         hrow = a.hidden + my_row * latent;
         const bool fresh = !live || a.records[my_env * a.rec_words + kRecTurn] == 0;
+        float* hin = (kExtra && a.hidden_in && live) ? a.hidden_in + my_row * latent : nullptr;  // h0 of my row, written before it is overwritten
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
             for (int e = 0; e < 16; ++e) {
                 const int j = 16 * (quarter + 4 * i) + e;
-                if (i < 2) hs[i][e] = (!fresh && j < latent) ? hrow[j] : 0.f;
-                else if (fresh && live && j < latent) hrow[j] = 0.f;
+                if (i < 2) {
+                    hs[i][e] = (!fresh && j < latent) ? hrow[j] : 0.f;
+                    if (hin && j < latent) hin[j] = hs[i][e];
+                } else if (fresh && live && j < latent) {
+                    hrow[j] = 0.f;
+                }
             }
+        if (hin)  // units 128.. (L > 128), zeroed above for a fresh row: groups 16 (quarter + 8) and 16 (quarter + 12)
+#pragma unroll 1
+            for (int j = 16 * (quarter + 8); j < latent; j += j % 16 == 15 ? 49 : 1) hin[j] = hrow[j];
         tc_fence_before();
         __syncthreads();
         // ---- the action head
@@ -379,6 +390,9 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
                 draw_block(a, me, turn, episode, k >> 2, w);
                 const uint32_t wk = (k & 3) == 0 ? w[0] : (k & 3) == 1 ? w[1] : (k & 3) == 2 ? w[2] : w[3];
                 const float x = draw_uniform(wk) * total;
+                // T and p of the drawn j wait for the log-probability in red[r] and red[kTileM + r] (free until the next
+                // step's partial sums), not in registers: this loop runs at the kernel's register bound
+                if (kExtra) red[r] = total;
                 float c = 0.f;
                 int sel = -1;
 #pragma unroll 1
@@ -391,6 +405,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
                         const int j = 16 * gi + e;
                         if (j < a.out_dim) {
                             c += __uint_as_float(v[e]);
+                            if (kExtra && sel < 0 && (x < c || j == a.out_dim - 1)) red[kTileM + r] = __uint_as_float(v[e]);
                             if (sel < 0 && x < c) sel = j;
                         }
                     }
@@ -398,6 +413,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
                 }
                 if (sel < 0) sel = a.out_dim - 1;
                 if (live) {
+                    if (kExtra && a.logp) a.logp[my_row * EVG_MAX_ACTIONS + k] = logf(red[kTileM + r] / red[r]);
                     if (a.idx) a.idx[my_row * EVG_MAX_ACTIONS + k] = sel;
                     store_action(a, me, k, sel);
                 }
@@ -423,25 +439,32 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
 
 cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
-                               int out_dim, int div, int mod, float* hidden, int8_t* actions, int64_t* idx, float* probs, int sm_count,
-                               cudaStream_t stream, const WireSrc* wire)
+                               int out_dim, int div, int mod, float* hidden, float* hidden_in, int8_t* actions, int64_t* idx, float* probs,
+                               float* logp, int sm_count, cudaStream_t stream, const WireSrc* wire)
 {
     RppoArgs a;
-    static_cast<ActorArgs&>(a) = actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs);
+    static_cast<ActorArgs&>(a) =
+        actor_args(t, records, obs, n_envs, player, w1_img, w2_img, w3_img, bias, latent, out_dim, div, mod, actions, idx, probs, logp);
     a.wi = reinterpret_cast<const unsigned char*>(wi_img);
     a.wh = reinterpret_cast<const unsigned char*>(wh_img);
     a.hidden = hidden;
+    a.hidden_in = hidden_in;
     a.latent = latent;
     a.ka = (latent + kAtomK - 1) / kAtomK;
     a.nrb = (a.lp + kPieceRows - 1) / kPieceRows;
-    return launch_persistent(wire ? evg_policy_rppo_kernel<true> : evg_policy_rppo_kernel<false>, a.rows, sm_count, kSmBytes, stream, a,
-                             wire ? *wire : WireSrc{});
+    const bool extra = logp || hidden_in;
+    auto* kernel = wire ? (extra ? evg_policy_rppo_kernel<true, true> : evg_policy_rppo_kernel<true, false>)
+                        : (extra ? evg_policy_rppo_kernel<false, true> : evg_policy_rppo_kernel<false, false>);
+    return launch_persistent(kernel, a.rows, sm_count, kSmBytes, stream, a, wire ? *wire : WireSrc{});
 }
 
 cudaError_t set_policy_rppo_smem()
 {
-    cudaError_t e = cudaFuncSetAttribute(evg_policy_rppo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
-    return e != cudaSuccess ? e : cudaFuncSetAttribute(evg_policy_rppo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    cudaError_t e = cudaSuccess;
+    for (auto* kernel : {evg_policy_rppo_kernel<false, false>, evg_policy_rppo_kernel<true, false>, evg_policy_rppo_kernel<false, true>,
+                         evg_policy_rppo_kernel<true, true>})
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmBytes);
+    return e;
 }
 
 }  // namespace evg

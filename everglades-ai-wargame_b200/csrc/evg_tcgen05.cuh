@@ -37,6 +37,7 @@ struct ActorArgs {
     int8_t* actions;
     int64_t* idx;
     float* probs;
+    float* logp;   // [rows][7]: log(p_j / T) of each draw (null: not written)
     int64_t rows;  // n_envs * (player < 0 ? 2 : 1)
     int player, in_dim, lp, out_dim, div, mod, rec_words;
     uint32_t env_base, seed_lo, seed_hi;
@@ -44,7 +45,7 @@ struct ActorArgs {
 
 inline ActorArgs actor_args(const Tables& t, const uint32_t* records, const void* obs, int64_t n_envs, int player, const void* w1_img,
                             const void* w2_img, const void* w3_img, const float* bias, int latent, int out_dim, int div, int mod,
-                            int8_t* actions, int64_t* idx, float* probs)
+                            int8_t* actions, int64_t* idx, float* probs, float* logp)
 {
     ActorArgs a;
     a.obs = obs;
@@ -56,6 +57,7 @@ inline ActorArgs actor_args(const Tables& t, const uint32_t* records, const void
     a.actions = actions;
     a.idx = idx;
     a.probs = probs;
+    a.logp = logp;
     a.rows = n_envs * (player < 0 ? 2 : 1);
     a.player = player;
     a.in_dim = t.obs_len;

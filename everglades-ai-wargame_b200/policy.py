@@ -143,6 +143,11 @@ def _wire_rows(env, obs, obs_format):
     return _capi.OBS_WIRE, obs
 
 
+def _ptr(t, wanted):
+    """An optional output of a fused actor: the tensor's address when it is asked for, else NULL (not written)."""
+    return C.c_void_p(t.data_ptr()) if wanted else None
+
+
 class FusedDQN:
     """Q-network forward + decode for a BatchedEvergladesEnv: ``actions = FusedDQN(env, net)()`` reads env.obs in place."""
 
@@ -267,6 +272,7 @@ class FusedPPO:
         shape = (env.num_envs, 2) if self.player < 0 else (env.num_envs,)
         self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
         self.probs = torch.empty(shape + (self.out_dim,), dtype=torch.float32, device=dev)
+        self.logp = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.float32, device=dev)
 
     @staticmethod
     def _params(net):
@@ -281,18 +287,21 @@ class FusedPPO:
         w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
         _capi.check(env._lib.evg_pack_ppo(env._h, *src, L, o, w1, w2, w3, bias, env._stream()))
 
-    def __call__(self, want_probs=False, obs_format="f32"):
+    def __call__(self, want_probs=False, obs_format="f32", want_logp=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); fills .idx (int64 [N, 2, 7] or [N, 7]) and, with want_probs,
-        .probs (float32 [N, 2, out] or [N, out]).  obs_format 'wire' reads env.obs_rows('wire') (the env stepped with
-        obs_format='wire'), with results bit for bit those of the float32 observations."""
+        .probs (float32 [N, 2, out] or [N, out]).  With want_logp, .logp (float32 [N, 2, 7] or [N, 7]): draw k's
+        log-probability log(p_j / T_k), T_k the sampler's float32 sum of the probabilities not drawn before it, so that
+        .logp.sum(-1) is the log-probability of the ordered 7 draws without replacement (the behaviour policy's term of
+        a PPO ratio).  No other output depends on want_probs / want_logp.  obs_format 'wire' reads env.obs_rows('wire')
+        (the env stepped with obs_format='wire'), with results bit for bit those of the float32 observations."""
         env = self.env
         fmt, obs = _wire_rows(env, None, obs_format)
         obs = env.obs if obs is None else obs
         w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
-        _capi.check(env._lib.evg_policy_ppo_fmt(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, w3, bias, self.latent,
-                                                self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
-                                                C.c_void_p(self.idx.data_ptr()), C.c_void_p(self.probs.data_ptr()) if want_probs else None,
-                                                env._stream()))
+        _capi.check(env._lib.evg_policy_ppo_logp(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, w3, bias, self.latent,
+                                                 self.out_dim, self.div, self.mod, C.c_void_p(env._actions.data_ptr()),
+                                                 C.c_void_p(self.idx.data_ptr()), _ptr(self.probs, want_probs), _ptr(self.logp, want_logp),
+                                                 env._stream()))
         return env._actions
 
 
@@ -401,6 +410,8 @@ class FusedRPPO:
         self.hidden = torch.zeros(shape + (self.latent,), dtype=torch.float32, device=dev)
         self.idx = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.int64, device=dev)
         self.probs = torch.empty(shape + (_capi.MAX_ACTIONS, self.out_dim), dtype=torch.float32, device=dev)
+        self.logp = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.float32, device=dev)
+        self.hidden_in = torch.zeros_like(self.hidden)
 
     def refresh(self, actor=None):
         """Re-pack the weight images and the bias vector in place from `actor` (default: the module this wrapper was built
@@ -414,16 +425,20 @@ class FusedRPPO:
         _capi.check(env._lib.evg_pack_rppo(env._h, w1, b1, w2, b2, w3, b3, wi, bi, wh, bh, L, o, i1, i2, ii, ih, i3, bias,
                                            env._stream()))
 
-    def __call__(self, want_probs=False, obs_format="f32"):
+    def __call__(self, want_probs=False, obs_format="f32", want_logp=False, want_hidden_in=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); steps .hidden, fills .idx (int64 [N, 2, 7] or [N, 7]) and, with
-        want_probs, .probs (float32 [N, 2, 7, out] or [N, 7, out]: step k's distribution).  obs_format 'wire' reads
-        env.obs_rows('wire'), as FusedPPO does."""
+        want_probs, .probs (float32 [N, 2, 7, out] or [N, 7, out]: step k's distribution).  With want_logp, .logp
+        (float32 [N, 2, 7] or [N, 7]): step k's log(p_k[j] / T_k), T_k the sampler's float32 sum of p_k.  With
+        want_hidden_in, .hidden_in (.hidden's shape): the state each row started this call from (zero for a row whose
+        match is at turn 0), which is what a PPO update re-evaluates the stored turn from.  No other output depends on
+        want_probs / want_logp / want_hidden_in.  obs_format 'wire' reads env.obs_rows('wire'), as FusedPPO does."""
         env = self.env
         fmt, obs = _wire_rows(env, None, obs_format)
         obs = env.obs if obs is None else obs
         w1, w2, wi, wh, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
-        _capi.check(env._lib.evg_policy_rppo_fmt(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, wi, wh, w3, bias, self.latent,
-                                                 self.out_dim, self.div, self.mod, C.c_void_p(self.hidden.data_ptr()),
-                                                 C.c_void_p(env._actions.data_ptr()), C.c_void_p(self.idx.data_ptr()),
-                                                 C.c_void_p(self.probs.data_ptr()) if want_probs else None, env._stream()))
+        _capi.check(env._lib.evg_policy_rppo_logp(env._h, fmt, C.c_void_p(obs.data_ptr()), self.player, w1, w2, wi, wh, w3, bias, self.latent,
+                                                  self.out_dim, self.div, self.mod, C.c_void_p(self.hidden.data_ptr()),
+                                                  _ptr(self.hidden_in, want_hidden_in), C.c_void_p(env._actions.data_ptr()),
+                                                  C.c_void_p(self.idx.data_ptr()), _ptr(self.probs, want_probs), _ptr(self.logp, want_logp),
+                                                  env._stream()))
         return env._actions

@@ -326,6 +326,7 @@ int evg_policy_mlp(EvgSim* sim, const float* d_obs, int64_t rows, const void* d_
  * current state, player) — independent of batch size, sharding and call order.
  *   d_idx (optional):   int64 [n_envs][2][7] (player -1) or [n_envs][7], the drawn indices in draw order.
  *   d_probs (optional): float32 [n_envs][2][out_dim] or [n_envs][out_dim], the probabilities the draws were made from.
+ *   (evg_policy_ppo_logp adds d_logp, each draw's log-probability; below.)
  * Weights are IMAGES in the kernel's shared-memory operand layout (bf16, K-major, 128-byte swizzle, zero padded, 16-byte
  * aligned).  With Lp = latent rounded up to 16 and Ka = latent rounded up to 64:
  *     d_w1_img: W1[n][k] as an [Lp x EVG_PPO_IN_PAD] block,  (EVG_PPO_IN_PAD / 64) * Lp * 128 bytes
@@ -359,6 +360,7 @@ int evg_policy_ppo(EvgSim* sim, const float* d_obs, int32_t player, const void* 
  * the first j whose ascending fp32 prefix sum of probs_k exceeds u_k times their ascending sum (none: the last j).
  *   d_idx (optional):   int64 [rows][7], the drawn indices.
  *   d_probs (optional): float32 [rows][7][out_dim], the distributions the draws were made from.
+ *   (evg_policy_rppo_logp adds d_logp, each draw's log-probability, and d_hidden_in, the starting state; below.)
  * Images as for evg_policy_ppo (Lp = latent rounded up to 16, Ka = latent rounded up to 64): d_w1_img, d_w2_img,
  * d_w3_img exactly as there, and
  *     d_wi_img: weight_ih_l0 as three [Lp x Ka] blocks, gate g (r, z, n) at g * (Ka / 64) * Lp * 128 bytes
@@ -386,6 +388,28 @@ int evg_policy_ppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t p
 int evg_policy_rppo_fmt(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
                         const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim,
                         int32_t div, int32_t mod, float* d_hidden, int8_t* d_actions, int64_t* d_idx, float* d_probs, void* stream);
+
+/* The two actors of evg_policy_ppo_fmt / evg_policy_rppo_fmt (which are these calls with the new pointers NULL) with what
+ * a PPO update needs of the behaviour policy, written by the same launch.  Every other output is bit for bit the same
+ * whether these are asked for or not.
+ *   d_logp (optional): float32 [rows][7] like d_idx ([n_envs][2][7] for player -1, [n_envs][7] for one player): the
+ *       log-probability of each draw, logf(p_j / T_k) in fp32 (accurate logf), in [-7, 0] (every probability is at least
+ *       1 / (1 + 143 e^2)).  j is the drawn index, p_j its fp32 probability (the value d_probs holds).
+ *       evg_policy_ppo_logp: T_k is the sampler's own fp32 sum, in ascending j, of the probabilities not chosen before
+ *       draw k (T_0 sums all of them) — the normaliser the draw used, also when no j was found through rounding and the
+ *       largest not-chosen j was taken.  Summed over k: the log-probability of the ordered 7-tuple under sequential
+ *       sampling without replacement.
+ *       evg_policy_rppo_logp: T_k is the fp32 ascending sum of probs_k; on the path where no j is found, j = out_dim - 1.
+ *   d_hidden_in (evg_policy_rppo_logp, optional): float32 [rows][latent] like d_hidden: the state each row's GRU started
+ *       from in this call, +0.0 for a row whose match record is at turn 0, otherwise what d_hidden held.  It must not
+ *       overlap d_hidden (EVG_E_ARG). */
+int evg_policy_ppo_logp(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                        const void* d_w3_img, const float* d_bias, int32_t latent, int32_t out_dim, int32_t div, int32_t mod,
+                        int8_t* d_actions, int64_t* d_idx, float* d_probs, float* d_logp, void* stream);
+int evg_policy_rppo_logp(EvgSim* sim, int32_t format, const void* d_obs, int32_t player, const void* d_w1_img, const void* d_w2_img,
+                         const void* d_wi_img, const void* d_wh_img, const void* d_w3_img, const float* d_bias, int32_t latent,
+                         int32_t out_dim, int32_t div, int32_t mod, float* d_hidden, float* d_hidden_in, int8_t* d_actions,
+                         int64_t* d_idx, float* d_probs, float* d_logp, void* stream);
 
 /* Wire rows -> the float32 observation vector on the device (csrc/evg_wire_expand.cu), bit for bit what the step writes
  * in EVG_OBS_F32 and what evgsim.wire.expand computes on the host; for training consumers that store the rows (a replay or

@@ -86,9 +86,14 @@ def main():
     ap.add_argument("--obs", default="f32", choices=["f32", "wire"], help="observation format of the step and the fused policy's input")
     ap.add_argument("--opponent", default="none", choices=["none", "random", "base_rush", "swarm"],
                     help="with --fused: a scripted agent plays player 1, the network player 0")
+    ap.add_argument("--want", default="none", choices=["none", "logp", "probs"],
+                    help="with --fused --policy ppo|rppo: what a PPO rollout keeps of each turn besides the draws: nothing, each "
+                         "draw's log-probability (and for rppo the starting state, hidden_in), or the whole distribution")
     args = ap.parse_args()
     if (args.obs == "wire" or args.opponent != "none") and not args.fused:
         ap.error("--obs wire and --opponent need --fused")
+    if args.want != "none" and not (args.fused and args.policy in ("ppo", "rppo")):
+        ap.error("--want needs --fused and --policy ppo or rppo")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -111,11 +116,14 @@ def main():
     opponent = {"none": None, "random": evgsim._capi.AGENT_RANDOM, "base_rush": evgsim._capi.AGENT_BASE_RUSH,
                 "swarm": evgsim._capi.AGENT_SWARM}[args.opponent]
 
+    want = {"none": {}, "probs": {"want_probs": True},
+            "logp": {"want_logp": True, **({"want_hidden_in": True} if args.policy == "rppo" else {})}}[args.want]
+
     def turn():
         if fused is None:
             env.step(policy_actions(env, net, args.policy, dtype, hidden))
         else:
-            actions = fused(obs_format=args.obs)
+            actions = fused(obs_format=args.obs, **want)
             if opponent is not None:  # player 1's rows from the scripted agent, player 0's from the network
                 env.agent_actions(evgsim._capi.AGENT_EXTERNAL, opponent)
             env.step(actions, obs_format=args.obs)
@@ -152,7 +160,7 @@ def main():
     if rank == 0:
         sec = float(ms.item()) / 1e3
         print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % {"dqn": "evg_policy_mlp", "ppo": "evg_policy_ppo", "rppo": "evg_policy_rppo"}[args.policy] if args.fused else args.dtype, "fused_forward": bool(args.fused), "obs_format": args.obs, "opponent": args.opponent,
-                          "cuda_graph": bool(args.graph),
+                          "cuda_graph": bool(args.graph), "want": args.want,
                           "n_gpus": world, "envs_per_gpu": E, "turns": args.turns, "env_turns_per_s": E * world * args.turns / sec,
                           "ms_per_turn": sec * 1e3 / args.turns, "episodes": stats["episodes"], "wins": stats["wins"], "ties": stats["ties"]}))
     if world > 1:

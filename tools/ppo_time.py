@@ -62,7 +62,8 @@ def main():
         return env.decode_indices(i.view(n, 2, 7), div=12, mod=11)
 
     print(json.dumps({"gpu": gpu_info(), "rows": 2 * n, "latent": latent,
-                      "fused_ppo_us": timed_us(fused), "fused_ppo_with_probs_us": timed_us(lambda: fused(want_probs=True)),
+                      "fused_ppo_us": timed_us(fused), "fused_ppo_with_logp_us": timed_us(lambda: fused(want_logp=True)),
+                      "fused_ppo_with_probs_us": timed_us(lambda: fused(want_probs=True)),
                       "torch_bf16_forward_us": timed_us(lambda: nb(x.to(torch.bfloat16))),
                       "torch_multinomial_us": timed_us(lambda: torch.multinomial(probs, 7, replacement=False)),
                       "decode_indices_us": timed_us(lambda: env.decode_indices(idx.view(n, 2, 7), div=12, mod=11)),

@@ -61,7 +61,9 @@ def main():
     stream = weight_bytes_per_tile(latent) * tiles
     with torch.no_grad():
         print(json.dumps({"gpu": gpu_info(), "rows": 2 * n, "latent": latent,
-                          "fused_rppo_us": fused_us, "fused_rppo_with_probs_us": timed_us(lambda: fused(want_probs=True)),
+                          "fused_rppo_us": fused_us, "fused_rppo_with_logp_us": timed_us(lambda: fused(want_logp=True)),
+                          "fused_rppo_with_logp_and_hidden_in_us": timed_us(lambda: fused(want_logp=True, want_hidden_in=True)),
+                          "fused_rppo_with_probs_us": timed_us(lambda: fused(want_probs=True)),
                           "weight_stream_bytes": stream, "weight_stream_gb_per_s": stream / fused_us / 1e3,
                           "torch_bf16_head_us": timed_us(lambda: nb.action_head(x.to(torch.bfloat16))),
                           "torch_bf16_gru_us": timed_us(lambda: nb.action_gru(seq, hidden)),
