@@ -26,6 +26,7 @@ OBS_F32, OBS_I16, OBS_WIRE = 0, 1, 2
 WIRE_NODE0 = 4
 MLP_IN_PAD, MLP_CHUNK, MLP_OUT_PAD = 128, 192, 144
 PPO_IN_PAD, PPO_MAX_LATENT, PPO_OUT_PAD = 128, 256, 144
+VALUE_OUT_PAD = 16
 BIND_RECORDS, BIND_HEALTH, BIND_STATS, BIND_TABLES, BIND_AGENTS, BIND_COUNT = 0, 1, 2, 3, 4, 5
 
 _N1 = MAX_NODES + 1
@@ -177,10 +178,12 @@ SYMBOLS = [
     ("evg_policy_ppo_logp", C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_policy_rppo_logp", C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                        _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_policy_value", C.c_int, [_P, C.c_int32, _P, C.c_int64, C.c_int32, _P, _P, _P, _P, C.c_int32, _P, _P]),
     ("evg_wire_expand", C.c_int, [_P, _P, C.c_int64, _P, C.c_int64, C.c_int32, _P, _P, _P, _P]),
     ("evg_pack_mlp", C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     ("evg_pack_ppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_pack_rppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_pack_value", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_decode_dqn_layout",C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     ("evg_shape_reward", C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_step_kernel_kind", C.c_int, [_P]),

@@ -366,7 +366,7 @@ int evg_create(const EvgConfig* cfg, int64_t n_envs, uint64_t seed, int64_t env_
     s->sm_count = prop.multiProcessorCount;
     // the shared-memory opt-ins are per device: made on the simulator's, for the step and the policy kernels
     if ((e = evg::set_step_smem(s->smem)) != cudaSuccess || (e = evg::set_policy_mlp_smem()) != cudaSuccess || (e = evg::set_policy_ppo_smem()) != cudaSuccess ||
-        (e = evg::set_policy_rppo_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
+        (e = evg::set_policy_rppo_smem()) != cudaSuccess || (e = evg::set_policy_value_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
     int per_sm = 0;
     if ((e = evg::step_occupancy(t, s->smem, &per_sm)) != cudaSuccess || per_sm < 1) { delete s; return cuda_fail(e, "occupancy query"); }
     // persistent CTAs: a whole number of resident waves, never more CTAs than matches need
@@ -1036,6 +1036,37 @@ int evg_policy_rppo(EvgSim* sim, const float* d_obs, int32_t player, const void*
                                 mod, d_hidden, nullptr, d_actions, d_idx, d_probs, nullptr, stream);
 }
 
+// the critic's checks (evg_policy_value, evg_pack_value); `aligned`: what the call reads or writes in 16 B
+static int check_value_shape(const char* fn, const EvgSim* sim, int32_t latent, std::initializer_list<const void*> aligned)
+{
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
+    for (const void* p : aligned)
+        if ((uintptr_t)p % 16) return fail(EVG_E_ARG, "%s: weight images and the packed bias vector must be 16-byte aligned", fn);
+    if (sim->layout.obs_len >= EVG_PPO_IN_PAD) return fail(EVG_E_ARG, "%s: observations of %d values exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    return EVG_OK;
+}
+
+int evg_policy_value(EvgSim* sim, int32_t format, const void* d_obs, int64_t n_matches, int32_t player, const void* d_w1_img,
+                     const void* d_w2_img, const void* d_w3_img, const float* d_bias, int32_t latent, float* d_value, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (!d_obs || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias || !d_value) return fail(EVG_E_ARG, "evg_policy_value: null argument");
+    if (n_matches < 0) return fail(EVG_E_ARG, "evg_policy_value: negative match count %lld", (long long)n_matches);
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_policy_value: player %d outside -1..1", player);
+    if ((uintptr_t)d_obs % 4 || (uintptr_t)d_value % 4) return fail(EVG_E_ARG, "evg_policy_value: observations and values must be 4-byte aligned");
+    evg::WireSrc ws;
+    bool wire;
+    if ((rc = policy_source("evg_policy_value", sim, format, d_obs, &ws, &wire))) return rc;
+    if ((rc = check_value_shape("evg_policy_value", sim, latent, {d_w1_img, d_w2_img, d_w3_img, d_bias}))) return rc;
+    if (n_matches == 0) return EVG_OK;
+    cudaError_t e = evg::launch_policy_value(d_obs, n_matches, player, sim->layout.obs_len, d_w1_img, d_w2_img, d_w3_img, d_bias, latent, d_value,
+                                             sim->sm_count, (cudaStream_t)stream, wire ? &ws : nullptr);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_value_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
 int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64_t* d_index, int64_t n_out, int32_t player, float* d_obs,
                     float* d_reward, uint8_t* d_done, void* stream)
 {
@@ -1081,6 +1112,21 @@ int evg_pack_rppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float
     if (!d_w_ih || !d_b_ih || !d_w_hh || !d_b_hh || !d_wi_img || !d_wh_img) return fail(EVG_E_ARG, "evg_pack_rppo: null argument");
     return pack_ppo_family("evg_pack_rppo", sim, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim,
                            d_w1_img, d_w2_img, d_wi_img, d_wh_img, d_w3_img, d_bias, stream);
+}
+
+int evg_pack_value(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                   const float* d_b3, int32_t latent, void* d_w1_img, void* d_w2_img, void* d_w3_img, float* d_bias, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (!d_w1 || !d_b1 || !d_w2 || !d_b2 || !d_w3 || !d_b3 || !d_w1_img || !d_w2_img || !d_w3_img || !d_bias)
+        return fail(EVG_E_ARG, "evg_pack_value: null argument");
+    if ((rc = check_value_shape("evg_pack_value", sim, latent, {d_w1_img, d_w2_img, d_w3_img, d_bias}))) return rc;
+    cudaError_t e = evg::launch_pack_value(sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, latent, d_w1_img, d_w2_img, d_w3_img, d_bias,
+                                           (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
 }
 
 int evg_shape_reward(EvgSim* sim, int32_t mode, const float* d_reward, const uint8_t* d_done, const float* d_obs, float* d_out,

@@ -170,6 +170,9 @@ cudaError_t launch_policy_rppo(const Tables& t, const uint32_t* records, const v
                                const void* w2_img, const void* wi_img, const void* wh_img, const void* w3_img, const float* bias, int latent,
                                int out_dim, int div, int mod, float* hidden, float* hidden_in, int8_t* actions, int64_t* idx, float* probs,
                                float* logp, int sm_count, cudaStream_t stream, const WireSrc* wire = nullptr);
+cudaError_t launch_policy_value(const void* obs, int64_t n_matches, int player, int in_dim, const void* w1_img, const void* w2_img,
+                                const void* w3_img, const float* bias, int latent, float* value, int sm_count, cudaStream_t stream,
+                                const WireSrc* wire = nullptr);
 // wire rows -> float32 observations, reward and done (evg_wire_expand.cu); index / reward / done may be null
 cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n_rows, const int64_t* index, int64_t n_out, int player,
                                float* obs, float* reward, uint8_t* done, cudaStream_t stream);
@@ -177,14 +180,17 @@ cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();
 cudaError_t set_policy_rppo_smem();
-// weight images of the three policy kernels from the float32 parameters (evg_policy_pack.cu); launch_pack_ppo packs the
-// recurrent actor's GRU as well when w_ih is not null
+cudaError_t set_policy_value_smem();
+// weight images of the policy kernels and the critic from the float32 parameters (evg_policy_pack.cu); launch_pack_ppo
+// packs the recurrent actor's GRU as well when w_ih is not null
 cudaError_t launch_pack_mlp(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, int hidden, int out_dim,
                             void* w1_img, void* w2_img, cudaStream_t stream);
 cudaError_t launch_pack_ppo(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
                             const float* b3, const float* w_ih, const float* b_ih, const float* w_hh, const float* b_hh, int latent,
                             int out_dim, void* w1_img, void* w2_img, void* wi_img, void* wh_img, void* w3_img, float* bias,
                             cudaStream_t stream);
+cudaError_t launch_pack_value(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
+                              const float* b3, int latent, void* w1_img, void* w2_img, void* w3_img, float* bias, cudaStream_t stream);
 cudaError_t launch_obs_to_i16(const float* obs, int16_t* out, int64_t n_values, cudaStream_t stream);
 cudaError_t launch_export(const Tables& t, const uint32_t* records, const double* health, int64_t first, int64_t count,
                           EvgEnvState* out, cudaStream_t stream);

@@ -1,9 +1,9 @@
 // evg_policy_pack.cu — the fused policies' weight images packed on the device, sm_100a.
 //
-// evg_policy_mlp / _ppo / _rppo read their weights as bf16 IMAGES of the shared-memory operand layout (K-major, 128-byte
-// swizzle; include/evgsim.h).  evgsim.policy.pack_mlp / pack_ppo / pack_rppo build them in numpy on the host; this kernel
-// writes the same bytes from the torch parameters where they sit (float32, contiguous, nn.Linear / nn.GRU layout), in
-// ONE launch, with no host synchronisation and no allocation, so that a training loop can refresh the images in place
+// evg_policy_mlp / _ppo / _rppo / _value read their weights as bf16 IMAGES of the shared-memory operand layout (K-major,
+// 128-byte swizzle; include/evgsim.h).  evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build them in numpy on
+// the host; this kernel writes the same bytes from the torch parameters where they sit (float32, contiguous, nn.Linear /
+// nn.GRU layout), in ONE launch, with no host synchronisation and no allocation, so that a training loop can refresh the images in place
 // after every optimiser step (and capture that in a CUDA graph).
 //
 //   One thread per 16-byte destination chunk: 8 bf16 of one image row, or 4 fp32 of a bias vector.  The chunks are
@@ -182,6 +182,21 @@ cudaError_t launch_pack_ppo(int in_dim, const float* w1, const float* b1, const 
         a.b[9] = gates(vec(gb + 3 * L, b_hh, L, 3 * latent), latent);
         a.n_blocks = 10;
     }
+    return launch(a, stream);
+}
+
+cudaError_t launch_pack_value(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
+                              const float* b3, int latent, void* w1_img, void* w2_img, void* w3_img, float* bias, cudaStream_t stream)
+{
+    const int lp = (latent + 15) / 16 * 16, ka = (latent + 63) / 64 * 64, L = EVG_PPO_MAX_LATENT;
+    PackArgs a{};
+    a.b[0] = image(w1_img, w1, lp, EVG_PPO_IN_PAD, latent, in_dim);
+    a.b[1] = image(w2_img, w2, lp, ka, latent, latent);
+    a.b[2] = image(w3_img, w3, EVG_VALUE_OUT_PAD, ka, 1, latent);
+    a.b[3] = vec(bias, b1, L, latent);
+    a.b[4] = vec(bias + L, b2, L, latent);
+    a.b[5] = vec(bias + 2 * L, b3, EVG_VALUE_OUT_PAD, 1);
+    a.n_blocks = 6;
     return launch(a, stream);
 }
 

@@ -10,10 +10,13 @@ TMEM, bf16 operands, fp32 accumulation) on the observation tensor the step kerne
   times on the head's output, Linear(L, 132) - Tanh - Softmax after every step, one draw per step): evg_policy_rppo, which
   carries the GRU state across turns and zeroes it when a match starts over.  ``pack_rppo`` builds its images,
   ``FusedRPPO`` wraps a module with the reference ActorCritic's ``action_head``, ``action_gru`` and ``action_layer``.
+- PPO's critic (agents/PPO/ActorCritic.py, value_layer — Linear(105, L) - Tanh - Linear(L, L) - Tanh - Linear(L, 1)):
+  evg_policy_value, the state values of the env's observations or of any number of stored rows.  ``pack_value`` builds
+  its images, ``FusedValue`` wraps the torch ``Sequential``.
 
 The images are what the kernels copy straight into shared memory (bf16, K-major, 128-byte swizzle; layout in
 include/evgsim.h).  The constructors pack them on the host; each wrapper's ``refresh()`` re-packs them in place on the
-device (evg_pack_mlp / _ppo / _rppo) after an optimiser step.  Plumbing only; the networks themselves are the caller's.
+device (evg_pack_mlp / _ppo / _rppo / _value) after an optimiser step.  Plumbing only; the networks themselves are the caller's.
 """
 from __future__ import annotations
 
@@ -25,6 +28,7 @@ from . import _capi
 
 IN_PAD, CHUNK, OUT_PAD, ATOM = _capi.MLP_IN_PAD, _capi.MLP_CHUNK, _capi.MLP_OUT_PAD, 64
 PPO_IN_PAD, PPO_MAX_LATENT, PPO_OUT_PAD = _capi.PPO_IN_PAD, _capi.PPO_MAX_LATENT, _capi.PPO_OUT_PAD
+VALUE_OUT_PAD = _capi.VALUE_OUT_PAD
 
 
 def to_bf16_bits(x):
@@ -250,6 +254,35 @@ def reference_forward_ppo(obs, w1, b1, w2, b2, w3, b3):
     return (e / e.sum(axis=-1, dtype=f32, keepdims=True)).astype(f32)
 
 
+def pack_value(w1, b1, w2, b2, w3, b3):
+    """The critic's weights w1 [L, in], b1 [L], w2 [L, L], b2 [L], w3 [1, L], b3 [1] (float32, torch.nn.Linear's layout)
+    -> (w1_img, w2_img, w3_img uint8, bias float32, latent) as evg_policy_value expects them: W1 and W2 exactly as
+    pack_ppo packs them, w3 as row 0 of a zero [16 x Ka] block, b1 | b2 | b3 at 0, 256 and 512 of one zero-padded
+    float32 vector of 528."""
+    w1, b1, w2, b2, w3, b3 = (np.asarray(a, dtype=np.float32) for a in (w1, b1, w2, b2, w3, b3))
+    latent, in_dim = w1.shape
+    assert in_dim < PPO_IN_PAD and 1 <= latent <= PPO_MAX_LATENT
+    assert w2.shape == (latent, latent) and w3.shape == (1, latent) and b1.shape == b2.shape == (latent,) and b3.shape == (1,)
+    lp, ka = -(-latent // 16) * 16, -(-latent // ATOM) * ATOM
+    bias = np.zeros(2 * PPO_MAX_LATENT + VALUE_OUT_PAD, dtype=np.float32)
+    bias[:latent] = b1
+    bias[PPO_MAX_LATENT:PPO_MAX_LATENT + latent] = b2
+    bias[2 * PPO_MAX_LATENT] = b3[0]
+    return _image(w1, lp, PPO_IN_PAD), _image(w2, lp, ka), _image(w3, VALUE_OUT_PAD, ka), bias, latent
+
+
+def reference_forward_value(obs, w1, b1, w2, b2, w3, b3):
+    """What evg_policy_value computes, in numpy: bf16-rounded operands (observations, W1, W2, w3, both hidden
+    activations), float32 accumulation, b1, b2 and b3 added in float32 (not rounded), no tanh after the last layer.
+    Returns float32 [rows]."""
+    f32 = np.float32
+    x = bf16_round(np.asarray(obs, dtype=f32))
+    h = np.tanh((x @ bf16_round(w1).T).astype(f32) + np.asarray(b1, f32)).astype(f32)
+    h = np.tanh((bf16_round(h) @ bf16_round(w2).T).astype(f32) + np.asarray(b2, f32)).astype(f32)
+    v = (bf16_round(h) @ bf16_round(np.asarray(w3, f32)).T).astype(f32) + np.asarray(b3, f32)
+    return v.astype(f32).reshape(-1)
+
+
 class FusedPPO:
     """PPO actor forward + PPOAgent.get_action's sampling for a BatchedEvergladesEnv, in one kernel:
     ``actions = FusedPPO(env, net)()`` reads env.obs in place (or, with obs_format='wire', the env's wire rows) and
@@ -442,3 +475,106 @@ class FusedRPPO:
                                                   C.c_void_p(self.idx.data_ptr()), _ptr(self.probs, want_probs), _ptr(self.logp, want_logp),
                                                   env._stream()))
         return env._actions
+
+
+def _value_params(net):
+    """The critic's (w1, b1, w2, b2, w3, b3) tensors of a Sequential(Linear, Tanh, Linear, Tanh, Linear(L, 1));
+    ValueError for another layer count or a last layer that is not Linear(L, 1)."""
+    import torch
+    lin = [m for m in net if isinstance(m, torch.nn.Linear)]
+    if len(lin) != 3:
+        raise ValueError("expected Sequential(Linear, Tanh, Linear, Tanh, Linear(L, 1)), got %d Linear layers" % len(lin))
+    if lin[2].out_features != 1:
+        raise ValueError("the critic's last layer must be Linear(L, 1), got Linear(%d, %d)" % (lin[2].in_features, lin[2].out_features))
+    return [t for m in lin for t in (m.weight, m.bias)]
+
+
+class FusedValue:
+    """PPO's critic for a BatchedEvergladesEnv, in one kernel: ``v = FusedValue(env, net)()`` is V of env.obs (float32
+    [N, 2] for player -1, [N] for player 0 or 1), written into ``.value``.  Called with stored rows it evaluates any
+    number M of matches in one launch: wire rows uint8 [M, row_bytes] or float32 observations [M, 2, obs_len] -> [M, 2]
+    (or [M]), e.g. a whole [T, N] rollout flattened.  bf16 operands and fp32 accumulation like the actors
+    (reference_forward_value); like FusedPPO.logp, values agree with a float32 torch critic to bf16 accuracy only."""
+
+    def __init__(self, env, net=None, weights=None, player=-1):
+        import torch
+        self._net = net if weights is None else None
+        if weights is None:
+            weights = _host_arrays(_value_params(net))
+        if len(weights) != 6:
+            raise ValueError("expected the 6 arrays (w1, b1, w2, b2, w3, b3), got %d" % len(weights))
+        _check_input_width(weights[0], env)
+        L = np.shape(weights[0])[0]
+        if not 1 <= L <= PPO_MAX_LATENT:
+            raise ValueError("the critic's width %d is outside 1..%d" % (L, PPO_MAX_LATENT))
+        shapes = [(L, env.obs_len), (L,), (L, L), (L,), (1, L), (1,)]
+        for i, (w, shape) in enumerate(zip(weights, shapes)):
+            if np.shape(w) != shape:
+                raise ValueError("parameter %d has shape %s, a critic of width %d needs %s (the last layer is Linear(L, 1))"
+                                 % (i, np.shape(w), L, shape))
+        if player not in (-1, 0, 1):
+            raise ValueError("player must be -1, 0 or 1, got %r" % (player,))
+        if env.obs_len >= PPO_IN_PAD:
+            raise ValueError("observations of %d values do not fit the %d input columns of the fused kernels" % (env.obs_len, PPO_IN_PAD))
+        img1, img2, img3, bias, self.latent = pack_value(*weights)
+        self.env, self.player = env, int(player)
+        dev = env.device
+        self._w = [torch.from_numpy(a).to(dev) for a in (img1, img2, img3, bias)]
+        self.value = torch.empty(self._shape(env.num_envs), dtype=torch.float32, device=dev)
+
+    def _shape(self, m):
+        return (m, 2) if self.player < 0 else (m,)
+
+    def refresh(self, net=None):
+        """Re-pack the weight images and the bias vector in place from `net` (default: the module this wrapper was built
+        with), on the device; see FusedDQN.refresh (CUDA graphs, the ValueError checks)."""
+        L, w = self.latent, self.env.obs_len
+        src = _refresh_sources(self, net, _value_params, [(L, w), (L,), (L, L), (L,), (1, L), (1,)])
+        env = self.env
+        i1, i2, i3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_pack_value(env._h, *src, L, i1, i2, i3, bias, env._stream()))
+
+    def __call__(self, obs=None, obs_format="f32", out=None):
+        """State values float32 [M, 2] (player -1) or [M].  obs None: the env's own observations (M = num_envs; 'wire'
+        reads env.obs_rows('wire'), the env stepped with obs_format='wire'), into .value unless `out` is given.
+        Otherwise `obs` is float32 [M, 2, obs_len] ('f32') or uint8 wire rows [M, row_bytes] ('wire'), contiguous on the
+        env's device, and the values go to `out` (allocated when None).  Wire rows give bit for bit the values of the
+        float32 observations they expand to.  ValueError, before anything is launched, for another format (the kernels
+        read no 'i16'), a tensor of the wrong dtype, shape or device, or one that is not contiguous."""
+        import torch
+        env = self.env
+        if obs_format not in ("f32", "wire"):
+            raise ValueError("obs_format must be 'f32' or 'wire', got %r" % (obs_format,))
+        fmt = _capi.OBS_F32 if obs_format == "f32" else _capi.OBS_WIRE
+        if obs is None:
+            obs = env.obs if fmt == _capi.OBS_F32 else env.obs_rows("wire")
+            m = env.num_envs
+            out = self.value if out is None else out
+        else:
+            if fmt == _capi.OBS_F32:
+                dtype, tail, what = torch.float32, (2, env.obs_len), "float32 observations [M, 2, %d]" % env.obs_len
+            else:
+                rb = int(env._lib.evg_obs_row_bytes(env._h, _capi.OBS_WIRE))
+                dtype, tail, what = torch.uint8, (rb,), "uint8 wire rows [M, %d]" % rb
+            if not isinstance(obs, torch.Tensor) or obs.dtype != dtype or not obs.is_contiguous() or obs.device != env.device \
+                    or obs.dim() != 1 + len(tail) or tuple(obs.shape[1:]) != tail:
+                raise ValueError("obs must be contiguous %s on %s, got %s" % (what, env.device, _describe(obs)))
+            m = obs.shape[0]
+            if out is None:
+                out = torch.empty(self._shape(m), dtype=torch.float32, device=env.device)
+        if not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or not out.is_contiguous() or out.device != env.device \
+                or tuple(out.shape) != self._shape(m):
+            raise ValueError("out must be a contiguous float32 tensor of shape %s on %s, got %s" % (self._shape(m), env.device, _describe(out)))
+        if m == 0:
+            return out
+        i1, i2, i3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
+        _capi.check(env._lib.evg_policy_value(env._h, fmt, C.c_void_p(obs.data_ptr()), m, self.player, i1, i2, i3, bias, self.latent,
+                                              C.c_void_p(out.data_ptr()), env._stream()))
+        return out
+
+
+def _describe(t):
+    import torch
+    if not isinstance(t, torch.Tensor):
+        return type(t).__name__
+    return "%s %s%s on %s" % (t.dtype, tuple(t.shape), "" if t.is_contiguous() else " (not contiguous)", t.device)

@@ -411,6 +411,32 @@ int evg_policy_rppo_logp(EvgSim* sim, int32_t format, const void* d_obs, int32_t
                          int32_t out_dim, int32_t div, int32_t mod, float* d_hidden, float* d_hidden_in, int8_t* d_actions,
                          int64_t* d_idx, float* d_probs, float* d_logp, void* stream);
 
+/* PPO's critic on the tensor cores (csrc/evg_policy_value.cu): the state value
+ *     v = Linear(latent, 1)(Tanh(Linear(latent, latent)(Tanh(Linear(obs_len, latent)(obs)))))
+ * — the value_layer of agents/PPO/ActorCritic.py — of n_matches matches' observations, for the rows of `player`
+ * (0, 1, or -1 = both).  n_matches is the caller's, not n_envs: the env's current observations, or a whole stored rollout
+ * ([T * N] rows flattened) in one call; 0 is a no-op.  Row i is (match i / 2, player i % 2) for player -1, else
+ * (match i, player).
+ *   format EVG_OBS_F32: d_obs float32 [n_matches][2][obs_len] (4-byte aligned).
+ *   format EVG_OBS_WIRE: d_obs wire rows [n_matches][evg_obs_row_bytes(sim, EVG_OBS_WIRE)] (16-byte aligned, needs
+ *       evg_bind), values bit for bit those of the float32 call on the expanded rows, as for evg_policy_ppo_fmt.
+ *   EVG_OBS_I16 and unknown formats return EVG_E_ARG.
+ *   d_value: float32 [n_matches][2] (player -1) or [n_matches].
+ * bf16 operands (observations, W1, W2, w3, both hidden activations), fp32 accumulation, b1, b2, b3 added in fp32, no tanh
+ * after the last layer.  Images as for evg_policy_ppo (Lp = latent rounded up to 16, Ka = latent rounded up to 64):
+ *     d_w1_img: W1[n][k] as an [Lp x EVG_PPO_IN_PAD] block, exactly as evg_policy_ppo's
+ *     d_w2_img: W2[n][k] as an [Lp x Ka] block, exactly as evg_policy_ppo's
+ *     d_w3_img: w3 as an [EVG_VALUE_OUT_PAD x Ka] block: row 0 = w3[k], the other rows zero,
+ *               (Ka / 64) * EVG_VALUE_OUT_PAD * 128 bytes
+ *     d_bias: float32 [2 * EVG_PPO_MAX_LATENT + EVG_VALUE_OUT_PAD] = b1 at 0, b2 at EVG_PPO_MAX_LATENT, b3 at
+ *             2 * EVG_PPO_MAX_LATENT, zero padded.
+ * Images and d_bias 16-byte aligned.  evgsim.policy.pack_value builds them on the host, evg_pack_value on the device.
+ * EVG_E_ARG for latent outside 1..EVG_PPO_MAX_LATENT, obs_len >= EVG_PPO_IN_PAD, a negative n_matches, a player outside
+ * -1..1 and NULL pointers. */
+#define EVG_VALUE_OUT_PAD 16
+int evg_policy_value(EvgSim* sim, int32_t format, const void* d_obs, int64_t n_matches, int32_t player, const void* d_w1_img,
+                     const void* d_w2_img, const void* d_w3_img, const float* d_bias, int32_t latent, float* d_value, void* stream);
+
 /* Wire rows -> the float32 observation vector on the device (csrc/evg_wire_expand.cu), bit for bit what the step writes
  * in EVG_OBS_F32 and what evgsim.wire.expand computes on the host; for training consumers that store the rows (a replay or
  * rollout memory: 128 bytes per match on DemoMap against 840) and expand a sampled minibatch.
@@ -426,7 +452,7 @@ int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64
                     float* d_reward, uint8_t* d_done, void* stream);
 
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
- * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo build on the host: one launch on `stream`, no host synchronisation,
+ * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
  * Sources are device arrays in torch's layouts (contiguous, row-major): d_w1 [hidden or latent][obs_len], d_w2 / d_w3
  * [out][in] as nn.Linear.weight, biases [out]; d_w_ih / d_w_hh [3 * latent][latent] and d_b_ih / d_b_hh [3 * latent] as
@@ -435,6 +461,7 @@ int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64
  *                  ceil((hidden + 1) / EVG_MLP_CHUNK) chunks each).
  *   evg_pack_ppo:  d_w1_img, d_w2_img, d_w3_img and d_bias as evg_policy_ppo reads them.
  *   evg_pack_rppo: the same, plus d_wi_img / d_wh_img and the GRU biases in d_bias as evg_policy_rppo reads them.
+ *   evg_pack_value: d_w1_img, d_w2_img, d_w3_img and d_bias as evg_policy_value reads them (d_w3 [1][latent], d_b3 [1]).
  * Every byte of every image and of d_bias is written, zero padding included.  Weights round to bf16 to nearest even
  * (overflow to +-Inf, subnormals kept); a NaN packs to a bf16 NaN of unspecified payload.  Images and d_bias must be
  * 16-byte aligned; hidden, latent, out_dim and obs_len are checked as the matching evg_policy_* checks them. */
@@ -445,6 +472,8 @@ int evg_pack_ppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float*
 int evg_pack_rppo(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3, const float* d_b3,
                   const float* d_w_ih, const float* d_b_ih, const float* d_w_hh, const float* d_b_hh, int32_t latent, int32_t out_dim,
                   void* d_w1_img, void* d_w2_img, void* d_wi_img, void* d_wh_img, void* d_w3_img, float* d_bias, void* stream);
+int evg_pack_value(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                   const float* d_b3, int32_t latent, void* d_w1_img, void* d_w2_img, void* d_w3_img, float* d_bias, void* stream);
 
 /* Reward shaping of the reference's training scripts (utils/reward_shaping.py:17-56) on the step's outputs:
  * d_out float32 [n_envs][2].  turnNum (steps played before this one) is read from the observation's turn

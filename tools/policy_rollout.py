@@ -18,7 +18,10 @@ evg_decode_dqn), PPO's forward, sampling and unravel in evg_policy_ppo, the recu
 and unravel in evg_policy_rppo, which also carries the hidden state and zeroes it when a match starts over (their draws
 come from the simulator's tape, not from torch's generator).  --obs wire (with --fused) steps the simulator in the wire
 format and the fused kernel reads those rows (128 B per match instead of 840); --opponent puts a scripted agent
-(env.agent_actions) on player 1's side, the fused network plays player 0.  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
+(env.agent_actions) on player 1's side, the fused network plays player 0.  --critic adds PPO's critic
+(Linear(105, 128) - Tanh - Linear(128, 128) - Tanh - Linear(128, 1), ActorCritic's value_layer) evaluated on every turn's
+observations, the value a PPO rollout stores next to the draws: in torch (bf16 forward, float32 observations) or fused
+(evg_policy_value, on the same rows the actor read).  Matches shard over the ranks with no collective on the path; rank 0 prints one JSON line.
 """
 import argparse
 import json
@@ -89,11 +92,18 @@ def main():
     ap.add_argument("--want", default="none", choices=["none", "logp", "probs"],
                     help="with --fused --policy ppo|rppo: what a PPO rollout keeps of each turn besides the draws: nothing, each "
                          "draw's log-probability (and for rppo the starting state, hidden_in), or the whole distribution")
+    ap.add_argument("--critic", default="none", choices=["none", "torch", "fused"],
+                    help="with --fused --policy ppo|rppo: the state value of every row each turn, from a torch bf16 critic or "
+                         "evg_policy_value")
     args = ap.parse_args()
     if (args.obs == "wire" or args.opponent != "none") and not args.fused:
         ap.error("--obs wire and --opponent need --fused")
     if args.want != "none" and not (args.fused and args.policy in ("ppo", "rppo")):
         ap.error("--want needs --fused and --policy ppo or rppo")
+    if args.critic != "none" and not (args.fused and args.policy in ("ppo", "rppo")):
+        ap.error("--critic needs --fused and --policy ppo or rppo")
+    if args.critic == "torch" and args.obs != "f32":
+        ap.error("--critic torch reads the float32 observations (--obs f32)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -116,6 +126,18 @@ def main():
     opponent = {"none": None, "random": evgsim._capi.AGENT_RANDOM, "base_rush": evgsim._capi.AGENT_BASE_RUSH,
                 "swarm": evgsim._capi.AGENT_SWARM}[args.opponent]
 
+    critic_net = value = critic = None
+    if args.critic != "none":
+        torch.manual_seed(1)
+        critic_net = torch.nn.Sequential(torch.nn.Linear(105, 128), torch.nn.Tanh(), torch.nn.Linear(128, 128), torch.nn.Tanh(),
+                                         torch.nn.Linear(128, 1)).to(env.device).eval()
+        if args.critic == "fused":
+            from evgsim import policy as evp
+            critic = evp.FusedValue(env, critic_net)
+        else:
+            critic_net = critic_net.to(torch.bfloat16)
+            value = torch.empty((E, 2), dtype=torch.float32, device=env.device)
+
     want = {"none": {}, "probs": {"want_probs": True},
             "logp": {"want_logp": True, **({"want_hidden_in": True} if args.policy == "rppo" else {})}}[args.want]
 
@@ -124,6 +146,11 @@ def main():
             env.step(policy_actions(env, net, args.policy, dtype, hidden))
         else:
             actions = fused(obs_format=args.obs, **want)
+            if critic is not None:  # V of the rows the actor read, into critic.value
+                critic(obs_format=args.obs)
+            elif value is not None:
+                with torch.no_grad():
+                    value.copy_(critic_net(env.obs.view(-1, env.obs_len).to(torch.bfloat16)).float().view(E, 2))
             if opponent is not None:  # player 1's rows from the scripted agent, player 0's from the network
                 env.agent_actions(evgsim._capi.AGENT_EXTERNAL, opponent)
             env.step(actions, obs_format=args.obs)
@@ -160,7 +187,7 @@ def main():
     if rank == 0:
         sec = float(ms.item()) / 1e3
         print(json.dumps({"workload": "policy-in-the-loop self-play (BASELINE.json configs[3])", "policy": args.policy, "dtype": "bf16 operands, fp32 accumulate (%s)" % {"dqn": "evg_policy_mlp", "ppo": "evg_policy_ppo", "rppo": "evg_policy_rppo"}[args.policy] if args.fused else args.dtype, "fused_forward": bool(args.fused), "obs_format": args.obs, "opponent": args.opponent,
-                          "cuda_graph": bool(args.graph), "want": args.want,
+                          "cuda_graph": bool(args.graph), "want": args.want, "critic": args.critic,
                           "n_gpus": world, "envs_per_gpu": E, "turns": args.turns, "env_turns_per_s": E * world * args.turns / sec,
                           "ms_per_turn": sec * 1e3 / args.turns, "episodes": stats["episodes"], "wins": stats["wins"], "ties": stats["ties"]}))
     if world > 1:
