@@ -1085,6 +1085,31 @@ int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64
     return EVG_OK;
 }
 
+int evg_gae(EvgSim* sim, int32_t n_turns, int64_t n_matches, int32_t player, const void* d_rows, const float* d_reward, const uint8_t* d_done,
+            const float* d_values, float gamma, float lam, float* d_adv, float* d_ret, void* stream)
+{
+    int rc = check_sim(sim, false);
+    if (rc) return rc;
+    if (n_turns < 1) return fail(EVG_E_ARG, "evg_gae: n_turns %d must be at least 1", n_turns);
+    if (n_matches < 1 || n_matches > INT32_MAX) return fail(EVG_E_ARG, "evg_gae: n_matches %lld outside 1..2^31-1", (long long)n_matches);
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "evg_gae: player %d outside -1..1", player);
+    if (!d_values || !d_adv || !d_ret) return fail(EVG_E_ARG, "evg_gae: null values, adv or ret");
+    if (!d_rows && (!d_reward || !d_done)) return fail(EVG_E_ARG, "evg_gae: the wire rows are needed unless both reward and done are given");
+    if ((uintptr_t)d_rows % 16) return fail(EVG_E_ARG, "evg_gae: wire rows must be 16-byte aligned");
+    const uintptr_t col = player < 0 ? 8 : 4;  // float2 operands of player -1
+    if (((uintptr_t)d_values | (uintptr_t)d_adv | (uintptr_t)d_ret) % col || (uintptr_t)d_reward % col)
+        return fail(EVG_E_ARG, "evg_gae: values, adv, ret and reward must be %d-byte aligned", (int)col);
+    if (!(gamma >= 0.f && gamma <= 1.f) || !(lam >= 0.f && lam <= 1.f))  // NaN fails both comparisons
+        return fail(EVG_E_ARG, "evg_gae: gamma %g and lambda %g must lie in [0, 1]", (double)gamma, (double)lam);
+    const int n = sim->tables.n_nodes;
+    cudaError_t e = evg::launch_gae(n_turns, n_matches, player, (const uint32_t*)d_rows, evg::wire_bytes(n) / 4,
+                                    (EVG_WIRE_NODE0 + 4 * n + 3 * evg::kGroupLanes) / 4, d_reward, d_done, d_values, gamma, lam, d_adv,
+                                    d_ret, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_gae_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
 int evg_pack_mlp(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, int32_t hidden, int32_t out_dim,
                  void* d_w1_img, void* d_w2_img, void* stream)
 {

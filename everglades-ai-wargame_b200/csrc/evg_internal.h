@@ -176,6 +176,10 @@ cudaError_t launch_policy_value(const void* obs, int64_t n_matches, int player, 
 // wire rows -> float32 observations, reward and done (evg_wire_expand.cu); index / reward / done may be null
 cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n_rows, const int64_t* index, int64_t n_out, int player,
                                float* obs, float* reward, uint8_t* done, cudaStream_t stream);
+// GAE(lambda) advantages and returns of a stored rollout (evg_gae.cu); rows (`words` 32-bit words each, the rewards at
+// `reward_word`) are read only for what reward / done do not give
+cudaError_t launch_gae(int n_turns, int64_t n_matches, int player, const uint32_t* rows, int words, int reward_word, const float* reward,
+                       const uint8_t* done, const float* values, float gamma, float lam, float* adv, float* ret, cudaStream_t stream);
 // the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();

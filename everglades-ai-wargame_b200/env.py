@@ -384,6 +384,16 @@ class BatchedEvergladesEnv:
                                                C.c_void_p(self.obs.data_ptr()), C.c_void_p(out.data_ptr()), self._stream()))
         return out
 
+    def _need(self, name, t, dtype, shape):
+        """ValueError unless t is a contiguous `dtype` tensor on this env's device (of `shape` unless it is None)."""
+        torch = _torch()
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != self.device or not t.is_contiguous() \
+                or (shape is not None and tuple(t.shape) != shape):
+            raise ValueError("%s must be a contiguous %s tensor%s on %s, got %s" % (
+                name, dtype, "" if shape is None else " of shape %s" % (shape,), self.device,
+                "%s %s%s on %s" % (t.dtype, tuple(t.shape), "" if t.is_contiguous() else " (not contiguous)", t.device)
+                if isinstance(t, torch.Tensor) else type(t).__name__))
+
     def expand_wire(self, rows, index=None, player=-1, out=None, reward=None, done=None):
         """Wire rows uint8 [M, row_bytes] (obs_rows('wire') of some turn, or rows stored since) -> the float32
         observations on the device, bit for bit what the step writes in the f32 format (evg_wire_expand).  Output row i
@@ -393,15 +403,8 @@ class BatchedEvergladesEnv:
         (allocated when None).  ValueError, before anything is launched, for a tensor of the wrong dtype, width, shape or
         device, or one that is not contiguous."""
         torch = _torch()
+        need = self._need
         rb = int(self._lib.evg_obs_row_bytes(self._h, _capi.OBS_WIRE))
-
-        def need(name, t, dtype, shape):
-            if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != self.device or not t.is_contiguous() \
-                    or (shape is not None and tuple(t.shape) != shape):
-                raise ValueError("%s must be a contiguous %s tensor%s on %s, got %s" % (
-                    name, dtype, "" if shape is None else " of shape %s" % (shape,), self.device,
-                    "%s %s%s on %s" % (t.dtype, tuple(t.shape), "" if t.is_contiguous() else " (not contiguous)", t.device)
-                    if isinstance(t, torch.Tensor) else type(t).__name__))
 
         need("rows", rows, torch.uint8, None)
         if rows.dim() != 2 or rows.shape[1] != rb:
@@ -428,6 +431,57 @@ class BatchedEvergladesEnv:
         _capi.check(self._lib.evg_wire_expand(self._h, ptr(rows), rows.shape[0], ptr(index), k, int(player), ptr(out), ptr(reward),
                                               ptr(done), self._stream()))
         return out
+
+    def gae(self, values, rows=None, reward=None, done=None, gamma=0.99, lam=0.95, player=-1, adv=None, ret=None):
+        """PPO's advantages and returns, GAE(lambda), of a stored rollout in one launch (evg_gae; PPOAgent.py:190-218).
+
+        values: float32 [T+1, M, 2] (player -1) or [T+1, M] (player 0 or 1), V of the states the actor read at turns
+        0..T, e.g. FusedValue over the T+1 stored wire rows; row T is the bootstrap state.  T and M come from it.
+        Turn t's reward and done flag come from reward (float32 [T, M, 2], both players, what env.reward or
+        env.shape_reward() gave per turn) and done (uint8 [T, M]) when given, otherwise from rows (uint8 [T+1, M,
+        row_bytes], obs_rows('wire') of each turn, row t+1 holding turn t's), which are needed when either is None.
+        The done flag cuts bootstrap and trace, a time limit included (include/evgsim.h gives the float32 recurrence,
+        tests/ppo_gae.py the numpy statement it equals bit for bit).  Returns (adv, ret), float32 [T, M, 2] or [T, M],
+        allocated when None; with both given the call allocates nothing and can be captured in a CUDA graph.  ValueError,
+        before anything is launched, for a tensor of the wrong dtype, shape, row width or device, or one that is not
+        contiguous, and for gamma or lam outside [0, 1]."""
+        torch = _torch()
+        if player not in (-1, 0, 1):
+            raise ValueError("player must be -1, 0 or 1, got %r" % (player,))
+        for name, x in (("gamma", gamma), ("lam", lam)):
+            if not 0.0 <= float(x) <= 1.0:
+                raise ValueError("%s must lie in [0, 1], got %r" % (name, x))
+        cols = (2,) if player < 0 else ()
+        need = self._need
+
+        need("values", values, torch.float32, None)
+        if values.dim() != 2 + len(cols) or tuple(values.shape[2:]) != cols or values.shape[0] < 2 or values.shape[1] < 1:
+            raise ValueError("values must be float32 [T+1, M%s] with T >= 1 and M >= 1 for player %d, got shape %s"
+                             % (", 2" if cols else "", player, tuple(values.shape)))
+        T, M = values.shape[0] - 1, values.shape[1]
+        if rows is None and (reward is None or done is None):
+            raise ValueError("gae needs the wire rows unless both reward and done are given")
+        if rows is not None:
+            rb = int(self._lib.evg_obs_row_bytes(self._h, _capi.OBS_WIRE))
+            need("rows", rows, torch.uint8, (T + 1, M, rb))
+        if reward is not None:
+            need("reward", reward, torch.float32, (T, M, 2))
+        if done is not None:
+            need("done", done, torch.uint8, (T, M))
+        shape = (T, M) + cols
+        if adv is None:
+            adv = torch.empty(shape, dtype=torch.float32, device=self.device)
+        if ret is None:
+            ret = torch.empty(shape, dtype=torch.float32, device=self.device)
+        need("adv", adv, torch.float32, shape)
+        need("ret", ret, torch.float32, shape)
+
+        def ptr(t):
+            return None if t is None else C.c_void_p(t.data_ptr())
+
+        _capi.check(self._lib.evg_gae(self._h, T, M, int(player), ptr(rows), ptr(reward), ptr(done), ptr(values), float(gamma),
+                                      float(lam), ptr(adv), ptr(ret), self._stream()))
+        return adv, ret
 
     # ------------------------------------------------------------------ snapshots
     def get_state(self, first=0, count=None):

@@ -451,6 +451,35 @@ int evg_policy_value(EvgSim* sim, int32_t format, const void* d_obs, int64_t n_m
 int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64_t* d_index, int64_t n_out, int32_t player, float* d_obs,
                     float* d_reward, uint8_t* d_done, void* stream);
 
+/* PPO's advantages and returns, GAE(lambda), of a stored rollout of T = n_turns >= 1 turns of M = n_matches matches
+ * (csrc/evg_gae.cu; agents/PPO/PPOAgent.py:190-218).  A column is a (match, player): both players for player -1, that
+ * one for 0 or 1.
+ *   d_values: float32 [T+1][M][2] (player -1) or [T+1][M]: V of the states the actor read at turns 0..T, i.e.
+ *             evg_policy_value on the T+1 stored wire rows; row T is the bootstrap state.
+ *   The reward and done flag of turn t < T come from
+ *     d_reward float32 [T][M][2] (both players' rewards, whatever `player` is) and d_done uint8 [T][M] when given, and
+ *     otherwise from d_rows, wire rows [T+1][M][evg_obs_row_bytes(sim, EVG_OBS_WIRE)] as the step wrote them: row t+1
+ *     holds turn t's rewards and done flag (row 0's are not read).  d_rows is needed when either of the two is NULL;
+ *     rows with the caller's own (e.g. shaped) rewards take d_reward and the rows' done flags.
+ *   d_adv, d_ret: float32 [T][M][2] or [T][M].
+ * In float32, each operation rounded on its own (no fused multiply-add), backward from A_T = 0, gl = fl(gamma * lam):
+ *     nv = d_t ? 0 : V_{t+1},   na = d_t ? 0 : A_{t+1}
+ *     delta_t = fl(fl(r_t + fl(gamma * nv)) - V_t),   A_t = fl(delta_t + fl(gl * na)),   R_t = fl(A_t + V_t)
+ * (0 is selected rather than multiplied by 1 - d, so a non-finite value past a done flag does not leak in).
+ * The done flag cuts both the bootstrap and the trace, whatever ended the match: reaching the turn limit
+ * (EVG_STATUS_TIME_EXPIRED) is a terminal of the game, with its score and reward, not a truncation.  Under
+ * EVG_AUTORESET_TERMINAL / _NEXT the values are those of the rows the actor read, the terminal observation that _TERMINAL
+ * shows to the next match's first turn included.  Under EVG_AUTORESET_OFF the pass takes each row's done flag as the step
+ * wrote it.  A finished match that keeps being stepped is still simulated and its end conditions are evaluated again every
+ * turn: done is 1 on every turn from the turn limit on, and on a turn where a capture or annihilation holds.  Each such
+ * turn is then a one-turn episode, A_t = fl(r_t - V_t); a turn between them (a base taken back) traces into the next one.
+ * None of them is a turn of a real match: masking them is the caller's.
+ * One launch on `stream`, no allocation, no synchronisation.  EVG_E_ARG for n_turns < 1, n_matches outside 1..2^31-1, a
+ * player outside -1..1, NULL values / adv / ret, no rows while d_reward or d_done is NULL, rows not 16-byte aligned,
+ * values / adv / ret / reward not 8-byte aligned for player -1 (4-byte otherwise), and gamma or lam outside [0, 1] or NaN. */
+int evg_gae(EvgSim* sim, int32_t n_turns, int64_t n_matches, int32_t player, const void* d_rows, const float* d_reward, const uint8_t* d_done,
+            const float* d_values, float gamma, float lam, float* d_adv, float* d_ret, void* stream);
+
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
  * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
