@@ -1110,6 +1110,55 @@ int evg_gae(EvgSim* sim, int32_t n_turns, int64_t n_matches, int32_t player, con
     return EVG_OK;
 }
 
+namespace {
+
+// evg_ppo_loss / _grad's shared argument checks, before the handle's, so they hold without a device
+int check_ppo_loss(const char* fn, int64_t n_rows, int32_t n_dist, int32_t n_actions, float clip, const void* const* f32, int n_f32,
+                   const int64_t* d_idx)
+{
+    if (n_rows < 1 || n_rows > INT32_MAX) return fail(EVG_E_ARG, "%s: n_rows %lld outside 1..2^31-1", fn, (long long)n_rows);
+    if (n_dist != 1 && n_dist != EVG_MAX_ACTIONS) return fail(EVG_E_ARG, "%s: n_dist %d must be 1 or %d", fn, n_dist, EVG_MAX_ACTIONS);
+    if (n_actions < EVG_MAX_ACTIONS || n_actions > 256) return fail(EVG_E_ARG, "%s: n_actions %d outside %d..256", fn, n_actions, EVG_MAX_ACTIONS);
+    if (!(clip >= 0.f && clip < 1.f)) return fail(EVG_E_ARG, "%s: clip %g outside [0, 1)", fn, (double)clip);  // NaN fails too
+    if (!d_idx) return fail(EVG_E_ARG, "%s: null idx", fn);
+    if ((uintptr_t)d_idx % 8) return fail(EVG_E_ARG, "%s: idx must be 8-byte aligned", fn);
+    for (int i = 0; i < n_f32; ++i) {
+        if (!f32[i]) return fail(EVG_E_ARG, "%s: null float32 operand %d", fn, i);
+        if ((uintptr_t)f32[i] % 4) return fail(EVG_E_ARG, "%s: float32 operand %d must be 4-byte aligned", fn, i);
+    }
+    return EVG_OK;
+}
+
+}  // namespace
+
+int evg_ppo_loss(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions, const float* d_z, const int64_t* d_idx, const float* d_old_logp,
+                 const float* d_adv, float clip, float* d_surr, float* d_ent, float* d_logp, float* d_ratio, void* stream)
+{
+    const void* f32[] = {d_z, d_old_logp, d_adv, d_surr, d_ent, d_logp, d_ratio};
+    int rc = check_ppo_loss("evg_ppo_loss", n_rows, n_dist, n_actions, clip, f32, 7, d_idx);
+    if (rc || (rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_ppo_loss(n_rows, n_dist, n_actions, d_z, d_idx, d_old_logp, d_adv, 1.f - clip, 1.f + clip, d_surr, d_ent, d_logp,
+                                         d_ratio, sim->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_ppo_loss kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_ppo_loss_grad(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions, const float* d_z, const int64_t* d_idx, const float* d_adv,
+                      const float* d_ratio, float clip, const float* d_g_surr, const float* d_g_ent, float* d_dz, void* stream)
+{
+    const void* f32[] = {d_z, d_adv, d_ratio, d_dz};
+    int rc = check_ppo_loss("evg_ppo_loss_grad", n_rows, n_dist, n_actions, clip, f32, 4, d_idx);
+    if (rc) return rc;
+    if ((uintptr_t)d_g_surr % 4 || (uintptr_t)d_g_ent % 4) return fail(EVG_E_ARG, "evg_ppo_loss_grad: g_surr and g_ent must be 4-byte aligned");
+    if ((rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_ppo_loss_grad(n_rows, n_dist, n_actions, d_z, d_idx, d_adv, d_ratio, 1.f - clip, 1.f + clip, d_g_surr, d_g_ent,
+                                              d_dz, sim->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_ppo_loss_grad kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
 int evg_pack_mlp(EvgSim* sim, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, int32_t hidden, int32_t out_dim,
                  void* d_w1_img, void* d_w2_img, void* stream)
 {

@@ -180,6 +180,12 @@ cudaError_t launch_wire_expand(const WireSrc& w, const uint32_t* rows, int64_t n
 // `reward_word`) are read only for what reward / done do not give
 cudaError_t launch_gae(int n_turns, int64_t n_matches, int player, const uint32_t* rows, int words, int reward_word, const float* reward,
                        const uint8_t* done, const float* values, float gamma, float lam, float* adv, float* ret, cudaStream_t stream);
+// PPO's policy loss from the actor's last Linear output, forward and gradient (evg_ppo_loss.cu); lo / hi are
+// fl(1 - clip) and fl(1 + clip); g_surr / g_ent may be null; sm_count sizes the persistent grid
+cudaError_t launch_ppo_loss(int64_t n_rows, int n_dist, int n, const float* z, const int64_t* idx, const float* old_logp, const float* adv,
+                            float lo, float hi, float* surr, float* ent, float* logp, float* ratio, int sm_count, cudaStream_t stream);
+cudaError_t launch_ppo_loss_grad(int64_t n_rows, int n_dist, int n, const float* z, const int64_t* idx, const float* adv, const float* ratio,
+                                 float lo, float hi, const float* g_surr, const float* g_ent, float* dz, int sm_count, cudaStream_t stream);
 // the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();

@@ -25,6 +25,41 @@ def _torch():
 
 OBS_FORMATS = {"f32": _capi.OBS_F32, "i16": _capi.OBS_I16, "wire": _capi.OBS_WIRE}
 
+_PPO_LOSS = None
+
+
+def _ppo_loss_function():
+    """The torch.autograd.Function of BatchedEvergladesEnv.ppo_loss (defined on first use: torch is imported lazily)."""
+    global _PPO_LOSS
+    if _PPO_LOSS is None:
+        torch = _torch()
+
+        class PPOLoss(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, z, env, idx, old_logp, adv, clip, K, n):
+                B = z.shape[0]
+                surr, ent, ratio = (torch.empty(B, dtype=torch.float32, device=z.device) for _ in range(3))
+                logp = torch.empty((B, _capi.MAX_ACTIONS), dtype=torch.float32, device=z.device)
+                env._ppo_loss_launch(z, idx, old_logp, adv, clip, K, n, surr, ent, logp, ratio)
+                ctx.save_for_backward(z, idx, adv, ratio)
+                ctx.env, ctx.clip, ctx.K, ctx.n = env, clip, K, n
+                ctx.mark_non_differentiable(logp, ratio)
+                ctx.set_materialize_grads(False)
+                return surr, ent, logp, ratio
+
+            @staticmethod
+            def backward(ctx, g_surr, g_ent, _g_logp, _g_ratio):
+                z, idx, adv, ratio = ctx.saved_tensors
+                if g_surr is None and g_ent is None:
+                    return (None,) * 8
+                g_surr, g_ent = (None if g is None else g.to(torch.float32).contiguous() for g in (g_surr, g_ent))
+                dz = torch.empty_like(z)
+                ctx.env._ppo_loss_grad_launch(z, idx, adv, ratio, ctx.clip, ctx.K, ctx.n, g_surr, g_ent, dz)
+                return (dz,) + (None,) * 7
+
+        _PPO_LOSS = PPOLoss
+    return _PPO_LOSS
+
 
 class BatchedEvergladesEnv:
     """N Everglades matches stepped in lockstep by one CUDA launch per turn.
@@ -482,6 +517,50 @@ class BatchedEvergladesEnv:
         _capi.check(self._lib.evg_gae(self._h, T, M, int(player), ptr(rows), ptr(reward), ptr(done), ptr(values), float(gamma),
                                       float(lam), ptr(adv), ptr(ret), self._stream()))
         return adv, ret
+
+    def ppo_loss(self, z, idx, old_logp, adv, clip=0.2):
+        """PPO's policy loss per row from the output of the actor's last Linear, before its Tanh and Softmax (evg_ppo_loss,
+        DESIGN.md §4.12): the stored draws' log-probabilities under the project's own sampling, the entropy and the
+        clipped surrogate, in one launch forward and one backward.
+
+        z: float32 [B, n] for FusedPPO's actor (one distribution, 7 draws without replacement) or [B, 7, n] for
+        FusedRPPO's (distribution k serves draw k, with replacement), n = 7..256 actions.  idx int64 [B, 7] and old_logp
+        float32 [B, 7] are the actor's .idx and .logp of the stored turn, adv float32 [B] its advantage (e.g. env.gae's,
+        viewed as [T * N * 2]); clip is epsilon in [0, 1).  Returns (surr, ent, info): surr = -min(r A, clamp(r, 1 - eps,
+        1 + eps) A) and ent = the mean over the K distributions of their entropy, float32 [B] each and differentiable with
+        respect to z (the backward is evg_ppo_loss_grad); info["logp"] float32 [B, 7] (each draw's new log-probability)
+        and info["ratio"] float32 [B] (r = exp(sum logp - sum old_logp)) carry no gradient.  Reduction and masking are the
+        caller's, e.g. (surr * w).sum() / w.sum() - c * (ent * w).sum() / w.sum().  A row with an index outside [0, n)
+        gives NaN outputs and a NaN gradient row.  ValueError, before anything is launched, for a tensor of the wrong
+        dtype, shape or device, one that is not contiguous, and for clip outside [0, 1)."""
+        K, n = self._ppo_loss_check(z, idx, old_logp, adv, clip)
+        surr, ent, logp, ratio = _ppo_loss_function().apply(z, self, idx, old_logp, adv, float(clip), K, n)
+        return surr, ent, {"logp": logp, "ratio": ratio}
+
+    def _ppo_loss_check(self, z, idx, old_logp, adv, clip):
+        """(K, n) of ppo_loss's z after its ValueError checks."""
+        torch = _torch()
+        if not (isinstance(clip, (int, float)) and 0.0 <= float(clip) and np.float32(clip) < 1.0):
+            raise ValueError("clip must lie in [0, 1), got %r" % (clip,))
+        self._need("z", z, torch.float32, None)
+        if z.dim() not in (2, 3) or (z.dim() == 3 and z.shape[1] != _capi.MAX_ACTIONS) or z.shape[0] < 1 \
+                or not _capi.MAX_ACTIONS <= z.shape[-1] <= 256:
+            raise ValueError("z must be float32 [B, n] or [B, 7, n] with B >= 1 and 7 <= n <= 256, got shape %s" % (tuple(z.shape),))
+        B = z.shape[0]
+        self._need("idx", idx, torch.int64, (B, _capi.MAX_ACTIONS))
+        self._need("old_logp", old_logp, torch.float32, (B, _capi.MAX_ACTIONS))
+        self._need("adv", adv, torch.float32, (B,))
+        return (1 if z.dim() == 2 else _capi.MAX_ACTIONS), int(z.shape[-1])
+
+    def _ppo_loss_launch(self, z, idx, old_logp, adv, clip, K, n, surr, ent, logp, ratio):
+        p = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
+        _capi.check(self._lib.evg_ppo_loss(self._h, z.shape[0], K, n, p(z), p(idx), p(old_logp), p(adv), clip, p(surr), p(ent), p(logp),
+                                           p(ratio), self._stream()))
+
+    def _ppo_loss_grad_launch(self, z, idx, adv, ratio, clip, K, n, g_surr, g_ent, dz):
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+        _capi.check(self._lib.evg_ppo_loss_grad(self._h, z.shape[0], K, n, p(z), p(idx), p(adv), p(ratio), clip, p(g_surr), p(g_ent),
+                                                p(dz), self._stream()))
 
     # ------------------------------------------------------------------ snapshots
     def get_state(self, first=0, count=None):

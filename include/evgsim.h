@@ -480,6 +480,41 @@ int evg_wire_expand(EvgSim* sim, const void* d_rows, int64_t n_rows, const int64
 int evg_gae(EvgSim* sim, int32_t n_turns, int64_t n_matches, int32_t player, const void* d_rows, const float* d_reward, const uint8_t* d_done,
             const float* d_values, float gamma, float lam, float* d_adv, float* d_ret, void* stream);
 
+/* PPO's policy loss for B = n_rows stored rows, from the output of the actor's last Linear (before its Tanh and Softmax),
+ * and its gradient (csrc/evg_ppo_loss.cu; DESIGN.md §4.12).  K = n_dist, n = n_actions (7..256, 132 on DemoMap):
+ *   d_z       float32 [B][K][n]. K = 1: the feed-forward actor, one distribution, 7 draws without replacement
+ *             (evg_policy_ppo_logp).  K = 7: the recurrent actor, distribution k serves draw k, with replacement
+ *             (evg_policy_rppo_logp).
+ *   d_idx     int64 [B][7], the draws as d_idx of those calls stored them;  d_old_logp float32 [B][7], their d_logp;
+ *   d_adv     float32 [B], the row's advantage A;  clip: epsilon in [0, 1).
+ * Per row, in float32 (accurate tanhf / expf / logf, no fast math):
+ *   y = tanh(z),  S_k = sum_i exp(y_k,i) (no max subtraction: y lies in [-1, 1]),  p_k,i = exp(y_k,i) / S_k,
+ *   log p_k,i = y_k,i - log S_k,  H_k = -sum_i p_k,i log p_k,i
+ *   K = 1:  T_k = sum of p_i over the i not in idx[0..k-1];   K = 7:  T_k = sum_i p_k,i (the sampler's normaliser)
+ *   logp_k = log p_{k or 0, idx_k} - log T_k;   ell = sum_{k=0..6} logp_k and ell_old = sum_k old_logp_k, both in k order
+ *   ratio = exp(ell - ell_old);  surr = -min(ratio A, clamp(ratio, lo, hi) A), lo = fl(1 - clip), hi = fl(1 + clip)
+ *   ent = fl(sum_k H_k / K), summed in k order
+ * Sums over i run in a fixed order (each lane of a warp adds elements lane + 32 s in ascending s, then an xor butterfly
+ * 16, 8, 4, 2, 1; tests/ppo_loss.py states it), so a row's logp fed back as its old_logp gives ratio == 1 exactly and
+ * surr == -A.  p >= 1 / (1 + (n-1) e^2) and, for K = 1, T_6 >= (n - 6) min p, so every log is finite.
+ * evg_ppo_loss writes d_surr [B], d_ent [B], d_logp [B][7] and d_ratio [B].
+ * evg_ppo_loss_grad writes d_dz [B][K][n] = g_surr d surr/dz + g_ent d ent/dz from d_ratio (evg_ppo_loss's) and the
+ * upstream gradients d_g_surr, d_g_ent float32 [B], either NULL for zero, recomputing y, p, T and H from d_z:
+ *   G = 0 where A > 0 and ratio > hi or A < 0 and ratio < lo (the clipped branch is the minimum), else fl(fl(-A ratio) g_surr)
+ *   (at a tie, ratio exactly lo, hi or 1, the unclipped branch's, as torch's autograd of the expression above gives)
+ *   d ell / d y_k,m = c_k,m - p_k,m Q_k,m: K = 1, c = the number of draws of m, Q = sum of 1 / T_j over the draws j
+ *   whose T_j counted m (a prefix sum in j);  K = 7, c = [m = idx_k], Q = 1 / T_k
+ *   dz = (1 - y^2) (G (c - p Q) - (g_ent / K) p (log p + H_k)), a term skipped when its factor G or g_ent is 0, so dz is
+ *   exactly +0 where both are 0 and a clipped row's dz is its entropy part alone.
+ * A row with an index outside [0, n) reads nothing out of bounds: its surr, ent, ratio and seven logp, and all of its dz,
+ * are NaN.  One launch on `stream` each, no allocation, no synchronisation.  EVG_E_ARG, checked before the handle, for
+ * n_rows outside 1..2^31-1, K not 1 or 7, n outside 7..256, clip outside [0, 1) or NaN, a NULL operand other than
+ * g_surr / g_ent, d_idx not 8-byte aligned and a float32 operand not 4-byte aligned. */
+int evg_ppo_loss(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions, const float* d_z, const int64_t* d_idx, const float* d_old_logp,
+                 const float* d_adv, float clip, float* d_surr, float* d_ent, float* d_logp, float* d_ratio, void* stream);
+int evg_ppo_loss_grad(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions, const float* d_z, const int64_t* d_idx, const float* d_adv,
+                      const float* d_ratio, float clip, const float* d_g_surr, const float* d_g_ent, float* d_dz, void* stream);
+
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
  * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
