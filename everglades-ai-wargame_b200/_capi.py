@@ -183,6 +183,9 @@ SYMBOLS = [
     ("evg_gae", C.c_int, [_P, C.c_int32, C.c_int64, C.c_int32, _P, _P, _P, _P, C.c_float, C.c_float, _P, _P, _P]),
     ("evg_ppo_loss", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_float, _P, _P, _P, _P, _P]),
     ("evg_ppo_loss_grad", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_float, _P, _P, _P, _P]),
+    ("evg_rppo_train_pack", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    ("evg_rppo_train_forward", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_rppo_train_backward", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     ("evg_pack_mlp", C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     ("evg_pack_ppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_pack_rppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),

@@ -366,7 +366,8 @@ int evg_create(const EvgConfig* cfg, int64_t n_envs, uint64_t seed, int64_t env_
     s->sm_count = prop.multiProcessorCount;
     // the shared-memory opt-ins are per device: made on the simulator's, for the step and the policy kernels
     if ((e = evg::set_step_smem(s->smem)) != cudaSuccess || (e = evg::set_policy_mlp_smem()) != cudaSuccess || (e = evg::set_policy_ppo_smem()) != cudaSuccess ||
-        (e = evg::set_policy_rppo_smem()) != cudaSuccess || (e = evg::set_policy_value_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
+        (e = evg::set_policy_rppo_smem()) != cudaSuccess || (e = evg::set_policy_value_smem()) != cudaSuccess ||
+        (e = evg::set_rppo_train_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
     int per_sm = 0;
     if ((e = evg::step_occupancy(t, s->smem, &per_sm)) != cudaSuccess || per_sm < 1) { delete s; return cuda_fail(e, "occupancy query"); }
     // persistent CTAs: a whole number of resident waves, never more CTAs than matches need
@@ -1155,6 +1156,69 @@ int evg_ppo_loss_grad(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_act
     cudaError_t e = evg::launch_ppo_loss_grad(n_rows, n_dist, n_actions, d_z, d_idx, d_adv, d_ratio, 1.f - clip, 1.f + clip, d_g_surr, d_g_ent,
                                               d_dz, sim->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_ppo_loss_grad kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+namespace {
+
+// evg_rppo_train_*'s shared argument checks, before the handle's, so they hold without a device: the sizes, then every
+// pointer non-null, images and the bias vector 16-byte aligned, float32 arrays 4-byte aligned
+int check_rppo_train(const char* fn, int64_t n_rows, int32_t latent, int32_t out_dim, std::initializer_list<const void*> img,
+                     std::initializer_list<const void*> f32)
+{
+    if (n_rows < 1 || n_rows > INT32_MAX) return fail(EVG_E_ARG, "%s: n_rows %lld outside 1..2^31-1", fn, (long long)n_rows);
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
+    if (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD) return fail(EVG_E_ARG, "%s: out_dim %d outside %d..%d", fn, out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
+    for (const void* p : img) {
+        if (!p) return fail(EVG_E_ARG, "%s: null image or bias vector", fn);
+        if ((uintptr_t)p % 16) return fail(EVG_E_ARG, "%s: images and the bias vector must be 16-byte aligned", fn);
+    }
+    for (const void* p : f32) {
+        if (!p) return fail(EVG_E_ARG, "%s: null float32 array", fn);
+        if ((uintptr_t)p % 4) return fail(EVG_E_ARG, "%s: float32 arrays must be 4-byte aligned", fn);
+    }
+    return EVG_OK;
+}
+
+}  // namespace
+
+int evg_rppo_train_pack(EvgSim* sim, const float* d_w3, const float* d_b3, const float* d_w_ih, const float* d_b_ih, const float* d_w_hh,
+                        const float* d_b_hh, int32_t latent, int32_t out_dim, void* d_wi_img, void* d_wh_img, void* d_wht_img, void* d_w3_img,
+                        float* d_bias, void* stream)
+{
+    int rc = check_rppo_train("evg_rppo_train_pack", 1, latent, out_dim, {d_wi_img, d_wh_img, d_wht_img, d_w3_img, d_bias},
+                              {d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh});
+    if (rc || (rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_pack_rppo_train(d_w3, d_b3, d_w_ih, d_b_ih, d_w_hh, d_b_hh, latent, out_dim, d_wi_img, d_wh_img, d_wht_img, d_w3_img,
+                                                d_bias, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_rppo_train_forward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t out_dim, const float* d_x, const float* d_h0, const void* d_wi_img,
+                           const void* d_wh_img, const void* d_w3_img, const float* d_bias, float* d_z, float* d_h, void* stream)
+{
+    int rc = check_rppo_train("evg_rppo_train_forward", n_rows, latent, out_dim, {d_wi_img, d_wh_img, d_w3_img, d_bias}, {d_x, d_h0, d_z, d_h});
+    if (rc || (rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_rppo_train_forward(n_rows, latent, out_dim, d_x, d_h0, d_wi_img, d_wh_img, d_w3_img, d_bias, d_z, d_h, sim->sm_count,
+                                                   (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_rppo_train_kernel<forward> launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_rppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t out_dim, const float* d_x, const float* d_h0, const float* d_h,
+                            const void* d_wi_img, const void* d_wh_img, const void* d_wht_img, const float* d_bias, float* d_g, float* d_dgh,
+                            float* d_s, void* stream)
+{
+    int rc = check_rppo_train("evg_rppo_train_backward", n_rows, latent, out_dim, {d_wi_img, d_wh_img, d_wht_img, d_bias},
+                              {d_x, d_h0, d_h, d_g, d_dgh, d_s});
+    if (rc || (rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_rppo_train_backward(n_rows, latent, out_dim, d_x, d_h0, d_h, d_wi_img, d_wh_img, d_wht_img, d_bias, d_g, d_dgh, d_s,
+                                                    sim->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_rppo_train_kernel<backward> launch");
     sim->launches += 1;
     return EVG_OK;
 }

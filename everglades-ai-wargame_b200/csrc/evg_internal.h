@@ -186,7 +186,15 @@ cudaError_t launch_ppo_loss(int64_t n_rows, int n_dist, int n, const float* z, c
                             float lo, float hi, float* surr, float* ent, float* logp, float* ratio, int sm_count, cudaStream_t stream);
 cudaError_t launch_ppo_loss_grad(int64_t n_rows, int n_dist, int n, const float* z, const int64_t* idx, const float* adv, const float* ratio,
                                  float lo, float hi, const float* g_surr, const float* g_ent, float* dz, int sm_count, cudaStream_t stream);
+// the recurrent actor's GRU and action layer for the update, forward and backward (evg_rppo_train.cu)
+cudaError_t launch_rppo_train_forward(int64_t n_rows, int latent, int out_dim, const float* x, const float* h0, const void* wi_img,
+                                      const void* wh_img, const void* w3_img, const float* bias, float* z, float* h, int sm_count,
+                                      cudaStream_t stream);
+cudaError_t launch_rppo_train_backward(int64_t n_rows, int latent, int out_dim, const float* x, const float* h0, const float* h,
+                                       const void* wi_img, const void* wh_img, const void* wht_img, const float* bias, float* g,
+                                       float* dgh, float* s, int sm_count, cudaStream_t stream);
 // the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
+cudaError_t set_rppo_train_smem();
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();
 cudaError_t set_policy_rppo_smem();
@@ -199,6 +207,10 @@ cudaError_t launch_pack_ppo(int in_dim, const float* w1, const float* b1, const 
                             const float* b3, const float* w_ih, const float* b_ih, const float* w_hh, const float* b_hh, int latent,
                             int out_dim, void* w1_img, void* w2_img, void* wi_img, void* wh_img, void* w3_img, float* bias,
                             cudaStream_t stream);
+// the recurrent actor's training images (evg_rppo_train_forward / _backward's)
+cudaError_t launch_pack_rppo_train(const float* w3, const float* b3, const float* w_ih, const float* b_ih, const float* w_hh,
+                                   const float* b_hh, int latent, int out_dim, void* wi_img, void* wh_img, void* wht_img, void* w3_img,
+                                   float* bias, cudaStream_t stream);
 cudaError_t launch_pack_value(int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
                               const float* b3, int latent, void* w1_img, void* w2_img, void* w3_img, float* bias, cudaStream_t stream);
 cudaError_t launch_obs_to_i16(const float* obs, int16_t* out, int64_t n_values, cudaStream_t stream);

@@ -25,7 +25,7 @@ namespace evg {
 namespace {
 
 constexpr int kPackThreads = 256;
-constexpr int kPackMaxBlocks = 10;  // the recurrent actor: 5 images and 5 bias vectors
+constexpr int kPackMaxBlocks = 10;  // the recurrent actor: 5 images and 5 bias vectors (its training images: 4 and 3)
 
 // Element (r, k) of piece p is source element (gr, gk) = (p * row_step + r, p * col_step + k):
 //     r >= valid_rows                          -> 0 (a GRU gate's rows past L, which belong to the next gate)
@@ -33,12 +33,14 @@ constexpr int kPackMaxBlocks = 10;  // the recurrent actor: 5 images and 5 bias 
 //     gk == bias_col and gr < src_rows         -> bias[gr]     (DQN: b1 as input column obs_len, b2 as hidden unit `hidden`)
 //     gk == bias_col and gr == one_row         -> 1            (DQN: the hidden unit that is relu(1) = 1)
 //     otherwise                                -> 0
+// A transposed block (the recurrent actor's training images) holds element (k, r) of that rule at (r, k).
 // An fp32 vector is a [rows x 1] column with src_cols = 1.
 struct PackBlock {
     void* dst;
     const float* src;
     const float* bias;
     int32_t is_vec;  // 0: bf16 images of [rows x cols] (cols a multiple of 64), 1: fp32 segments of `rows` values
+    int32_t transposed;
     int32_t rows, cols, pieces;
     int32_t row_step, col_step, valid_rows;
     int32_t src_rows, src_cols, bias_col, one_row;
@@ -52,6 +54,11 @@ struct PackArgs {
 
 __device__ __forceinline__ float pack_src(const PackBlock& b, int p, int r, int k)
 {
+    if (b.transposed) {
+        const int t = r;
+        r = k;
+        k = t;
+    }
     if (r >= b.valid_rows) return 0.f;
     const int gr = p * b.row_step + r, gk = p * b.col_step + k;
     if (gr < b.src_rows && gk < b.src_cols) return b.src[gr * b.src_cols + gk];
@@ -182,6 +189,24 @@ cudaError_t launch_pack_ppo(int in_dim, const float* w1, const float* b1, const 
         a.b[9] = gates(vec(gb + 3 * L, b_hh, L, 3 * latent), latent);
         a.n_blocks = 10;
     }
+    return launch(a, stream);
+}
+
+cudaError_t launch_pack_rppo_train(const float* w3, const float* b3, const float* w_ih, const float* b_ih, const float* w_hh,
+                                   const float* b_hh, int latent, int out_dim, void* wi_img, void* wh_img, void* wht_img, void* w3_img,
+                                   float* bias, cudaStream_t stream)
+{
+    const int lp = (latent + 15) / 16 * 16, ka = (latent + 63) / 64 * 64, L = EVG_PPO_MAX_LATENT;
+    PackArgs a{};
+    a.b[0] = gates(image(wi_img, w_ih, lp, ka, 3 * latent, latent), latent);
+    a.b[1] = gates(image(wh_img, w_hh, lp, ka, 3 * latent, latent), latent);
+    a.b[2] = gates(image(wht_img, w_hh, lp, ka, 3 * latent, latent), latent);  // gate g's W_hg^T: (j, i) = w_hh[g L + i][j]
+    a.b[2].transposed = 1;
+    a.b[3] = image(w3_img, w3, EVG_PPO_OUT_PAD, ka, out_dim, latent);
+    a.b[4] = vec(bias, b3, EVG_PPO_OUT_PAD, out_dim);
+    a.b[5] = gates(vec(bias + EVG_PPO_OUT_PAD, b_ih, L, 3 * latent), latent);
+    a.b[6] = gates(vec(bias + EVG_PPO_OUT_PAD + 3 * L, b_hh, L, 3 * latent), latent);
+    a.n_blocks = 7;
     return launch(a, stream);
 }
 

@@ -32,6 +32,7 @@
 // u_k = (w[k] >> 8) * 2^-24 — the uniforms of evg_policy_ppo.  T = fp32 sum of p_k in ascending j, x = u_k * T, the draw
 // is the first j whose ascending fp32 prefix exceeds x (none, through rounding: the last j): tests/ppo_sampling.py's
 // ppo_sample(probs_k, [u_k]).
+#include "evg_gru.cuh"
 #include "evg_internal.h"
 #include "evg_tcgen05.cuh"
 
@@ -73,8 +74,6 @@ struct RppoArgs : ActorArgs {
     float* hidden_in;  // [rows][L]: the state each row started this call from (null: not written)
     int latent, ka, nrb;
 };
-
-__device__ __forceinline__ float sigmoid(float v) { return __frcp_rn(1.f + expf(-v)); }  // = 1 / (1 + e^-v), correctly rounded
 
 // kWire: the observations are wire rows (ws), else float32
 // kExtra: a.logp / a.hidden_in may be written (the instantiation without them is the kernel as it was before they
@@ -303,10 +302,9 @@ __global__ void __launch_bounds__(kCtaThreads, 1) evg_policy_rppo_kernel(const _
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
                             const int j = j0 + 4 * g + e;
-                            const float rr = sigmoid(__uint_as_float(vr[e]) + sb[kBr + j]);
-                            const float zz = sigmoid(__uint_as_float(vz[e]) + sb[kBz + j]);
-                            const float nn = tanhf((__uint_as_float(vn[e]) + sb[kBin + j]) + rr * (__uint_as_float(vh[e]) + sb[kBhn + j]));
-                            hv[4 * g + e] = (1.f - zz) * nn + zz * hv[4 * g + e];
+                            const GruGates q = gru_gates(__uint_as_float(vr[e]), __uint_as_float(vz[e]), __uint_as_float(vn[e]),
+                                                         __uint_as_float(vh[e]), sb[kBr + j], sb[kBz + j], sb[kBin + j], sb[kBhn + j]);
+                            hv[4 * g + e] = gru_state(q, hv[4 * g + e]);
                         }
                     }
                     h_keep(i, hv);

@@ -445,6 +445,7 @@ class FusedRPPO:
         self.probs = torch.empty(shape + (_capi.MAX_ACTIONS, self.out_dim), dtype=torch.float32, device=dev)
         self.logp = torch.empty(shape + (_capi.MAX_ACTIONS,), dtype=torch.float32, device=dev)
         self.hidden_in = torch.zeros_like(self.hidden)
+        self._t = None
 
     def refresh(self, actor=None):
         """Re-pack the weight images and the bias vector in place from `actor` (default: the module this wrapper was built
@@ -457,6 +458,60 @@ class FusedRPPO:
         i1, i2, ii, ih, i3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
         _capi.check(env._lib.evg_pack_rppo(env._h, w1, b1, w2, b2, w3, b3, wi, bi, wh, bh, L, o, i1, i2, ii, ih, i3, bias,
                                            env._stream()))
+
+    def evaluate(self, x, hidden_in):
+        """The GRU's 7 steps and action_layer[0] for a PPO update, on the tensor cores (evg_rppo_train_forward / _backward):
+        x float32 [R, L], the action head's output, and hidden_in float32 [R, L], the state each stored row started from
+        (the acting call's .hidden_in) -> z float32 [R, 7, out], step k's output of action_layer[0] before its Tanh, as
+        env.ppo_loss takes it with K = 7.  Differentiable with respect to x and the wrapped actor's weight_ih_l0,
+        weight_hh_l0, bias_ih_l0, bias_hh_l0, action_layer[0].weight and .bias (autograd accumulates their .grad); no
+        gradient flows to hidden_in.  The arithmetic is the acting kernel's (bf16 operands, fp32 accumulation and gates),
+        so from the same x and state h_7 is what an acting call leaves in .hidden.  The actor's current parameters are
+        packed into images of this call's own (one device launch); the acting images stay as they are until refresh().
+        The backward's weight-gradient reductions are float32 torch.matmul calls on what the kernel writes (torch's
+        default precision: TF32 is used only where the caller enabled it).  ValueError, before any launch, for a tensor
+        of the wrong dtype, shape, device or contiguity; R = 0 gives an empty tensor.  No host synchronisation."""
+        import torch
+        env, L, o = self.env, self.latent, self.out_dim
+        for name, t in (("x", x), ("hidden_in", hidden_in)):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or not t.is_contiguous() or t.device != env.device \
+                    or t.dim() != 2 or t.shape[1] != L:
+                raise ValueError("%s must be a contiguous float32 tensor [R, %d] on %s, got %s" % (name, L, env.device, _describe(t)))
+        if hidden_in.shape != x.shape:
+            raise ValueError("hidden_in has %d rows, x has %d" % (hidden_in.shape[0], x.shape[0]))
+        params = _rppo_params(self._net)
+        for i, (t, shape) in enumerate(zip(params, [(L, env.obs_len), (L,), (L, L), (L,), (3 * L, L), (3 * L,), (3 * L, L), (3 * L,), (o, L), (o,)])):
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != env.device or tuple(t.shape) != shape:
+                raise ValueError("parameter %d must be a contiguous float32 tensor of shape %s on %s, got %s" % (i, shape, env.device, _describe(t)))
+        if x.shape[0] == 0:
+            return torch.empty((0, _capi.MAX_ACTIONS, o), dtype=torch.float32, device=env.device)
+        return _rppo_train_function().apply(x, hidden_in, self, *params[4:])
+
+    def _train_images(self):
+        """The training images (wi, wh, wht, w3 uint8, bias float32), allocated on first use."""
+        import torch
+        if self._t is None:
+            lp, ka = -(-self.latent // 16) * 16, -(-self.latent // ATOM) * ATOM
+            dev = self.env.device
+            gate_bytes = 3 * (ka // ATOM) * lp * 128
+            self._t = [torch.empty(gate_bytes, dtype=torch.uint8, device=dev) for _ in range(3)]
+            self._t.append(torch.empty((ka // ATOM) * PPO_OUT_PAD * 128, dtype=torch.uint8, device=dev))
+            self._t.append(torch.empty(PPO_OUT_PAD + 6 * PPO_MAX_LATENT, dtype=torch.float32, device=dev))
+        return self._t
+
+    def _train_forward(self, x, h0, w_ih, b_ih, w_hh, b_hh, w3, b3, z, h):
+        env, p = self.env, (lambda t: C.c_void_p(t.data_ptr()))
+        wi, wh, wht, i3, bias = (p(t) for t in self._train_images())
+        _capi.check(env._lib.evg_rppo_train_pack(env._h, p(w3), p(b3), p(w_ih), p(b_ih), p(w_hh), p(b_hh), self.latent, self.out_dim,
+                                                 wi, wh, wht, i3, bias, env._stream()))
+        _capi.check(env._lib.evg_rppo_train_forward(env._h, x.shape[0], self.latent, self.out_dim, p(x), p(h0), wi, wh, i3, bias, p(z), p(h),
+                                                    env._stream()))
+
+    def _train_backward(self, x, h0, h, g, dgh, s):
+        env, p = self.env, (lambda t: C.c_void_p(t.data_ptr()))
+        wi, wh, wht, _, bias = (p(t) for t in self._train_images())
+        _capi.check(env._lib.evg_rppo_train_backward(env._h, x.shape[0], self.latent, self.out_dim, p(x), p(h0), p(h), wi, wh, wht, bias,
+                                                     p(g), p(dgh), p(s), env._stream()))
 
     def __call__(self, want_probs=False, obs_format="f32", want_logp=False, want_hidden_in=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); steps .hidden, fills .idx (int64 [N, 2, 7] or [N, 7]) and, with
@@ -475,6 +530,48 @@ class FusedRPPO:
                                                   C.c_void_p(self.idx.data_ptr()), _ptr(self.probs, want_probs), _ptr(self.logp, want_logp),
                                                   env._stream()))
         return env._actions
+
+
+_RPPO_TRAIN = None
+
+
+def _rppo_train_function():
+    """The torch.autograd.Function of FusedRPPO.evaluate (defined on first use: torch is imported lazily)."""
+    global _RPPO_TRAIN
+    if _RPPO_TRAIN is None:
+        import torch
+
+        def bf16(t):
+            return t.to(torch.bfloat16).to(torch.float32)
+
+        class RPPOTrain(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, x, hidden_in, fused, w_ih, b_ih, w_hh, b_hh, w3, b3):
+                R, L = x.shape
+                z = torch.empty((R, _capi.MAX_ACTIONS, fused.out_dim), dtype=torch.float32, device=x.device)
+                h = torch.empty((R, _capi.MAX_ACTIONS, L), dtype=torch.float32, device=x.device)
+                fused._train_forward(x, hidden_in, w_ih, b_ih, w_hh, b_hh, w3, b3, z, h)
+                ctx.save_for_backward(x, hidden_in, h, w_ih, w_hh, w3)
+                ctx.fused = fused
+                return z
+
+            @staticmethod
+            def backward(ctx, dz):
+                x, h0, h, w_ih, w_hh, w3 = ctx.saved_tensors
+                R, L = x.shape
+                K, o = _capi.MAX_ACTIONS, w3.shape[0]
+                dz = dz.to(torch.float32).contiguous().view(R * K, o)
+                g = (dz @ bf16(w3)).view(R, K, L)  # W3^T dz_k; the kernel adds the carries in place
+                dgh = torch.empty((R, K, 3 * L), dtype=torch.float32, device=x.device)
+                s = torch.empty((R, 3 * L), dtype=torch.float32, device=x.device)
+                ctx.fused._train_backward(x, h0, h, g, dgh, s)
+                dgh = dgh.view(R * K, 3 * L)
+                h_prev = bf16(torch.cat([h0.unsqueeze(1), h[:, :K - 1]], dim=1)).view(R * K, L)
+                return (s @ bf16(w_ih), None, None, s.t() @ bf16(x), s.sum(0), dgh.t() @ h_prev, dgh.sum(0),
+                        dz.t() @ bf16(h).view(R * K, L), dz.sum(0))
+
+        _RPPO_TRAIN = RPPOTrain
+    return _RPPO_TRAIN
 
 
 def _value_params(net):

@@ -515,6 +515,45 @@ int evg_ppo_loss(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions,
 int evg_ppo_loss_grad(EvgSim* sim, int64_t n_rows, int32_t n_dist, int32_t n_actions, const float* d_z, const int64_t* d_idx, const float* d_adv,
                       const float* d_ratio, float clip, const float* d_g_surr, const float* d_g_ent, float* d_dz, void* stream);
 
+/* The recurrent actor's GRU and action layer for a PPO update, forward and backward, on the tensor cores
+ * (csrc/evg_rppo_train.cu; DESIGN.md §4.13).  Per row of B = n_rows, L = latent (1..EVG_PPO_MAX_LATENT), out = out_dim
+ * (7..EVG_PPO_OUT_PAD): x float32 [L] is the head's output (d_x [B][L]) and h_0 float32 [L] the stored starting state
+ * (d_h0 [B][L], evg_policy_rppo_logp's d_hidden_in).  For k = 1..7, gates r, z, n in torch.nn.GRU's order:
+ *     r = sigmoid(W_ir x + W_hr h + (b_ir + b_hr)),   u = sigmoid(W_iz x + W_hz h + (b_iz + b_hz)),   c = W_hn h + b_hn
+ *     n = tanh(W_in x + b_in + r c),   h_k = (1 - u) n + u h_{k-1},   z_k = W3 bf16(h_k) + b3
+ * z_k is action_layer[0]'s output before its Tanh: evg_ppo_loss's z with K = 7.  The arithmetic is evg_policy_rppo's:
+ * bf16 operands (x, h as the MMA operand, the weights), fp32 accumulation, X W_ir^T and H W_hr^T in one accumulator then
+ * the pre-summed bias, the same sigmoid (1 / (1 + expf(-v)) correctly rounded) and tanhf, h kept in fp32.  So from the
+ * head output and state of an acting call, h_7 is what that call leaves in d_hidden.
+ *   evg_rppo_train_pack: the images both read, packed on the device from the float32 parameters in torch's layouts
+ *       (d_w3 [out][L], d_b3 [out], d_w_ih / d_w_hh [3L][L], d_b_ih / d_b_hh [3L]), every byte written:
+ *         d_wi_img, d_wh_img: weight_ih_l0 / weight_hh_l0 exactly as for evg_policy_rppo (three [Lp x Ka] blocks)
+ *         d_wht_img: gate g's W_hg^T, three [Lp x Ka] blocks the same size: element (j, i) of block g = w_hh[g L + i][j]
+ *         d_w3_img: exactly as for evg_policy_rppo
+ *         d_bias: float32 [EVG_PPO_OUT_PAD + 6 * EVG_PPO_MAX_LATENT] = b3, then b_ih gate g at EVG_PPO_OUT_PAD + g * 256
+ *                 and b_hh gate g at EVG_PPO_OUT_PAD + (3 + g) * 256, zero padded.
+ *   evg_rppo_train_forward: d_z float32 [B][7][out] and d_h float32 [B][7][L] = h_1..h_7.
+ *   evg_rppo_train_backward, from d_h (the forward's) and d_g float32 [B][7][L], which holds W3^T dz_k on entry
+ *       (dz = dL/dz; the caller's fp32 product with bf16(W3)) and g_k on return, recomputing r, u, n, c bit for bit:
+ *     g_k = W3^T dz_k + carry_{k+1} (carry_8 = 0);  dn = g (1 - u),  da_n = dn (1 - n^2),  da_u = g (h_{k-1} - n) u (1 - u),
+ *     da_r = da_n c r (1 - r);  dgi_k = [da_r, da_u, da_n],  dgh_k = [da_r, da_u, da_n r]
+ *     carry_k = fl(g u) + bf16(W_hh)^T bf16(dgh_k)  (tensor cores, bf16(dgh_k) the MMA operand), added as
+ *     d_g[k-1] = fl(fl(W3^T dz_{k-1} + g_k u_k) + W_hh^T dgh_k)
+ *     d_dgh float32 [B][7][3L] = dgh_1..dgh_7;  d_s float32 [B][3L] = sum_k dgi_k (k = 7 down to 1).
+ *   The parameter gradients are the reductions dW_ih = S^T bf16(x), dW_hh = sum_{rows,k} dgh_k^T bf16(h_{k-1}),
+ *   dW3 = sum dz_k^T bf16(h_k), the biases' the column sums, and dx = bf16(W_ih)^T S; no gradient flows to h_0.
+ * Images and d_bias 16-byte aligned, float32 arrays 4-byte aligned.  One launch on `stream` each, no allocation, no
+ * synchronisation.  EVG_E_ARG, checked before the handle, for n_rows outside 1..2^31-1 (the pack takes none), latent or
+ * out_dim out of range, a NULL pointer and a misaligned one. */
+int evg_rppo_train_pack(EvgSim* sim, const float* d_w3, const float* d_b3, const float* d_w_ih, const float* d_b_ih, const float* d_w_hh,
+                        const float* d_b_hh, int32_t latent, int32_t out_dim, void* d_wi_img, void* d_wh_img, void* d_wht_img, void* d_w3_img,
+                        float* d_bias, void* stream);
+int evg_rppo_train_forward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t out_dim, const float* d_x, const float* d_h0, const void* d_wi_img,
+                           const void* d_wh_img, const void* d_w3_img, const float* d_bias, float* d_z, float* d_h, void* stream);
+int evg_rppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t out_dim, const float* d_x, const float* d_h0, const float* d_h,
+                            const void* d_wi_img, const void* d_wh_img, const void* d_wht_img, const float* d_bias, float* d_g, float* d_dgh,
+                            float* d_s, void* stream);
+
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
  * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
