@@ -1,5 +1,6 @@
 """CPU checks of the recurrent actor's update operation: its analytic backward against torch float64 autograd and central
-differences, the float32 statement within the derived step bound, the transposed image layout, and the C ABI's refusals."""
+differences, the float32 forward within the derived step bound, the float32 backward within the derived backward step
+bound and each of its plausible defects outside it, the transposed image layout, and the C ABI's refusals."""
 import ctypes as C
 
 import numpy as np
@@ -151,3 +152,52 @@ def test_abi_refuses_bad_arguments_without_a_device(lib):
                 assert rc == -1 and "n_rows" in msg, (call.__name__, B, msg)
         rc, msg = call()
         assert rc == -1 and "null EvgSim handle" in msg, (call.__name__, msg)
+
+
+def backward_case(L, R=64, seed=None):
+    """A random float network, its float32 forward and an entry value G of d_g: (x, h0, h, w, wb, G)."""
+    rng = np.random.default_rng(L if seed is None else seed)
+    w = [a.astype(np.float32) for a in weights(rng, L, 132)]
+    wb = [rt.bf16(w[0]), w[1], rt.bf16(w[2]), w[3], rt.bf16(w[4]), w[5]]
+    x, h0 = rng.uniform(-1, 1, (R, L)).astype(np.float32), rng.uniform(-1, 1, (R, L)).astype(np.float32)
+    _, h = rt.forward32(x, h0, w)
+    G = rng.normal(size=(R, 7, L)).astype(np.float32)
+    return x, h0, h, w, wb, G
+
+
+@pytest.mark.parametrize("L", [1, 16, 17, 128, 129, 248])
+def test_float32_backward_within_the_backward_step_bound(L):
+    """backward32 (the kernel's statement in numpy's summation order) keeps dgh_k, g_{k-1} and S of every step within
+    under half of backward_step_bound, leaves g_7 as it came in, and the bound is far below a bf16-sized error."""
+    x, h0, h, w, wb, G = backward_case(L)
+    g, dgh, s = rt.backward32(x, h0, h, w, G)
+    assert np.array_equal(g[:, 6], G[:, 6])
+    worst = rt.worst(rt.backward_ratios(x, h0, h, wb, G, g, dgh, s))
+    assert all(v[0] < 0.5 for v in worst.values()), worst
+    b = rt.backward_step_bound(x, h[:, 5], wb, g[:, 6], G[:, 5], dgh[:, 6])
+    assert b.dgh_b.max() < 2.0 ** -12 * np.abs(b.dgh).max() and b.g_b.max() < 2.0 ** -12 * np.abs(b.g).max()
+
+
+@pytest.mark.parametrize("L", [17, 129, 248])
+def test_each_backward_mutant_leaves_the_bound(L):
+    """Every plausible defect of BACKWARD_MUTANTS takes every row out of the bound (share 1.0), in the quantity it
+    corrupts: dgh for the gradient formulas, g_{k-1} for the carry, S for its sum.  The carry without its last group of
+    atoms is only a defect for L > 64 (one group below); nothing is claimed for it at L = 17."""
+    x, h0, h, w, wb, G = backward_case(L)
+    where = {"carry_g": "g", "carry_g_1mu": "g", "carry_untransposed": "g", "carry_last_group_dropped": "g", "dgh_rz": "g",
+             "s_sums_dgh": "S"}
+    for mutant in rt.BACKWARD_MUTANTS:
+        if mutant == "carry_last_group_dropped" and L <= 64:
+            continue
+        g, dgh, s = rt.backward32(x, h0, h, w, G, mutant)
+        ratio = rt.backward_ratios(x, h0, h, wb, G, g, dgh, s)[where.get(mutant, "dgh")]
+        caught = ~(ratio.reshape(len(x), -1) <= 1).all(1)
+        assert caught.mean() == 1.0, (mutant, caught.mean())
+
+
+def test_gate_bounds_are_the_step_bounds():
+    """step_bound is gate_bounds' e_n and e_u carried through h' = (1 - u) n + u h, and e_c holds c's one dot product."""
+    x, h0, h, w, wb, G = backward_case(33, R=8)
+    e_r, e_u, e_n, e_c = rt.gate_bounds(x, h0, wb)
+    assert np.array_equal(rt.step_bound(x, h0, wb), e_n + e_u * (1 + np.abs(h0)) + 4 * rt.U32 * (1 + np.abs(h0)))
+    assert (e_r >= 8 * rt.U32).all() and (e_u >= 8 * rt.U32).all() and (e_c > 0).all()
