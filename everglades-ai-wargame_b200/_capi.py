@@ -27,6 +27,7 @@ WIRE_NODE0 = 4
 MLP_IN_PAD, MLP_CHUNK, MLP_OUT_PAD = 128, 192, 144
 PPO_IN_PAD, PPO_MAX_LATENT, PPO_OUT_PAD = 128, 256, 144
 VALUE_OUT_PAD = 16
+PPO_TRAIN_ACTOR, PPO_TRAIN_CRITIC, PPO_TRAIN_HEAD = 0, 1, 2
 BIND_RECORDS, BIND_HEALTH, BIND_STATS, BIND_TABLES, BIND_AGENTS, BIND_COUNT = 0, 1, 2, 3, 4, 5
 
 _N1 = MAX_NODES + 1
@@ -186,6 +187,9 @@ SYMBOLS = [
     ("evg_rppo_train_pack", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
     ("evg_rppo_train_forward", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     ("evg_rppo_train_backward", C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_ppo_train_pack", C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    ("evg_ppo_train_forward", C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P]),
+    ("evg_ppo_train_backward", C.c_int, [_P, C.c_int64, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     ("evg_pack_mlp", C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     ("evg_pack_ppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     ("evg_pack_rppo", C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),

@@ -367,7 +367,7 @@ int evg_create(const EvgConfig* cfg, int64_t n_envs, uint64_t seed, int64_t env_
     // the shared-memory opt-ins are per device: made on the simulator's, for the step and the policy kernels
     if ((e = evg::set_step_smem(s->smem)) != cudaSuccess || (e = evg::set_policy_mlp_smem()) != cudaSuccess || (e = evg::set_policy_ppo_smem()) != cudaSuccess ||
         (e = evg::set_policy_rppo_smem()) != cudaSuccess || (e = evg::set_policy_value_smem()) != cudaSuccess ||
-        (e = evg::set_rppo_train_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
+        (e = evg::set_rppo_train_smem()) != cudaSuccess || (e = evg::set_ppo_train_smem()) != cudaSuccess) { delete s; return cuda_fail(e, "cudaFuncSetAttribute(max dynamic smem)"); }
     int per_sm = 0;
     if ((e = evg::step_occupancy(t, s->smem, &per_sm)) != cudaSuccess || per_sm < 1) { delete s; return cuda_fail(e, "occupancy query"); }
     // persistent CTAs: a whole number of resident waves, never more CTAs than matches need
@@ -1219,6 +1219,93 @@ int evg_rppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t
     cudaError_t e = evg::launch_rppo_train_backward(n_rows, latent, out_dim, d_x, d_h0, d_h, d_wi_img, d_wh_img, d_wht_img, d_bias, d_g, d_dgh, d_s,
                                                     sim->sm_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "evg_rppo_train_kernel<backward> launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+namespace {
+
+// evg_ppo_train_*'s shared argument checks, before the handle's: the network and its widths, then every pointer
+// non-null, images and the bias vector 16-byte aligned, float32 arrays 4-byte aligned
+int check_ppo_train(const char* fn, int32_t net, int32_t latent, int32_t out_dim, std::initializer_list<const void*> img,
+                    std::initializer_list<const void*> f32)
+{
+    if (net != EVG_PPO_TRAIN_ACTOR && net != EVG_PPO_TRAIN_CRITIC && net != EVG_PPO_TRAIN_HEAD) return fail(EVG_E_ARG, "%s: unknown network %d", fn, net);
+    if (latent < 1 || latent > EVG_PPO_MAX_LATENT) return fail(EVG_E_ARG, "%s: latent %d outside 1..%d", fn, latent, EVG_PPO_MAX_LATENT);
+    if (net == EVG_PPO_TRAIN_ACTOR && (out_dim < EVG_MAX_ACTIONS || out_dim > EVG_PPO_OUT_PAD))
+        return fail(EVG_E_ARG, "%s: out_dim %d outside %d..%d", fn, out_dim, EVG_MAX_ACTIONS, EVG_PPO_OUT_PAD);
+    if (net == EVG_PPO_TRAIN_CRITIC && out_dim != 1) return fail(EVG_E_ARG, "%s: the critic's out_dim %d must be 1", fn, out_dim);
+    if (net == EVG_PPO_TRAIN_HEAD && out_dim != latent) return fail(EVG_E_ARG, "%s: the head's out_dim %d must be latent %d", fn, out_dim, latent);
+    for (const void* p : img) {
+        if (!p) return fail(EVG_E_ARG, "%s: null image or bias vector", fn);
+        if ((uintptr_t)p % 16) return fail(EVG_E_ARG, "%s: images and the bias vector must be 16-byte aligned", fn);
+    }
+    for (const void* p : f32) {
+        if (!p) return fail(EVG_E_ARG, "%s: null float32 array", fn);
+        if ((uintptr_t)p % 4) return fail(EVG_E_ARG, "%s: float32 arrays must be 4-byte aligned", fn);
+    }
+    return EVG_OK;
+}
+
+int check_obs_len(const char* fn, const EvgSim* sim)
+{
+    if (sim->layout.obs_len >= EVG_PPO_IN_PAD)
+        return fail(EVG_E_ARG, "%s: observations of %d values exceed the %d the kernel is tiled for", fn, sim->layout.obs_len, EVG_PPO_IN_PAD - 1);
+    return EVG_OK;
+}
+
+}  // namespace
+
+int evg_ppo_train_pack(EvgSim* sim, int32_t net, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                       const float* d_b3, int32_t latent, int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_w3_img, void* d_w2t_img,
+                       float* d_bias, void* stream)
+{
+    const bool last = net != EVG_PPO_TRAIN_HEAD;
+    int rc = check_ppo_train("evg_ppo_train_pack", net, latent, out_dim, {d_w1_img, d_w2_img, last ? d_w3_img : d_w1_img, d_w2t_img, d_bias},
+                             {d_w1, d_b1, d_w2, d_b2, last ? d_w3 : d_w1, last ? d_b3 : d_b1});
+    if (rc || (rc = check_sim(sim, false)) || (rc = check_obs_len("evg_ppo_train_pack", sim))) return rc;
+    cudaError_t e = evg::launch_pack_ppo_train(net, sim->layout.obs_len, d_w1, d_b1, d_w2, d_b2, d_w3, d_b3, latent, out_dim, d_w1_img, d_w2_img,
+                                               d_w3_img, d_w2t_img, d_bias, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_policy_pack_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_ppo_train_forward(EvgSim* sim, int32_t net, int32_t format, const void* d_obs, int64_t n_matches, int32_t player, int32_t latent,
+                          int32_t out_dim, const void* d_w1_img, const void* d_w2_img, const void* d_w3_img, const float* d_bias, float* d_out,
+                          float* d_h1, float* d_h2, void* stream)
+{
+    const char* fn = "evg_ppo_train_forward";
+    const bool last = net != EVG_PPO_TRAIN_HEAD;
+    int rc = check_ppo_train(fn, net, latent, out_dim, {d_w1_img, d_w2_img, last ? d_w3_img : d_w1_img, d_bias},
+                             {d_h1, d_h2, last ? d_out : d_h1});
+    if (rc) return rc;
+    if (player < -1 || player > 1) return fail(EVG_E_ARG, "%s: player %d outside -1..1", fn, player);
+    const int64_t rows = n_matches * (player < 0 ? 2 : 1);
+    if (n_matches < 1 || rows > INT32_MAX) return fail(EVG_E_ARG, "%s: n_matches %lld gives rows outside 1..2^31-1", fn, (long long)n_matches);
+    if (format != EVG_OBS_F32 && format != EVG_OBS_WIRE) return fail(EVG_E_ARG, "%s: observation format %d (EVG_OBS_F32 or EVG_OBS_WIRE)", fn, format);
+    if (!d_obs) return fail(EVG_E_ARG, "%s: null observations", fn);
+    if ((uintptr_t)d_obs % (format == EVG_OBS_WIRE ? 16 : 4)) return fail(EVG_E_ARG, "%s: float32 observations must be 4-byte aligned, wire rows 16-byte", fn);
+    if ((rc = check_sim(sim, false)) || (rc = check_obs_len(fn, sim))) return rc;
+    evg::WireSrc ws;
+    bool wire;
+    if ((rc = policy_source(fn, sim, format, d_obs, &ws, &wire))) return rc;
+    cudaError_t e = evg::launch_ppo_train_forward(net, d_obs, n_matches, player, sim->layout.obs_len, latent, out_dim, d_w1_img, d_w2_img, d_w3_img,
+                                                  d_bias, d_out, d_h1, d_h2, sim->sm_count, (cudaStream_t)stream, wire ? &ws : nullptr);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_ppo_train_forward_kernel launch");
+    sim->launches += 1;
+    return EVG_OK;
+}
+
+int evg_ppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, const void* d_w2t_img, const float* d_g2, const float* d_h1,
+                           const float* d_h2, float* d_dd2, float* d_dd1, void* stream)
+{
+    const char* fn = "evg_ppo_train_backward";
+    if (n_rows < 1 || n_rows > INT32_MAX) return fail(EVG_E_ARG, "%s: n_rows %lld outside 1..2^31-1", fn, (long long)n_rows);
+    int rc = check_ppo_train(fn, EVG_PPO_TRAIN_HEAD, latent, latent, {d_w2t_img}, {d_g2, d_h1, d_h2, d_dd2, d_dd1});
+    if (rc || (rc = check_sim(sim, false))) return rc;
+    cudaError_t e = evg::launch_ppo_train_backward(n_rows, latent, d_w2t_img, d_g2, d_h1, d_h2, d_dd2, d_dd1, sim->sm_count, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(e, "evg_ppo_train_backward_kernel launch");
     sim->launches += 1;
     return EVG_OK;
 }

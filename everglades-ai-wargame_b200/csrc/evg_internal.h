@@ -193,7 +193,19 @@ cudaError_t launch_rppo_train_forward(int64_t n_rows, int latent, int out_dim, c
 cudaError_t launch_rppo_train_backward(int64_t n_rows, int latent, int out_dim, const float* x, const float* h0, const float* h,
                                        const void* wi_img, const void* wh_img, const void* wht_img, const float* bias, float* g,
                                        float* dgh, float* s, int sm_count, cudaStream_t stream);
+// PPO's feed-forward networks for the update, forward and backward (evg_ppo_train.cu); net = EVG_PPO_TRAIN_*
+cudaError_t launch_ppo_train_forward(int net, const void* obs, int64_t n_matches, int player, int in_dim, int latent, int out_dim,
+                                     const void* w1_img, const void* w2_img, const void* w3_img, const float* bias, float* out, float* h1,
+                                     float* h2, int sm_count, cudaStream_t stream, const WireSrc* wire);
+cudaError_t launch_ppo_train_backward(int64_t n_rows, int latent, const void* w2t_img, const float* g2, const float* h1, const float* h2,
+                                      float* dd2, float* dd1, int sm_count, cudaStream_t stream);
+// the float32 length of a network's packed bias vector: b1 | b2, then the actor's or the critic's b3
+inline int ppo_train_bias_floats(int net)
+{
+    return 2 * EVG_PPO_MAX_LATENT + (net == EVG_PPO_TRAIN_ACTOR ? EVG_PPO_OUT_PAD : net == EVG_PPO_TRAIN_CRITIC ? EVG_VALUE_OUT_PAD : 0);
+}
 // the policy kernels' opt-in to their dynamic shared memory, on the current device (the attribute is per device)
+cudaError_t set_ppo_train_smem();
 cudaError_t set_rppo_train_smem();
 cudaError_t set_policy_mlp_smem();
 cudaError_t set_policy_ppo_smem();
@@ -207,6 +219,10 @@ cudaError_t launch_pack_ppo(int in_dim, const float* w1, const float* b1, const 
                             const float* b3, const float* w_ih, const float* b_ih, const float* w_hh, const float* b_hh, int latent,
                             int out_dim, void* w1_img, void* w2_img, void* wi_img, void* wh_img, void* w3_img, float* bias,
                             cudaStream_t stream);
+// the feed-forward networks' training images (evg_ppo_train_forward / _backward's); w3 null for the head
+cudaError_t launch_pack_ppo_train(int net, int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
+                                  const float* b3, int latent, int out_dim, void* w1_img, void* w2_img, void* w3_img, void* w2t_img,
+                                  float* bias, cudaStream_t stream);
 // the recurrent actor's training images (evg_rppo_train_forward / _backward's)
 cudaError_t launch_pack_rppo_train(const float* w3, const float* b3, const float* w_ih, const float* b_ih, const float* w_hh,
                                    const float* b_hh, int latent, int out_dim, void* wi_img, void* wh_img, void* wht_img, void* w3_img,

@@ -25,7 +25,8 @@ namespace evg {
 namespace {
 
 constexpr int kPackThreads = 256;
-constexpr int kPackMaxBlocks = 10;  // the recurrent actor: 5 images and 5 bias vectors (its training images: 4 and 3)
+constexpr int kPackMaxBlocks = 10;  // the recurrent actor: 5 images and 5 bias vectors (its training images: 4 and 3; the
+                                    // feed-forward networks' training images: up to 4 and 3)
 
 // Element (r, k) of piece p is source element (gr, gk) = (p * row_step + r, p * col_step + k):
 //     r >= valid_rows                          -> 0 (a GRU gate's rows past L, which belong to the next gate)
@@ -207,6 +208,31 @@ cudaError_t launch_pack_rppo_train(const float* w3, const float* b3, const float
     a.b[5] = gates(vec(bias + EVG_PPO_OUT_PAD, b_ih, L, 3 * latent), latent);
     a.b[6] = gates(vec(bias + EVG_PPO_OUT_PAD + 3 * L, b_hh, L, 3 * latent), latent);
     a.n_blocks = 7;
+    return launch(a, stream);
+}
+
+cudaError_t launch_pack_ppo_train(int net, int in_dim, const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
+                                  const float* b3, int latent, int out_dim, void* w1_img, void* w2_img, void* w3_img, void* w2t_img,
+                                  float* bias, cudaStream_t stream)
+{
+    const int lp = (latent + 15) / 16 * 16, ka = (latent + 63) / 64 * 64, L = EVG_PPO_MAX_LATENT;
+    PackArgs a{};
+    a.b[0] = image(w1_img, w1, lp, EVG_PPO_IN_PAD, latent, in_dim);
+    a.b[1] = image(w2_img, w2, lp, ka, latent, latent);
+    a.b[2] = image(w2t_img, w2, lp, ka, latent, latent);  // W2^T: (j, i) = w2[i][j]
+    a.b[2].transposed = 1;
+    a.b[3] = vec(bias, b1, L, latent);
+    a.b[4] = vec(bias + L, b2, L, latent);
+    a.n_blocks = 5;
+    if (net == EVG_PPO_TRAIN_ACTOR) {
+        a.b[5] = image(w3_img, w3, EVG_PPO_OUT_PAD, ka, out_dim, latent);
+        a.b[6] = vec(bias + 2 * L, b3, EVG_PPO_OUT_PAD, out_dim);
+        a.n_blocks = 7;
+    } else if (net == EVG_PPO_TRAIN_CRITIC) {
+        a.b[5] = image(w3_img, w3, EVG_VALUE_OUT_PAD, ka, 1, latent);
+        a.b[6] = vec(bias + 2 * L, b3, EVG_VALUE_OUT_PAD, 1);
+        a.n_blocks = 7;
+    }
     return launch(a, stream);
 }
 

@@ -320,6 +320,18 @@ class FusedPPO:
         w1, w2, w3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
         _capi.check(env._lib.evg_pack_ppo(env._h, *src, L, o, w1, w2, w3, bias, env._stream()))
 
+    def evaluate(self, obs, obs_format="wire"):
+        """The actor for a PPO update, on the tensor cores (evg_ppo_train_forward / _backward): stored observations, wire
+        rows uint8 [M, row_bytes] ('wire') or float32 [M, 2, obs_len] ('f32'), -> z float32 [R, out], the output of the
+        actor's last Linear before its Tanh (what env.ppo_loss takes), R = 2M rows ordered like .idx / .logp for player -1
+        (row i = match i // 2, player i % 2), else M.  Differentiable with respect to the wrapped net's six parameters
+        (autograd accumulates their .grad).  The arithmetic and the MMAs are the acting kernel's, so with the parameters
+        the acting images were packed from, tanh(z) is what the acting call took its softmax of, bit for bit.  The net's
+        current parameters are packed into images of this call's own (one device launch); the acting images stay the
+        behaviour policy until refresh().  See _ff_evaluate for the backward and the ValueError checks."""
+        L, o = self.latent, self.out_dim
+        return _ff_evaluate(self, _capi.PPO_TRAIN_ACTOR, obs, obs_format, self.player, o, [(o, L), (o,)], self._params)
+
     def __call__(self, want_probs=False, obs_format="f32", want_logp=False):
         """Action rows int8 [N, 2, 7, 2] (env._actions); fills .idx (int64 [N, 2, 7] or [N, 7]) and, with want_probs,
         .probs (float32 [N, 2, out] or [N, out]).  With want_logp, .logp (float32 [N, 2, 7] or [N, 7]): draw k's
@@ -487,6 +499,16 @@ class FusedRPPO:
             return torch.empty((0, _capi.MAX_ACTIONS, o), dtype=torch.float32, device=env.device)
         return _rppo_train_function().apply(x, hidden_in, self, *params[4:])
 
+    def evaluate_head(self, obs, obs_format="wire"):
+        """The action head for a PPO update, on the tensor cores (evg_ppo_train_forward / _backward): stored observations,
+        wire rows uint8 [M, row_bytes] ('wire') or float32 [M, 2, obs_len] ('f32'), -> x float32 [R, L] = tanh(W2
+        bf16(tanh(W1 bf16(obs) + b1)) + b2), rows ordered like .idx / .hidden_in, ready for evaluate(x, hidden_in).
+        Differentiable with respect to action_head's four parameters.  bf16(x) is the operand the acting kernel's GRU
+        read, bit for bit, so from the acting call's .hidden_in, evaluate's h_7 is what that call left in .hidden.  See
+        _ff_evaluate for the images, the backward and the ValueError checks."""
+        return _ff_evaluate(self, _capi.PPO_TRAIN_HEAD, obs, obs_format, self.player, self.latent, [],
+                            lambda actor: _rppo_params(actor)[:4])
+
     def _train_images(self):
         """The training images (wi, wh, wht, w3 uint8, bias float32), allocated on first use."""
         import torch
@@ -631,6 +653,15 @@ class FusedValue:
         i1, i2, i3, bias = (C.c_void_p(t.data_ptr()) for t in self._w)
         _capi.check(env._lib.evg_pack_value(env._h, *src, L, i1, i2, i3, bias, env._stream()))
 
+    def evaluate(self, obs, obs_format="wire"):
+        """The critic for a PPO update, on the tensor cores (evg_ppo_train_forward / _backward): stored observations, wire
+        rows uint8 [M, row_bytes] ('wire') or float32 [M, 2, obs_len] ('f32'), -> V float32 [M, 2] (player -1) or [M],
+        bit for bit what self(obs, obs_format) gives with the acting images packed from the same parameters.
+        Differentiable with respect to the wrapped net's six parameters.  See _ff_evaluate for the images, the backward
+        and the ValueError checks."""
+        L = self.latent
+        return _ff_evaluate(self, _capi.PPO_TRAIN_CRITIC, obs, obs_format, self.player, 1, [(1, L), (1,)], _value_params)
+
     def __call__(self, obs=None, obs_format="f32", out=None):
         """State values float32 [M, 2] (player -1) or [M].  obs None: the env's own observations (M = num_envs; 'wire'
         reads env.obs_rows('wire'), the env stepped with obs_format='wire'), into .value unless `out` is given.
@@ -668,6 +699,131 @@ class FusedValue:
         _capi.check(env._lib.evg_policy_value(env._h, fmt, C.c_void_p(obs.data_ptr()), m, self.player, i1, i2, i3, bias, self.latent,
                                               C.c_void_p(out.data_ptr()), env._stream()))
         return out
+
+
+def _ff_evaluate(fused, net, obs, obs_format, player, out_dim, last_shapes, params_of):
+    """FusedPPO.evaluate, FusedValue.evaluate and FusedRPPO.evaluate_head: the network `net` (_capi.PPO_TRAIN_*) of the
+    wrapper's module on stored observations.  ValueError, before any launch, for a wrapper built from weights= (no module
+    to differentiate), an obs_format other than 'wire' or 'f32' (the kernels read no 'i16'), observations of the wrong
+    dtype, shape, device or contiguity, and parameters that are not contiguous float32 tensors on the env's device of the
+    wrapper's shapes.  M = 0 gives an empty tensor.  No host synchronisation: the call can be captured in a CUDA graph.
+
+    The forward packs the current parameters (evg_ppo_train_pack) and runs evg_ppo_train_forward, which also writes h1 and
+    h2.  The backward computes g2 = dL/dh2 in float32 torch (dz bf16(W3), dv bf16(w3) or the upstream dx), runs
+    evg_ppo_train_backward for dD2 and dD1, and reduces the parameter gradients with float32 torch.matmul / sum on what
+    the kernels wrote (torch's default precision: TF32 only where the caller enabled it): dW3 = dz^T bf16(h2), dW2 =
+    dD2^T bf16(h1), dW1 = dD1^T bf16(obs), the biases' the column sums.  Wire rows are expanded for dW1 on the device
+    (env.expand_wire).  No gradient flows to the observations.  The backward reads the wrapper's one W2^T image, packed
+    by the latest call: W2 is saved for backward, so changing it in place between a call and its backward (an
+    optimiser step under retain_graph) raises torch's version-counter error instead of using the newer W2; W3 is
+    saved for the same reason.  Several calls with unchanged parameters may be backpropagated in any order."""
+    import torch
+    env = fused.env
+    if fused._net is None:
+        raise ValueError("this wrapper was built from weights= arrays: it has no module to differentiate")
+    if obs_format not in ("f32", "wire"):
+        raise ValueError("obs_format must be 'f32' or 'wire', got %r" % (obs_format,))
+    if env.obs_len >= PPO_IN_PAD:
+        raise ValueError("observations of %d values do not fit the %d input columns of the fused kernels" % (env.obs_len, PPO_IN_PAD))
+    if obs_format == "f32":
+        fmt, dtype, tail, what = _capi.OBS_F32, torch.float32, (2, env.obs_len), "float32 observations [M, 2, %d]" % env.obs_len
+    else:
+        rb = int(env._lib.evg_obs_row_bytes(env._h, _capi.OBS_WIRE))
+        fmt, dtype, tail, what = _capi.OBS_WIRE, torch.uint8, (rb,), "uint8 wire rows [M, %d]" % rb
+    if not isinstance(obs, torch.Tensor) or obs.dtype != dtype or not obs.is_contiguous() or obs.device != env.device \
+            or obs.dim() != 1 + len(tail) or tuple(obs.shape[1:]) != tail:
+        raise ValueError("obs must be contiguous %s on %s, got %s" % (what, env.device, _describe(obs)))
+    L = fused.latent
+    params = params_of(fused._net)
+    for i, (t, shape) in enumerate(zip(params, [(L, env.obs_len), (L,), (L, L), (L,)] + last_shapes)):
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != env.device or tuple(t.shape) != shape:
+            raise ValueError("parameter %d must be a contiguous float32 tensor of shape %s on %s, got %s" % (i, shape, env.device, _describe(t)))
+    rows = obs.shape[0] * (2 if player < 0 else 1)
+    if obs.shape[0] == 0:
+        shape = {_capi.PPO_TRAIN_ACTOR: (0, out_dim), _capi.PPO_TRAIN_HEAD: (0, L)}.get(net, (0, 2) if player < 0 else (0,))
+        return torch.empty(shape, dtype=torch.float32, device=env.device)
+    y = _ff_train_function().apply(obs, fused, net, fmt, player, out_dim, *params)
+    return y.view(-1, 2) if net == _capi.PPO_TRAIN_CRITIC and player < 0 else y
+
+
+def _ff_train_images(fused, net):
+    """The training images of a wrapper (w1, w2, w3, w2t uint8, bias float32; w3 empty for the head), allocated on first use."""
+    import torch
+    if getattr(fused, "_ft", None) is None:
+        lp, ka = -(-fused.latent // 16) * 16, -(-fused.latent // ATOM) * ATOM
+        dev = fused.env.device
+        w3_rows = {_capi.PPO_TRAIN_ACTOR: PPO_OUT_PAD, _capi.PPO_TRAIN_CRITIC: VALUE_OUT_PAD}.get(net, 0)
+        b3 = {_capi.PPO_TRAIN_ACTOR: PPO_OUT_PAD, _capi.PPO_TRAIN_CRITIC: VALUE_OUT_PAD}.get(net, 0)
+        fused._ft = [torch.empty(n, dtype=torch.uint8, device=dev)
+                     for n in ((PPO_IN_PAD // ATOM) * lp * 128, (ka // ATOM) * lp * 128, max(1, (ka // ATOM) * w3_rows * 128), (ka // ATOM) * lp * 128)]
+        fused._ft.append(torch.empty(2 * PPO_MAX_LATENT + b3, dtype=torch.float32, device=dev))
+    return fused._ft
+
+
+_FF_TRAIN = None
+
+
+def _ff_train_function():
+    """The torch.autograd.Function of _ff_evaluate (defined on first use: torch is imported lazily)."""
+    global _FF_TRAIN
+    if _FF_TRAIN is None:
+        import torch
+
+        def bf16(t):
+            return t.to(torch.bfloat16).to(torch.float32)
+
+        def p(t):
+            return C.c_void_p(t.data_ptr()) if t is not None else None
+
+        class FFTrain(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, obs, fused, net, fmt, player, out_dim, w1, b1, w2, b2, w3=None, b3=None):
+                env, L = fused.env, fused.latent
+                R = obs.shape[0] * (2 if player < 0 else 1)
+                i1, i2, i3, i2t, bias = _ff_train_images(fused, net)
+                head = net == _capi.PPO_TRAIN_HEAD
+                _capi.check(env._lib.evg_ppo_train_pack(env._h, net, p(w1), p(b1), p(w2), p(b2), p(w3), p(b3), L, out_dim, p(i1), p(i2),
+                                                        None if head else p(i3), p(i2t), p(bias), env._stream()))
+                h1 = torch.empty((R, L), dtype=torch.float32, device=obs.device)
+                h2 = torch.empty((R, L), dtype=torch.float32, device=obs.device)
+                out = None if head else torch.empty((R, out_dim) if net == _capi.PPO_TRAIN_ACTOR else (R,), dtype=torch.float32, device=obs.device)
+                _capi.check(env._lib.evg_ppo_train_forward(env._h, net, fmt, p(obs), obs.shape[0], player, L, out_dim, p(i1), p(i2),
+                                                           None if head else p(i3), p(bias), p(out), p(h1), p(h2), env._stream()))
+                # w2 is saved for its version counter: the backward reads the wrapper's W2^T image, which the next
+                # evaluate re-packs, so a parameter changed in place in between must raise, as torch's own layers do
+                ctx.save_for_backward(obs, h1, h2, w2, w3)
+                ctx.fused, ctx.net, ctx.fmt, ctx.player = fused, net, fmt, player
+                return h2 if head else out
+
+            @staticmethod
+            def backward(ctx, dy):
+                obs, h1, h2, _, w3 = ctx.saved_tensors
+                fused, net, player = ctx.fused, ctx.net, ctx.player
+                env, (R, L) = fused.env, h1.shape
+                dy = dy.to(torch.float32).reshape(R, -1).contiguous()
+                if net == _capi.PPO_TRAIN_ACTOR:
+                    g2 = dy @ bf16(w3)
+                elif net == _capi.PPO_TRAIN_CRITIC:
+                    g2 = dy * bf16(w3)  # [R, 1] x [1, L]: dv_i w3_j
+                else:
+                    g2 = dy
+                g2 = g2.contiguous()
+                dd2 = torch.empty_like(h1)
+                dd1 = torch.empty_like(h1)
+                _capi.check(env._lib.evg_ppo_train_backward(env._h, R, L, p(_ff_train_images(fused, net)[3]), p(g2), p(h1), p(h2), p(dd2), p(dd1),
+                                                            env._stream()))
+                if ctx.fmt == _capi.OBS_WIRE:
+                    x = env.expand_wire(obs, player=player)
+                else:
+                    x = obs if player < 0 else obs[:, player]
+                x = bf16(x.reshape(R, env.obs_len))
+                grads = [dd1.t() @ x, dd1.sum(0), dd2.t() @ bf16(h1), dd2.sum(0)]
+                if net != _capi.PPO_TRAIN_HEAD:
+                    grads += [dy.t() @ bf16(h2), dy.sum(0)]
+                return (None,) * 6 + tuple(grads)
+
+        _FF_TRAIN = FFTrain
+    return _FF_TRAIN
 
 
 def _describe(t):

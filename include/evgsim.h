@@ -554,6 +554,54 @@ int evg_rppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, int32_t
                             const void* d_wi_img, const void* d_wh_img, const void* d_wht_img, const float* d_bias, float* d_g, float* d_dgh,
                             float* d_s, void* stream);
 
+/* PPO's feed-forward networks for an update, forward and backward, on the tensor cores (csrc/evg_ppo_train.cu;
+ * DESIGN.md §4.14).  `net` picks one of three networks that share their first two layers; L = latent (1..EVG_PPO_MAX_LATENT):
+ *     h1 = tanh(W1 bf16(obs) + b1),   h2 = tanh(W2 bf16(h1) + b2)
+ *     EVG_PPO_TRAIN_ACTOR  (the feed-forward actor, evg_policy_ppo): z = W3 bf16(h2) + b3, out = out_dim (7..EVG_PPO_OUT_PAD),
+ *                          the output of the actor's last Linear before its Tanh: evg_ppo_loss's z with K = 1.
+ *     EVG_PPO_TRAIN_CRITIC (evg_policy_value): v = w3 . bf16(h2) + b3 in evg_policy_value's order (fp32 FMAs in ascending
+ *                          column within each of four quarters of the 16-column groups, the four partials added in order,
+ *                          then b3); out_dim must be 1.
+ *     EVG_PPO_TRAIN_HEAD   (the recurrent actor's action_head, evg_policy_rppo): no last layer, the output is x = h2;
+ *                          out_dim must be L.
+ * The arithmetic is the acting kernels': bf16 operands, fp32 accumulation, fp32 biases, accurate tanhf, and the same MMAs
+ * (instruction N, K order, accumulate flags) as the acting kernel of the network (the head splits N into pieces of
+ * <= 128 rows as evg_policy_rppo does).  So z is what evg_policy_ppo takes tanh and softmax of, v is evg_policy_value's
+ * value, and bf16(x) is the operand evg_policy_rppo's GRU reads, all bit for bit.
+ *   evg_ppo_train_pack: the images, packed on the device from the float32 parameters in torch's layouts (d_w1 [L][obs_len],
+ *       d_w2 [L][L], d_w3 [out][L], biases [out]; d_w3 / d_b3 NULL for the head), every byte written:
+ *         d_w1_img, d_w2_img: exactly as for evg_policy_ppo;  d_w3_img: the actor's as for evg_policy_ppo, the critic's as
+ *         for evg_policy_value, NULL for the head;  d_w2t_img: W2^T as an [Lp x Ka] block, element (j, i) = w2[i][j];
+ *         d_bias: float32 b1 at 0, b2 at EVG_PPO_MAX_LATENT, then the actor's b3 [EVG_PPO_OUT_PAD] or the critic's
+ *         [EVG_VALUE_OUT_PAD] at 2 * EVG_PPO_MAX_LATENT (the head's vector ends there), zero padded.
+ *   evg_ppo_train_forward: n_matches stored matches' observations in `format` (EVG_OBS_F32 float32 [n_matches][2][obs_len],
+ *       4-byte aligned, or EVG_OBS_WIRE rows, 16-byte aligned, needs evg_bind; EVG_OBS_I16 is refused), the rows of
+ *       `player` as for evg_policy_value: R = n_matches * 2 for player -1 (row i = match i / 2, player i % 2), else n_matches.
+ *       Writes d_out (actor: z float32 [R][out]; critic: v float32 [R]; head: not read, may be NULL) and d_h1, d_h2
+ *       float32 [R][L].
+ *   evg_ppo_train_backward, from g2 = dL/dh2 (d_g2 float32 [R][L]; the caller's: dz bf16(W3) for the actor, dv bf16(w3)
+ *       for the critic, dx for the head) and the forward's d_h1, d_h2, with the bf16 roundings taken as the identity:
+ *         dD2 = g2 (1 - h2^2),   dD1 = (bf16(dD2) . bf16(W2)) (1 - h1^2)   (tensor cores, bf16(dD2) the MMA operand,
+ *         fp32 accumulation; FMA contraction allowed in the elementwise products)
+ *       into d_dd2, d_dd1 float32 [R][L].
+ *   The parameter gradients are the caller's reductions dW3 = dz^T bf16(h2), dW2 = dD2^T bf16(h1), dW1 = dD1^T bf16(obs),
+ *   the biases' the column sums; no gradient flows to the observations.
+ * Images and d_bias 16-byte aligned, float32 arrays 4-byte aligned.  One launch on `stream` each, no allocation, no
+ * synchronisation.  EVG_E_ARG, checked before the handle, for `net` unknown, R outside 1..2^31-1, latent or out_dim out of
+ * range, player outside -1..1, a format other than EVG_OBS_F32 / EVG_OBS_WIRE, a NULL pointer and a misaligned one; after
+ * it, for obs_len >= EVG_PPO_IN_PAD (and EVG_E_STATE for wire rows without evg_bind). */
+#define EVG_PPO_TRAIN_ACTOR 0
+#define EVG_PPO_TRAIN_CRITIC 1
+#define EVG_PPO_TRAIN_HEAD 2
+int evg_ppo_train_pack(EvgSim* sim, int32_t net, const float* d_w1, const float* d_b1, const float* d_w2, const float* d_b2, const float* d_w3,
+                       const float* d_b3, int32_t latent, int32_t out_dim, void* d_w1_img, void* d_w2_img, void* d_w3_img, void* d_w2t_img,
+                       float* d_bias, void* stream);
+int evg_ppo_train_forward(EvgSim* sim, int32_t net, int32_t format, const void* d_obs, int64_t n_matches, int32_t player, int32_t latent,
+                          int32_t out_dim, const void* d_w1_img, const void* d_w2_img, const void* d_w3_img, const float* d_bias, float* d_out,
+                          float* d_h1, float* d_h2, void* stream);
+int evg_ppo_train_backward(EvgSim* sim, int64_t n_rows, int32_t latent, const void* d_w2t_img, const float* d_g2, const float* d_h1,
+                           const float* d_h2, float* d_dd2, float* d_dd1, void* stream);
+
 /* The images above packed ON THE DEVICE from the network's float32 parameters (csrc/evg_policy_pack.cu), byte for byte
  * what evgsim.policy.pack_mlp / pack_ppo / pack_rppo / pack_value build on the host: one launch on `stream`, no host synchronisation,
  * so a training loop refreshes the images in place after each optimiser step (and can capture that in a CUDA graph).
